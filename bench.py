@@ -4,6 +4,7 @@ decoded per second at beam=100).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--kind gauss|peaky]
                   [--workload cfg1|cfg2|cfg3|cfg4|cfg5]   (default cfg2, the shape the metric is quoted on)
+                  [--dump-outputs DIR]
 
 One "step" = one decode of one batch of synthetic logits: the LibriSpeech char-CTC shape the metric
 is quoted on (BASELINE.json configs[1]): T=500, B=256 per GPU, C=29 (blank=28), beam_width=100,
@@ -20,6 +21,10 @@ implementation (oracle/_ref, compiled from the reference's unmodified headers; f
 plain-C port in oracle/) on the host cores on a bounded sample of the same workload.
 
 Reference arm (--impl reference): the reference CPU op on all host cores, same config and metric.
+
+--dump-outputs DIR: after the timed steps, the raw outputs of the last device-resident step (rank 0)
+are written as DIR/<output>[_<path>].npy. The inputs depend only on the arguments, so two builds run
+with the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -53,11 +58,42 @@ WORKLOADS = {
 }
 CFG = dict(WORKLOADS["cfg2"])
 L2_BYTES = 126 * 1024 * 1024
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
 
 
 def make_batch(kind, seed, T, B, C, blank):
     import ctcx_testlib as L
     return L.make_logits(kind, T, B, C, blank, seed)
+
+
+def outputs_to_numpy(raw):
+    """The raw op's outputs as {file name: array}: one array per output and path (decoded_values_0,
+    ...), log_probability as one [B, top_paths] array. Integer outputs become float64, which holds
+    every index and label exactly; log-probabilities keep their float type. Above DUMP_LIMIT_BYTES in
+    all, every sparse output keeps the same fixed, seeded sample of its entries (indices and values of
+    one path stay paired)."""
+    arrays = {}
+    for name, group in zip(raw._fields, raw):
+        for key, t in ([(name, group)] if name == "log_probability" else
+                       [("%s_%d" % (name, p), t) for p, t in enumerate(group)]):
+            a = t.detach().cpu().numpy()
+            arrays[key] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    sparse = [k for k in arrays if k.startswith(("decoded_indices", "decoded_values", "alignment_indices",
+                                                 "alignment_values"))]
+    sparse_bytes = sum(arrays[k].nbytes for k in sparse)
+    budget = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values()) + sparse_bytes
+    if sparse_bytes > budget:
+        for key in sparse:
+            n = arrays[key].shape[0]
+            keep = np.random.default_rng(0).choice(n, n * budget // sparse_bytes, replace=False)
+            arrays[key] = arrays[key][np.sort(keep)]
+    return arrays
+
+
+def write_outputs(arrays, out_dir):
+    os.makedirs(out_dir, exist_ok=True)
+    for key, a in arrays.items():
+        np.save(os.path.join(out_dir, key + ".npy"), a)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -259,14 +295,18 @@ def run_own_arm(args, rank, world, local_rank, out_fd=1):
     wall0 = time.perf_counter()
     for i, (e0, e1) in enumerate(evs):
         e0.record()
-        step_device(i)
+        res = step_device(i)
         e1.record()
         lib.ctcx_profile_get(buf)
         kern_ms[i] = list(buf)
+        if i < args.steps - 1:
+            res = None  # freed before the next step, as in the warm-up; the last step's result is kept
     barrier()
     wall_dev = time.perf_counter() - wall0
     lib.ctcx_profile_enable(0)
     dev_ms = float(sum(e0.elapsed_time(e1) for e0, e1 in evs))
+    dumped = outputs_to_numpy(res) if args.dump_outputs and rank == 0 else None
+    del res
 
     # ---- end-to-end timing: pinned host logits in, host results out ----
     barrier()
@@ -329,7 +369,7 @@ def run_own_arm(args, rank, world, local_rank, out_fd=1):
     if args.workload == "cfg2" and args.dtype == "f32" and not args.scorer and not args.no_sharded:
         del dev_batches, host_batches
         torch.cuda.empty_cache()
-        sharded = run_sharded_cfg5(rank, world, local_rank, steps=max(3, min(args.steps, 10)), warmup=3)
+        sharded = run_sharded_cfg5(rank, world, local_rank, steps=args.steps, warmup=3)
     if rank != 0:
         return
 
@@ -400,6 +440,8 @@ def run_own_arm(args, rank, world, local_rank, out_fd=1):
                                 "sample": "%d utterances of this workload on one thread (%.1f s)" % (n1, dt1),
                                 "all_host_threads": {"value": n_utt * T / dt, "cores": cores,
                                                      "sample": "%d utterances, one per thread (%.1f s)" % (n_utt, dt)}}
+    if dumped is not None:
+        write_outputs(dumped, args.dump_outputs)
     sys.stdout.flush()
     os.write(out_fd, (json.dumps(line) + "\n").encode())
 
@@ -409,7 +451,9 @@ def run_sharded_cfg5(rank, world, local_rank, steps, warmup):
     beam 100), batch-sharded over the ranks through the product's sharding API (decode_distributed: rank r
     decodes block r IN PLACE from a view of the time-major tensor, the sparse outputs are gathered on rank 0
     INSIDE the timed region). Strong scaling: frames/s = 8192 * 500 / max-over-ranks wall time per step.
-    Two variants: logits resident on each GPU / in page-locked host memory."""
+    Two variants: logits resident on each GPU / in page-locked host memory. Each runs `steps` timed steps
+    (--steps): about 80 ms per step for the two together on one B200 (1000 W power limit), so about 4 s at
+    the default of 50 steps."""
     import torch
     import torch.distributed as dist
     import ctc_beam_search_op_b200 as op
@@ -483,7 +527,14 @@ def main():
     ap.add_argument("--scorer", action="store_true", help="decode with a label-bigram expansion-score table")
     ap.add_argument("--no-numa-bind", action="store_true",
                     help="do not move the process next to its GPU (bind_host_to_device) before allocating host buffers")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the raw outputs of the last timed device-resident step as "
+                         "DIR/<output>_<path>.npy and DIR/log_probability.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to --impl ours")
     CFG.clear()
     CFG.update(WORKLOADS[args.workload])
     rank = int(os.environ.get("RANK", "0"))

@@ -1,5 +1,6 @@
 import os, sys, time
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import numpy as np, torch
 import ctcx_testlib as L
 import ctc_beam_search_op_b200 as op
