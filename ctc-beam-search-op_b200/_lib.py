@@ -36,7 +36,7 @@ EXPORTS = ("ctcx_strerror", "ctcx_last_cuda_error", "ctcx_error_batch_index", "c
            "ctcx_stream_workspace_bytes", "ctcx_stream_reset", "ctcx_stream_step_f32", "ctcx_stream_top_paths",
            # measurement and test hooks
            "ctcx_workspace_views", "ctcx_profile_enable", "ctcx_profile_get", "ctcx_debug_set_cycles_buffer",
-           "ctcx_debug_set_beam_impl", "ctcx_debug_math_f32", "ctcx_debug_math_f64")
+           "ctcx_debug_set_beam_impl", "ctcx_debug_math_f32", "ctcx_debug_math_f64", "ctcx_debug_prepass")
 
 F32, F16, BF16, F64 = 0, 1, 2, 3  # CTCX_F32 ... (include/ctcx.h)
 
@@ -120,5 +120,7 @@ def load():
     lib.ctcx_debug_set_cycles_buffer.restype = None
     lib.ctcx_debug_math_f32.argtypes = [ctypes.c_int, _vp, _vp, ctypes.c_int, _vp]
     lib.ctcx_debug_math_f64.argtypes = [ctypes.c_int, _vp, _vp, ctypes.c_int, _vp]
+    lib.ctcx_debug_prepass.argtypes = [_i, _vp, _i, _i, _i, _i, ctypes.c_longlong, _i, _i, _vp, _vp, _vp,
+                                       ctypes.POINTER(_i), _vp]
     _lib = lib
     return lib

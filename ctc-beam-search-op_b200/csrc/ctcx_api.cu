@@ -1102,7 +1102,43 @@ void ctcx_debug_set_cycles_buffer(long long* dev_buf) { g_dbg_cycles = dev_buf; 
  * the independent second implementation the parity tests compare with the fast ones. */
 void ctcx_debug_set_beam_impl(int impl) { g_force_generic.store(impl == 1 ? 1 : 0); }
 
-/* y = f(x) element-wise with the exact device math; op 0 expf, 1 log1pf, 2 logf */
+/* The normaliser pre-pass of a decode on its own, through the launchers the decode calls: route 0 the
+ * generic path's (LaunchLogNorm; half inputs upcast first), route 1 the wide path's fused normaliser
+ * and sorted-class list (LaunchNormTopClasses). */
+int ctcx_debug_prepass(int route, const void* logits_dev, int in_dtype, int T, int B, int C, long long tstride,
+                       int blank_index, int beam_width, void* off_dev, float* srt_pl_dev, uint16_t* srt_cls_dev,
+                       int* ks_out, void* stream_v) {
+  cudaStream_t stream = (cudaStream_t)stream_v;
+  if (tstride == 0) tstride = (long long)B * C;
+  if (T < 1 || B < 1 || C < 1 || C > kMaxClasses || blank_index < 0 || blank_index >= C ||
+      tstride < (long long)B * C || ElemBytes(in_dtype) == 0 || logits_dev == nullptr || off_dev == nullptr)
+    return CTCX_ERR_BAD_ARGUMENT;
+  const long long rows = (long long)T * B;
+  if (route == 0) {
+    if (ks_out) *ks_out = 0;
+    if (in_dtype == CTCX_F64)
+      return FromLaunch(ctcx::LaunchLogNorm((const double*)logits_dev, (double*)off_dev, rows, C, B, tstride, stream));
+    if (in_dtype == CTCX_F32)
+      return FromLaunch(ctcx::LaunchLogNorm((const float*)logits_dev, (float*)off_dev, rows, C, B, tstride, stream));
+    float* scratch = nullptr;
+    CTCX_CUDA(cudaMallocAsync((void**)&scratch, (size_t)rows * C * sizeof(float), stream));
+    int rc = FromLaunch(ctcx::LaunchUpcast(logits_dev, InDtypeOf(in_dtype), scratch, T, B, C, tstride, stream));
+    if (rc == CTCX_OK)
+      rc = FromLaunch(ctcx::LaunchLogNorm(scratch, (float*)off_dev, rows, C, B, (long long)B * C, stream));
+    if (!Check(cudaFreeAsync(scratch, stream), "cudaFreeAsync") && rc == CTCX_OK) rc = CTCX_ERR_CUDA;
+    return rc;
+  }
+  if (route != 1) return CTCX_ERR_BAD_ARGUMENT;
+  if (in_dtype == CTCX_F64 || beam_width < 1 || !ctcx::WideFastShape(beam_width, C)) return CTCX_ERR_UNSUPPORTED;
+  if (srt_pl_dev == nullptr || srt_cls_dev == nullptr) return CTCX_ERR_BAD_ARGUMENT;
+  if (ks_out) *ks_out = ctcx::WideKs(beam_width, C);
+  return FromLaunch(ctcx::LaunchNormTopClasses(logits_dev, InDtypeOf(in_dtype), (float*)off_dev, rows, C, blank_index,
+                                               beam_width, srt_pl_dev, (unsigned short*)srt_cls_dev, B, tstride,
+                                               stream));
+}
+
+/* y = f(x) element-wise with the exact device math; op 0 expf, 1 log1pf, 2 logf, 3 LogSumExp(x, 0),
+ * 4 LogSumExp(0, x) */
 int ctcx_debug_math_f32(int op, const float* x_dev, float* y_dev, int n, void* stream_v) {
   if (n <= 0) return CTCX_OK;
   CTCX_LAUNCH(ctcx::LaunchMathTest(op, x_dev, y_dev, n, (cudaStream_t)stream_v));

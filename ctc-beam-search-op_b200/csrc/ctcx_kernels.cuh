@@ -1412,6 +1412,7 @@ static __global__ void __launch_bounds__(128) PackKernel(PackParams p) {
 }
 
 // Test hook: element-wise evaluation of the exact math functions.
+// op 0: expf, 1: log1pf, 2: logf, 3: LogSumExp(x, 0), 4: LogSumExp(0, x)
 static __global__ void MathTestKernel(int op, const float* x, float* y, int n) {
   __shared__ unsigned long long s_tab[32];
   LoadExpTable(s_tab, threadIdx.x, blockDim.x);
@@ -1419,7 +1420,8 @@ static __global__ void MathTestKernel(int op, const float* x, float* y, int n) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float v = x[i];
-  y[i] = (op == 0) ? ExpfExact(v, s_tab) : (op == 1) ? Log1pfExact(v) : LogfExact(v);
+  y[i] = (op == 0) ? ExpfExact(v, s_tab) : (op == 1) ? Log1pfExact(v) : (op == 2) ? LogfExact(v)
+       : (op == 3) ? LogSumExp(v, 0.0f, s_tab) : LogSumExp(0.0f, v, s_tab);
 }
 
 // op 0: exp (x <= 0), 1: log (x >= 1), 2: LogSumExp(x, 0) of the double path

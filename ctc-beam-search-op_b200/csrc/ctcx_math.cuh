@@ -5,8 +5,10 @@
 // (Arm Optimized Routines expf/logf in double precision with every product-sum fused; fdlibm
 // log1pf in single precision without contraction). All operations use explicit round-to-nearest
 // intrinsics so nvcc can neither contract nor re-associate them; the results are bit-identical to
-// the host libm (checked exhaustively on the CPU for the portable twin of this code, see DESIGN.md
-// "Numerics"), which makes device scores bit-identical to the reference's.
+// the host libm, which makes device scores bit-identical to the reference's. tests/test_gpu_exact_math.py
+// checks these device functions against glibc on every float of the domains below (and LogSumExp on
+// every float difference in [-104, 0]); the double functions further down at every reduction-cell and
+// table edge plus 2^27 random arguments each (DESIGN.md "Numerics").
 //
 // Domains used by the decoder: expf(x <= 0 or -inf), log1pf(0 <= x <= 1), logf(1 <= x < 2^16).
 #pragma once

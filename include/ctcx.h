@@ -298,9 +298,22 @@ void ctcx_debug_set_cycles_buffer(long long* dev_buf);
 void ctcx_debug_set_beam_impl(int impl);
 
 /* y = f(x) element-wise with the exact device math (bit-identical to glibc 2.39, DESIGN.md section 6):
- * f32 op 0 expf (x <= 0), 1 log1pf (0 <= x <= 1), 2 logf (x >= 1); f64 op 0 exp, 1 log, 2 LogSumExp(x, 0). */
+ * f32 op 0 expf (x <= 0), 1 log1pf (0 <= x <= 1), 2 logf (x >= 1), 3 LogSumExp(x, 0), 4 LogSumExp(0, x);
+ * f64 op 0 exp, 1 log, 2 LogSumExp(x, 0). */
 int ctcx_debug_math_f32(int op, const float* x_dev, float* y_dev, int n, void* stream);
 int ctcx_debug_math_f64(int op, const double* x_dev, double* y_dev, int n, void* stream);
+
+/* The softmax-normaliser pre-pass of a decode, run alone on the T*B rows of a [T, B, C] tensor of
+ * element type `in_dtype` (CTCX_F32 ... ; time stride `tstride` elements, 0 = B*C) with the launchers
+ * the decode uses. off_dev[T*B] (double for CTCX_F64, float otherwise) receives max + log(sum exp).
+ * route 0: the generic path's normaliser (half inputs are upcast to float32 first).
+ * route 1: the wide path's fused pre-pass (32 < C <= 2048, shapes the wide kernel takes, not CTCX_F64):
+ *   also srt_pl_dev / srt_cls_dev[T*B, *ks_out] receive per row the first min(C-1, 2*beam_width+3)
+ *   non-blank classes by (log-prob desc, class asc), then (-inf, 0xffff) padding.
+ * Returns CTCX_ERR_UNSUPPORTED for a shape the route does not serve. Asynchronous on `stream`. */
+int ctcx_debug_prepass(int route, const void* logits_dev, int in_dtype, int T, int B, int C, long long tstride,
+                       int blank_index, int beam_width, void* off_dev, float* srt_pl_dev, uint16_t* srt_cls_dev,
+                       int* ks_out, void* stream);
 
 #ifdef __cplusplus
 }

@@ -27,6 +27,40 @@ long long ctcx_port_mismatches(unsigned stride, long long* out) {
   return be + bl + bg;
 }
 
+/* util/ctc_loss_util.h:33-41 with the host libm */
+static float ctcx_libm_lse(float a, float b) {
+  if (a == -INFINITY) return b;
+  if (b == -INFINITY) return a;
+  return (a > b) ? a + log1pf(expf(b - a)) : b + log1pf(expf(a - b));
+}
+
+/* Compares n results `got` of a device function with the host libm at the inputs whose bit patterns
+ * are u0 ... u0+n-1. op 0 expf, 1 log1pf, 2 logf, 3 LogSumExp(x, 0), 4 LogSumExp(0, x) (the ops of
+ * ctcx_debug_math_f32). Returns the number of inputs whose results differ in any bit; the first
+ * min(count, max_bad) of them go to first_bad. */
+long long ctcx_libm_mismatches_f32(int op, uint32_t u0, long long n, const float* got, uint32_t* first_bad,
+                                   int max_bad) {
+  long long bad = 0;
+  for (long long i = 0; i < n; ++i) {
+    const uint32_t u = u0 + (uint32_t)i;
+    volatile float x = ctcx_asfloat(u);
+    float want;
+    switch (op) {
+      case 0: want = expf(x); break;
+      case 1: want = log1pf(x); break;
+      case 2: want = logf(x); break;
+      case 3: want = ctcx_libm_lse(x, 0.0f); break;
+      case 4: want = ctcx_libm_lse(0.0f, x); break;
+      default: return -1;
+    }
+    if (ctcx_asuint(want) != ctcx_asuint(got[i])) {
+      if (bad < max_bad) first_bad[bad] = u;
+      ++bad;
+    }
+  }
+  return bad;
+}
+
 /* element-wise helpers for the Python side of the tests */
 void ctcx_port_expf_v(const float* x, float* y, int n) { for (int i = 0; i < n; ++i) y[i] = ctcx_port_expf(x[i]); }
 void ctcx_port_log1pf_v(const float* x, float* y, int n) { for (int i = 0; i < n; ++i) y[i] = ctcx_port_log1pf(x[i]); }

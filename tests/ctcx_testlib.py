@@ -26,8 +26,8 @@ class OracleError(Exception):
 
 def build_oracles(force=False):
     """Compile oracle/libctcx_oracle.so and (where /root/reference exists) oracle/_ref."""
-    if force or not os.path.exists(ORACLE_SO) or (
-            os.path.getmtime(ORACLE_SO) < os.path.getmtime(os.path.join(ORACLE_DIR, "ctcx_oracle.c"))):
+    if force or not os.path.exists(ORACLE_SO) or os.path.getmtime(ORACLE_SO) < max(
+            os.path.getmtime(os.path.join(ORACLE_DIR, f)) for f in ("ctcx_oracle.c", "libm_port_check.c")):
         subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "oracle"])
     if os.path.isdir("/root/reference/tensorflow_ctc_ext_beam_search_decoder") and (
             force or not os.path.exists(REF_SO)
