@@ -40,11 +40,12 @@ int FromLaunch(const ctcx::LaunchStatus& st) {
   if (st.code == ctcx::kLaunchCuda) Check(st.cuda, st.what);
   return st.code;
 }
-#define CTCX_LAUNCH(call)                       \
+#define CTCX_RC(call)                           \
   do {                                          \
-    const int rc_ = FromLaunch(call);           \
+    const int rc_ = (call);                     \
     if (rc_ != CTCX_OK) return rc_;             \
   } while (0)
+#define CTCX_LAUNCH(call) CTCX_RC(FromLaunch(call))
 
 constexpr int kMaxBeamWidth = 1024;
 constexpr int kMaxClasses = 65535;
@@ -53,17 +54,30 @@ constexpr int kNStats = 16;
 
 size_t Align256(size_t v) { return (v + 255) / 256 * 256; }
 
+// The result block, ONE copy to the host: sizes [4,P] int64, then the kNStats status words (stats[0..5]
+// as FlagsKernel reduces them; stats[6] = the compact pack's overflow word).
+size_t StatsOffset(int P) { return 4 * (size_t)P * 8; }
+size_t ResultBytes(int P) { return StatsOffset(P) + kNStats * 4; }
+// status words before the kernels run: no flags, and B (= none) as every "first failing utterance"
+void InitStats(int* stats, int B) {
+  stats[0] = 0;
+  for (int k = 1; k < 6; ++k) stats[k] = B;
+}
+
 // test hook (ctcx_debug_set_beam_impl): 1 = route every decode to the generic beam kernel
 std::atomic<int> g_force_generic{0};
 // measurement hook (ctcx_debug_set_cycles_buffer)
 thread_local long long* g_dbg_cycles = nullptr;
 
 enum Path { kPathNarrow, kPathWide, kPathGeneric };
+// which beam kernel (and with it which pre-pass) decodes this shape with R scores
+template <typename R>
 Path PathOf(int W, int C, bool scorer) {
   if (g_force_generic.load(std::memory_order_relaxed)) return kPathGeneric;
   if (ctcx::NarrowFastShape(W, C)) return kPathNarrow;  // (has a scorer variant: all 32 classes tested per row)
-  // a scorer table breaks the wide kernel's monotone-prefix argument: generic kernel
-  if (scorer) return kPathGeneric;
+  // a scorer table breaks the wide kernel's monotone-prefix argument, and the wide kernel has no
+  // float64 form: generic kernel
+  if (scorer || sizeof(R) == 8) return kPathGeneric;
   if (ctcx::WideFastShape(W, C)) return kPathWide;
   return kPathGeneric;
 }
@@ -77,7 +91,7 @@ struct Workspace {
     int T, B, C, W, P;
     int real_bytes;  // 4: float32 decode, 8: float64 decode
   };
-  size_t header, result, ctrl, dec_len, ali_len, dec_off, ali_off, ptrs, fin_total, fin_kind, dec, ali,
+  size_t header, result, stats, ctrl, dec_len, ali_len, dec_off, ali_off, ptrs, fin_total, fin_kind, dec, ali,
       seq, chunk_len, fin_n, flags, t_done, state, off, bp, srt_pl, srt_cls, scratch, bytes;
   int Cs;         // row stride of the sorted-class arrays (0 when the wide fast path does not apply)
   int rec_bytes;  // back-pointer record size
@@ -85,7 +99,8 @@ struct Workspace {
     size_t o = 0;
     const size_t b = (size_t)B, t = (size_t)T, pp = (size_t)P;
     header = o; o += Align256(sizeof(Header));
-    result = o; o += Align256(4 * pp * 8 + kNStats * 4);         // sizes [4,P] int64, then stats: ONE copy to the host
+    result = o; o += Align256(ResultBytes(P));
+    stats = result + StatsOffset(P);
     ctrl = o; o += 256;                                          // [0] utterance queue, [1] frames landed
     dec_len = o; o += Align256(b * pp * 4);
     ali_len = o; o += Align256(b * pp * 4);
@@ -119,6 +134,9 @@ struct Workspace {
     scratch = o; o += (narrow || wide) ? 0 : Align256(t * b * (size_t)C * 4);
     bytes = o;
   }
+  // the upcast room, or null where a fast kernel takes the shape (even with the generic kernel forced:
+  // the layout does not depend on the test hook)
+  float* Scratch(unsigned char* base) const { return bytes > scratch ? (float*)(base + scratch) : nullptr; }
 };
 
 thread_local int g_err_batch = -1;
@@ -151,8 +169,27 @@ struct DecodeOpts {
   const cudaEvent_t* slab_event = nullptr;
 };
 
-int ReportSizes(const long long* h_sizes, const int* h_stats, int B, int T, int P, ctcx_sizes* sizes,
-                int32_t* flags_out) {
+// header + zeroed sizes + initial stats + control words, staged in one host block -> one H2D copy
+struct InitBlock {
+  std::vector<unsigned char> bytes;
+  InitBlock(const Workspace& ws, const Workspace::Header& hdr, int B) : bytes(ws.dec_len, 0) {
+    std::memcpy(bytes.data() + ws.header, &hdr, sizeof(hdr));
+    InitStats(reinterpret_cast<int*>(bytes.data() + ws.stats), B);
+  }
+};
+
+// per-kernel times of the LAST decode this thread enqueued (ctcx_profile_enable), once it has completed
+void CollectProfile(int B) {
+  if (!g_profile || B <= 0 || !g_ev_ready || cudaEventQuery(g_ev[4]) != cudaSuccess) return;
+  for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&g_ms[k], g_ev[k], g_ev[k + 1]);
+  cudaEventElapsedTime(&g_ms[4], g_ev[0], g_ev[4]);
+}
+
+// the result block as it arrived on the host -> sizes, flags, return code
+int ParseResult(const unsigned char* h_res, int T, int B, int P, ctcx_sizes* sizes, int32_t* flags_out) {
+  const long long* h_sizes = (const long long*)h_res;
+  const int* h_stats = (const int*)(h_res + StatsOffset(P));
+  if (h_stats[6] != 0) return CTCX_ERR_WORKSPACE;  // ctcx_pack_compact: the caller's buffer was too small
   if (h_stats[5] < B) {
     std::snprintf(g_cuda_err, sizeof(g_cuda_err), "the host->device copy of the logits never delivered the frames of utterance %d",
                   h_stats[5]);
@@ -180,33 +217,6 @@ int ReportSizes(const long long* h_sizes, const int* h_stats, int B, int T, int 
   return CTCX_OK;
 }
 
-// header + zeroed sizes + initial stats + control words, staged in one host block -> one H2D copy
-struct InitBlock {
-  std::vector<unsigned char> bytes;
-  InitBlock(const Workspace& ws, const Workspace::Header& hdr, int B, int P) : bytes(ws.dec_len, 0) {
-    std::memcpy(bytes.data() + ws.header, &hdr, sizeof(hdr));
-    int* stats = reinterpret_cast<int*>(bytes.data() + ws.result + 4 * (size_t)P * 8);
-    stats[0] = 0;
-    for (int k = 1; k < 6; ++k) stats[k] = B;
-  }
-};
-
-size_t ResultBytes(int P) { return 4 * (size_t)P * 8 + kNStats * 4; }
-
-// per-kernel times of the LAST decode this thread enqueued (ctcx_profile_enable), once it has completed
-void CollectProfile(int B) {
-  if (!g_profile || B <= 0 || !g_ev_ready || cudaEventQuery(g_ev[4]) != cudaSuccess) return;
-  for (int k = 0; k < 4; ++k) cudaEventElapsedTime(&g_ms[k], g_ev[k], g_ev[k + 1]);
-  cudaEventElapsedTime(&g_ms[4], g_ev[0], g_ev[4]);
-}
-
-// the result block (sizes [4,P] + status words) as it arrived on the host -> sizes, flags, return code
-int ParseResult(const unsigned char* h_res, int T, int B, int P, ctcx_sizes* sizes, int32_t* flags_out) {
-  const int* h_stats = (const int*)(h_res + 4 * (size_t)P * 8);
-  if (h_stats[6] != 0) return CTCX_ERR_WORKSPACE;  // ctcx_pack_compact: the caller's buffer was too small
-  return ReportSizes((const long long*)h_res, h_stats, B, T, P, sizes, flags_out);
-}
-
 // ONE copy brings the sparse sizes and the status words to the host; the only synchronisation of a decode
 int FinishImpl(const unsigned char* d_result, int T, int B, int P, cudaStream_t stream, ctcx_sizes* sizes,
                int32_t* flags_out) {
@@ -217,12 +227,125 @@ int FinishImpl(const unsigned char* d_result, int T, int B, int P, cudaStream_t 
   return ParseResult(h_res.data(), T, B, P, sizes, flags_out);
 }
 
+// Logits as the kernels read them: [T,B,C] of element type in_dtype (float64 decodes: kInF32, unused),
+// row (t, b) at element t * tstride + b * C.
+struct Logits {
+  const void* p;
+  int in_dtype;
+  long long tstride;
+};
+
+// Enqueues the normaliser pre-pass the beam kernel of `path` needs, over the T*B rows of `x`: nothing
+// for the narrow kernel, which normalises inside; the normaliser and every row's best classes, sorted,
+// for the wide kernel; the normaliser alone for the generic kernel, half-precision logits first widened
+// exactly into `scratch` ([T,B,C] float32; null = no room), which then stands in for `x`.
+template <typename R>
+int PrePass(Path path, Logits& x, int T, int B, int C, int blank_index, int W, R* off, float* srt_pl,
+            unsigned short* srt_cls, float* scratch, cudaStream_t stream) {
+  const long long rows = (long long)T * B;
+  if (path == kPathNarrow) return CTCX_OK;
+  if constexpr (sizeof(R) == 8) {
+    CTCX_LAUNCH(ctcx::LaunchLogNorm((const double*)x.p, off, rows, C, B, x.tstride, stream));
+  } else if (path == kPathWide) {
+    CTCX_LAUNCH(ctcx::LaunchNormTopClasses(x.p, x.in_dtype, off, rows, C, blank_index, W, srt_pl, srt_cls, B,
+                                           x.tstride, stream));
+  } else {
+    if (x.in_dtype != ctcx::kInF32) {
+      if (scratch == nullptr) return CTCX_ERR_UNSUPPORTED;
+      CTCX_LAUNCH(ctcx::LaunchUpcast(x.p, x.in_dtype, scratch, T, B, C, x.tstride, stream));
+      x = {scratch, ctcx::kInF32, (long long)B * C};
+    }
+    CTCX_LAUNCH(ctcx::LaunchLogNorm((const float*)x.p, off, rows, C, B, x.tstride, stream));
+  }
+  return CTCX_OK;
+}
+
+// The beam kernels' parameters over a workspace laid out for Tcap frames: a pass over all of them that
+// carries no beam in or out. Streamed passes add state and t_done.
+template <typename R>
+ctcx::BeamParamsT<R> BeamParamsOf(const Workspace& ws, unsigned char* base, int Tcap, int B, int C, int W, int P,
+                                  int blank_index, const int* seq_len) {
+  ctcx::BeamParamsT<R> bp;
+  std::memset(&bp, 0, sizeof(bp));
+  bp.off = (const R*)(base + ws.off);
+  bp.seq_len = seq_len;
+  bp.T = Tcap; bp.B = B; bp.C = C; bp.W = W; bp.P = P;
+  bp.blank_index = blank_index;
+  if (ws.rec_bytes == 4) bp.bp32 = (unsigned*)(base + ws.bp); else bp.bp = (uint2*)(base + ws.bp);
+  bp.fin_total = (R*)(base + ws.fin_total);
+  bp.fin_kind = (int*)(base + ws.fin_kind);
+  bp.fin_n = (int*)(base + ws.fin_n);
+  bp.flags = (int*)(base + ws.flags);
+  bp.Tcap = Tcap;
+  if (ws.Cs > 0) {  // the wide kernel's sorted classes
+    bp.srt_pl = (const R*)(base + ws.srt_pl);
+    bp.srt_cls = (const unsigned short*)(base + ws.srt_cls);
+  }
+  bp.queue = (int*)(base + ws.ctrl);
+  bp.n_slices = 1;
+  bp.slice_frames = Tcap;
+  return bp;
+}
+
+// One beam pass over the frames [0, bp.T) of `x`: the pre-pass of `path` into the workspace, then the
+// beam kernel of `path`. `after_prepass`, if set, is recorded between the two.
+template <typename R>
+int BeamPass(Path path, Logits x, ctcx::BeamParamsT<R>& bp, const Workspace& ws, unsigned char* base,
+             cudaEvent_t after_prepass, cudaStream_t stream) {
+  CTCX_RC(PrePass<R>(path, x, bp.T, bp.B, bp.C, bp.blank_index, bp.W, (R*)(base + ws.off), (float*)(base + ws.srt_pl),
+                     (unsigned short*)(base + ws.srt_cls), ws.Scratch(base), stream));
+  if (after_prepass != nullptr) cudaEventRecord(after_prepass, stream);
+  bp.logits = (const R*)x.p;
+  bp.tstride = x.tstride;
+  if (path == kPathGeneric) CTCX_LAUNCH(ctcx::LaunchBeamGeneric(bp, stream));
+  else if constexpr (sizeof(R) == 8) CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, stream));  // (no float64 wide kernel)
+  else if (path == kPathNarrow) CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, x.in_dtype, stream));
+  else CTCX_LAUNCH(ctcx::LaunchBeamWide(bp, x.in_dtype, stream));
+  return CTCX_OK;
+}
+
+// Trace-back of the top paths over the first seq_len[b] frames, then the sparse offsets and sizes and the
+// status words into the result block.
+int TraceScanFlags(const Workspace& ws, unsigned char* base, const int* seq_len, int T, int B, int W, int P,
+                   int merge_repeated, int blank_label, cudaEvent_t after_trace, cudaStream_t stream) {
+  ctcx::TraceParams tp;
+  tp.bp = base + ws.bp; tp.seq_len = seq_len;
+  tp.fin_kind = (const int*)(base + ws.fin_kind); tp.fin_n = (const int*)(base + ws.fin_n);
+  tp.T = T; tp.B = B; tp.W = W; tp.P = P;
+  tp.merge_repeated = merge_repeated ? 1 : 0; tp.blank_label = blank_label;
+  tp.dec_len = (int*)(base + ws.dec_len); tp.dec = (int*)(base + ws.dec);
+  tp.ali_len = (int*)(base + ws.ali_len); tp.ali = (int*)(base + ws.ali);
+  ctcx::ScanParams sp;
+  sp.dec_len = tp.dec_len; sp.ali_len = tp.ali_len; sp.B = B; sp.P = P;
+  sp.dec_off = (long long*)(base + ws.dec_off); sp.ali_off = (long long*)(base + ws.ali_off);
+  sp.sizes = (long long*)(base + ws.result);
+  return FromLaunch(ctcx::LaunchTraceScanFlags(tp, ws.rec_bytes, sp, (const int*)(base + ws.flags),
+                                               (int*)(base + ws.stats), stream, after_trace));
+}
+
+// The sparse outputs from the dense rows a decode left in the workspace, through the pointer table at
+// ws.ptrs. `skip`: optional device word, non-zero = write nothing.
+int Pack(const Workspace& ws, const unsigned char* base, int T, int B, int P, void* log_prob, const int* skip,
+         int real_bytes, cudaStream_t stream) {
+  ctcx::PackParams pp;
+  pp.dec_len = (const int*)(base + ws.dec_len); pp.dec = (const int*)(base + ws.dec);
+  pp.ali_len = (const int*)(base + ws.ali_len); pp.ali = (const int*)(base + ws.ali);
+  pp.dec_off = (const long long*)(base + ws.dec_off); pp.ali_off = (const long long*)(base + ws.ali_off);
+  pp.sizes = (const long long*)(base + ws.result);
+  pp.fin_total = (const void*)(base + ws.fin_total);
+  pp.ptrs = (long long* const*)(base + ws.ptrs);
+  pp.log_prob = log_prob;
+  pp.skip = skip;
+  pp.real_bytes = real_bytes;
+  pp.T = T; pp.B = B; pp.P = P;
+  return FromLaunch(ctcx::LaunchPack(pp, stream));
+}
+
 template <typename R>
 int DecodeImpl(const void* logits_dev, int T, int B, int C, const int32_t* seq_len_dev, int W,
                int P, int merge_repeated, int blank_index, int blank_label, void* workspace,
                size_t workspace_bytes, void* stream_v, ctcx_sizes* sizes, int32_t* flags_out,
                const DecodeOpts& opt) {
-  constexpr bool kF32 = (sizeof(R) == 4);
   cudaStream_t stream = (cudaStream_t)stream_v;
   // --- validation, in the reference's order (kernels.cc:111-138), then TopPaths' (decoder.h:237) ---
   if (T == 0) return CTCX_ERR_MAX_TIME_ZERO;
@@ -237,8 +360,7 @@ int DecodeImpl(const void* logits_dev, int T, int B, int C, const int32_t* seq_l
   if (workspace == nullptr || workspace_bytes < ws.bytes || ((uintptr_t)workspace & 255u))
     return CTCX_ERR_WORKSPACE;
   unsigned char* base = (unsigned char*)workspace;
-  long long* d_sizes = (long long*)(base + ws.result);
-  int* d_stats = (int*)(base + ws.result + 4 * (size_t)P * 8);
+  int* d_stats = (int*)(base + ws.stats);
   int* d_ctrl = (int*)(base + ws.ctrl);
 
   // sequence_length lives on the device: its range check (kernels.cc:134-138) is folded into the
@@ -248,7 +370,7 @@ int DecodeImpl(const void* logits_dev, int T, int B, int C, const int32_t* seq_l
   Workspace::Header hdr = {kMagic, T, B, C, W, P, (int)sizeof(R)};
   {
     // the control words are not part of this copy when a host->device feed owns them (opt.ready)
-    InitBlock init(ws, hdr, B, P);
+    InitBlock init(ws, hdr, B);
     const size_t n = (opt.ready != nullptr) ? ws.ctrl : ws.dec_len;
     CTCX_CUDA(cudaMemcpyAsync(base, init.bytes.data(), n, cudaMemcpyHostToDevice, stream));
     if (opt.ready != nullptr) CTCX_CUDA(cudaMemsetAsync(d_ctrl, 0, 4, stream));  // the queue word only
@@ -270,114 +392,50 @@ int DecodeImpl(const void* logits_dev, int T, int B, int C, const int32_t* seq_l
 
   if (B > 0) {
     ProfRecord(0, stream);
-    ctcx::BeamParamsT<R> bp;
-    std::memset(&bp, 0, sizeof(bp));
-    bp.logits = (const R*)logits_dev;
-    bp.off = (const R*)(base + ws.off);
-    bp.seq_len = seq_len_dev;
-    bp.T = T; bp.B = B; bp.C = C; bp.W = W; bp.P = P;
-    bp.blank_index = blank_index;
-    if (ws.rec_bytes == 4) bp.bp32 = (unsigned*)(base + ws.bp); else bp.bp = (uint2*)(base + ws.bp);
-    bp.fin_total = (R*)(base + ws.fin_total);
-    bp.fin_kind = (int*)(base + ws.fin_kind);
-    bp.fin_n = (int*)(base + ws.fin_n);
-    bp.flags = (int*)(base + ws.flags);
-    bp.Tcap = T;  // one-shot decode: t_done / state stay null
+    const Path path = PathOf<R>(W, C, opt.lm != nullptr);
+    ctcx::BeamParamsT<R> bp = BeamParamsOf<R>(ws, base, T, B, C, W, P, blank_index, seq_len_dev);
     bp.lm = (const R*)opt.lm;
-    bp.tstride = tstride;
-    bp.queue = d_ctrl;
+    bp.ready = opt.ready;
     bp.dbg_cycles = g_dbg_cycles;
-    bp.n_slices = 1;
-    bp.slice_frames = T;
-    if constexpr (kF32) {
-      const Path path = PathOf(W, C, opt.lm != nullptr);
-      int in_dtype = opt.in_dtype;
-      if (path == kPathGeneric && in_dtype != ctcx::kInF32) {
-        // half-precision logits on the generic path: exact upcast into the workspace scratch
-        if (ctcx::NarrowFastShape(W, C) || ctcx::WideFastShape(W, C)) return CTCX_ERR_UNSUPPORTED;  // (forced generic: no scratch)
-        CTCX_LAUNCH(ctcx::LaunchUpcast(logits_dev, in_dtype, (float*)(base + ws.scratch), T, B, C, tstride, stream));
-        bp.logits = (const float*)(base + ws.scratch);
-        bp.tstride = (long long)B * C;
-        in_dtype = ctcx::kInF32;
-      }
-      if (path == kPathNarrow) {
-        bp.ready = opt.ready;
-        // time-sliced work queue (large batches): per-utterance state block + progress words (the regions
-        // the streaming entries use for the same purpose between calls)
-        bp.state = base + ws.state;
-        bp.progress = (int*)(base + ws.t_done);
-        CTCX_CUDA(cudaMemsetAsync(bp.progress, 0, (size_t)B * 4, stream));
-        ProfRecord(1, stream);
-        CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, in_dtype, stream));
-      } else if (path == kPathWide && opt.n_slabs == 0) {
-        // wide vocabulary: normaliser and candidate classes in one pass over the logits
-        bp.srt_pl = (const float*)(base + ws.srt_pl);
-        bp.srt_cls = (const unsigned short*)(base + ws.srt_cls);
-        CTCX_LAUNCH(ctcx::LaunchNormTopClasses(logits_dev, in_dtype, (float*)(base + ws.off), (long long)T * B, C,
-                                               blank_index, W, (float*)(base + ws.srt_pl),
-                                               (unsigned short*)(base + ws.srt_cls), B, tstride, stream));
-        ProfRecord(1, stream);
-        CTCX_LAUNCH(ctcx::LaunchBeamWide(bp, in_dtype, stream));
-      } else if (path == kPathWide && opt.n_slabs > 0) {
-        // Host feed of a wide-vocabulary batch: the copy (hundreds of MB) takes longer than the decode, so
-        // the decode runs time chunk by time chunk behind it -- plain stream order, one event per slab. The
-        // beam crosses chunks through the per-utterance state block, exactly as in a streamed decode
-        // (ctcx_stream_step_f32); the class-selection arrays are chunk-relative and stay in L2.
-        const size_t es = (in_dtype == ctcx::kInF32) ? 4 : 2;
-        int* d_chunk_len = (int*)(base + ws.chunk_len);
-        bp.srt_pl = (const float*)(base + ws.srt_pl);
-        bp.srt_cls = (const unsigned short*)(base + ws.srt_cls);
-        bp.seq_len = d_chunk_len;
-        bp.t_done = (int*)(base + ws.t_done);
-        bp.state = base + ws.state;
-        CTCX_CUDA(cudaMemsetAsync(bp.t_done, 0, (size_t)B * 4, stream));
-        ProfRecord(1, stream);
-        int t0 = 0;
-        for (int k = 0; k < opt.n_slabs; ++k) {
-          const int len = opt.slab_end[k] - t0;
-          const unsigned char* chunk = (const unsigned char*)logits_dev + (size_t)t0 * (size_t)tstride * es;
-          CTCX_CUDA(cudaStreamWaitEvent(stream, opt.slab_event[k], 0));
-          CTCX_LAUNCH(ctcx::LaunchChunkLen(seq_len_dev, B, T, t0, len, d_chunk_len, stream));
-          CTCX_LAUNCH(ctcx::LaunchNormTopClasses(chunk, in_dtype, (float*)(base + ws.off), (long long)len * B, C,
-                                                 blank_index, W, (float*)(base + ws.srt_pl),
-                                                 (unsigned short*)(base + ws.srt_cls), B, tstride, stream));
-          bp.logits = (const float*)chunk;
-          bp.T = len;
-          bp.slice_frames = len;
-          CTCX_LAUNCH(ctcx::LaunchBeamWide(bp, in_dtype, stream));
-          t0 = opt.slab_end[k];
-        }
-        bp.seq_len = seq_len_dev;
-      } else {
-        CTCX_LAUNCH(ctcx::LaunchLogNorm(bp.logits, (float*)(base + ws.off), (long long)T * B, C, B, bp.tstride, stream));
-        ProfRecord(1, stream);
-        CTCX_LAUNCH(ctcx::LaunchBeamGeneric(bp, stream));
-      }
-    } else if (PathOf(W, C, false) == kPathNarrow) {
-      // float64 logits, narrow vocabulary: the fast kernel computing in double (normaliser inside)
-      bp.ready = opt.ready;
+    const Logits x = {logits_dev, opt.in_dtype, tstride};
+    if (path == kPathWide && opt.n_slabs > 0) {
+      // Host feed of a wide-vocabulary batch: the copy (hundreds of MB) takes longer than the decode, so
+      // the decode runs time chunk by time chunk behind it -- plain stream order, one event per slab. The
+      // beam crosses chunks through the per-utterance state block, exactly as in a streamed decode
+      // (ctcx_stream_step_f32); the class-selection arrays are chunk-relative and stay in L2.
+      const size_t es = (x.in_dtype == ctcx::kInF32) ? 4 : 2;
+      int* d_chunk_len = (int*)(base + ws.chunk_len);
+      bp.seq_len = d_chunk_len;
+      bp.t_done = (int*)(base + ws.t_done);
+      bp.state = base + ws.state;
+      CTCX_CUDA(cudaMemsetAsync(bp.t_done, 0, (size_t)B * 4, stream));
       ProfRecord(1, stream);
-      CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, stream));
+      int t0 = 0;
+      for (int k = 0; k < opt.n_slabs; ++k) {
+        const int len = opt.slab_end[k] - t0;
+        CTCX_CUDA(cudaStreamWaitEvent(stream, opt.slab_event[k], 0));
+        CTCX_LAUNCH(ctcx::LaunchChunkLen(seq_len_dev, B, T, t0, len, d_chunk_len, stream));
+        bp.T = len;
+        const Logits chunk = {(const unsigned char*)x.p + (size_t)t0 * (size_t)tstride * es, x.in_dtype, tstride};
+        CTCX_RC(BeamPass(path, chunk, bp, ws, base, nullptr, stream));
+        t0 = opt.slab_end[k];
+      }
     } else {
-      CTCX_LAUNCH(ctcx::LaunchLogNorm((const double*)logits_dev, (double*)(base + ws.off), (long long)T * B, C, B,
-                                      tstride, stream));
-      ProfRecord(1, stream);
-      CTCX_LAUNCH(ctcx::LaunchBeamGeneric(bp, stream));
+      if constexpr (sizeof(R) == 4) {
+        if (path == kPathNarrow) {
+          // time-sliced work queue (large batches): per-utterance state block + progress words (the regions
+          // the streaming entries use for the same purpose between calls); the float64 kernel takes whole
+          // utterances
+          bp.state = base + ws.state;
+          bp.progress = (int*)(base + ws.t_done);
+          CTCX_CUDA(cudaMemsetAsync(bp.progress, 0, (size_t)B * 4, stream));
+        }
+      }
+      CTCX_RC(BeamPass(path, x, bp, ws, base, g_profile ? g_ev[1] : nullptr, stream));
     }
     ProfRecord(2, stream);
-
-    ctcx::TraceParams tp;
-    tp.bp = base + ws.bp; tp.seq_len = seq_len_dev; tp.fin_kind = bp.fin_kind;
-    tp.fin_n = bp.fin_n; tp.T = T; tp.B = B; tp.W = W; tp.P = P;
-    tp.merge_repeated = merge_repeated ? 1 : 0; tp.blank_label = blank_label;
-    tp.dec_len = (int*)(base + ws.dec_len); tp.dec = (int*)(base + ws.dec);
-    tp.ali_len = (int*)(base + ws.ali_len); tp.ali = (int*)(base + ws.ali);
-    ctcx::ScanParams sp;
-    sp.dec_len = tp.dec_len; sp.ali_len = tp.ali_len; sp.B = B; sp.P = P;
-    sp.dec_off = (long long*)(base + ws.dec_off); sp.ali_off = (long long*)(base + ws.ali_off);
-    sp.sizes = d_sizes;
-    CTCX_LAUNCH(ctcx::LaunchTraceScanFlags(tp, ws.rec_bytes, sp, bp.flags, d_stats, stream,
-                                           g_profile ? g_ev[3] : nullptr));
+    CTCX_RC(TraceScanFlags(ws, base, seq_len_dev, T, B, W, P, merge_repeated, blank_label,
+                           g_profile ? g_ev[3] : nullptr, stream));
     ProfRecord(4, stream);
   }
 
@@ -409,18 +467,7 @@ int PackImpl(const void* workspace, int T, int B, int P, int64_t* const* decoded
   CTCX_CUDA(cudaMemcpyAsync(wbase + ws.ptrs, table.data(), table.size() * sizeof(void*),
                             cudaMemcpyHostToDevice, stream));
   if (B > 0) {
-    ctcx::PackParams pp;
-    pp.dec_len = (const int*)(base + ws.dec_len); pp.dec = (const int*)(base + ws.dec);
-    pp.ali_len = (const int*)(base + ws.ali_len); pp.ali = (const int*)(base + ws.ali);
-    pp.dec_off = (const long long*)(base + ws.dec_off); pp.ali_off = (const long long*)(base + ws.ali_off);
-    pp.sizes = (const long long*)(base + ws.result);
-    pp.fin_total = (const void*)(base + ws.fin_total);
-    pp.ptrs = (long long* const*)(base + ws.ptrs);
-    pp.log_prob = log_probability;
-    pp.skip = nullptr;
-    pp.real_bytes = real_bytes;
-    pp.T = T; pp.B = B; pp.P = P;
-    CTCX_LAUNCH(ctcx::LaunchPack(pp, stream));
+    CTCX_RC(Pack(ws, base, T, B, P, log_probability, nullptr, real_bytes, stream));
   } else {
     // empty batch: shapes [0, 0]
     const long long zeros[2] = {0, 0};
@@ -666,7 +713,7 @@ int ctcx_decode_hostin(const void* logits_host, int dtype, int64_t host_time_str
 
   // overlap needs a truly asynchronous copy (page-locked source) and the stream-ordered flag store;
   // pageable sources are staged by the driver, which may wait for the kernel that waits for them
-  const bool overlap = (B > 0) && PathOf(W, C, false) == kPathNarrow && P <= W &&
+  const bool overlap = (B > 0) && PathOf<float>(W, C, false) == kPathNarrow && P <= W &&
                        IsPinned(logits_host) && StreamWriteValue32() != nullptr;
   Feed feed = {(const unsigned char*)logits_host, (unsigned char*)staging_dev, (size_t)B * C * es,
                (size_t)hstride * es, T, d_ctrl + 1, overlap, copy_stream};
@@ -679,7 +726,7 @@ int ctcx_decode_hostin(const void* logits_host, int dtype, int64_t host_time_str
   int slab_end[kMaxSlabs];
   cudaEvent_t slab_event[kMaxSlabs] = {};
   int n_slabs = 0;
-  if (B > 0 && dtype != CTCX_F64 && PathOf(W, C, false) == kPathWide && P <= W && IsPinned(logits_host) &&
+  if (B > 0 && dtype != CTCX_F64 && PathOf<float>(W, C, false) == kPathWide && P <= W && IsPinned(logits_host) &&
       T >= 2 * kMinSlabFrames) {
     n_slabs = std::min(kMaxSlabs, T / kMinSlabFrames);
     for (int k = 0; k < n_slabs; ++k) slab_end[k] = (int)(((long long)T * (k + 1)) / n_slabs);
@@ -755,22 +802,10 @@ int ctcx_pack_compact(void* workspace, int T, int B, int P, int real_bytes, int6
   unsigned char* base = (unsigned char*)workspace;
   Workspace ws;
   ws.InitPack(T, B, P);
-  int* d_stats = (int*)(base + ws.result + 4 * (size_t)P * 8);
+  int* overflow = (int*)(base + ws.stats) + 6;
   CTCX_LAUNCH(ctcx::LaunchPackTable((const long long*)(base + ws.result), B, P, real_bytes, (long long*)packed_dev,
-                                    (unsigned long long)packed_elems, (long long**)(base + ws.ptrs), d_stats + 6, stream));
-  ctcx::PackParams pp;
-  pp.dec_len = (const int*)(base + ws.dec_len); pp.dec = (const int*)(base + ws.dec);
-  pp.ali_len = (const int*)(base + ws.ali_len); pp.ali = (const int*)(base + ws.ali);
-  pp.dec_off = (const long long*)(base + ws.dec_off); pp.ali_off = (const long long*)(base + ws.ali_off);
-  pp.sizes = (const long long*)(base + ws.result);
-  pp.fin_total = (const void*)(base + ws.fin_total);
-  pp.ptrs = (long long* const*)(base + ws.ptrs);
-  pp.log_prob = nullptr;
-  pp.skip = d_stats + 6;
-  pp.real_bytes = real_bytes;
-  pp.T = T; pp.B = B; pp.P = P;
-  CTCX_LAUNCH(ctcx::LaunchPack(pp, stream));
-  return CTCX_OK;
+                                    (unsigned long long)packed_elems, (long long**)(base + ws.ptrs), overflow, stream));
+  return Pack(ws, base, T, B, P, nullptr, overflow, real_bytes, stream);
 }
 
 /* Completes a decode that was enqueued with sizes == NULL: one device->host copy of the sizes and the
@@ -983,7 +1018,7 @@ int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int T_total, int 
     return CTCX_ERR_WORKSPACE;
   unsigned char* base = (unsigned char*)workspace;
   Workspace::Header hdr = {kMagic, T_total, B, C, W, P, 4};
-  InitBlock init(ws, hdr, B, P);
+  InitBlock init(ws, hdr, B);
   CTCX_CUDA(cudaMemcpyAsync(base, init.bytes.data(), ws.dec_len, cudaMemcpyHostToDevice, stream));
   if (B > 0) {
     // decoder.h:212-227: with zero frames consumed the kernels start from the root; TopPaths before
@@ -1010,43 +1045,14 @@ int ctcx_stream_step_f32(void* workspace, int T_total, int B, int C, int W, int 
   Workspace ws;
   ws.Init(T_total, B, C, W, P);
   unsigned char* base = (unsigned char*)workspace;
-  int* d_ctrl = (int*)(base + ws.ctrl);
-  ctcx::BeamParams bp;
-  std::memset(&bp, 0, sizeof(bp));
-  bp.logits = logits_dev;
-  bp.off = (const float*)(base + ws.off);
-  bp.seq_len = chunk_len_dev;  // frames of THIS chunk to consume, per utterance
-  bp.T = chunk_time; bp.B = B; bp.C = C; bp.W = W; bp.P = P;
-  bp.blank_index = blank_index;
-  if (ws.rec_bytes == 4) bp.bp32 = (unsigned*)(base + ws.bp); else bp.bp = (uint2*)(base + ws.bp);
-  bp.fin_total = (float*)(base + ws.fin_total);
-  bp.fin_kind = (int*)(base + ws.fin_kind);
-  bp.fin_n = (int*)(base + ws.fin_n);
-  bp.flags = (int*)(base + ws.flags);
-  bp.Tcap = T_total;
+  ctcx::BeamParams bp = BeamParamsOf<float>(ws, base, T_total, B, C, W, P, blank_index,
+                                            chunk_len_dev);  // frames of THIS chunk to consume, per utterance
+  bp.T = chunk_time;
   bp.t_done = (int*)(base + ws.t_done);
   bp.state = base + ws.state;
-  bp.tstride = (long long)B * C;
-  bp.queue = d_ctrl;
-  bp.dbg_cycles = nullptr;
-  bp.n_slices = 1;
-  bp.slice_frames = chunk_time;
-  const Path path = PathOf(W, C, false);
-  if (path == kPathNarrow) {
-    CTCX_CUDA(cudaMemsetAsync(d_ctrl, 0, 4, stream));
-    CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, ctcx::kInF32, stream));
-  } else if (path == kPathWide) {
-    bp.srt_pl = (const float*)(base + ws.srt_pl);
-    bp.srt_cls = (const unsigned short*)(base + ws.srt_cls);
-    CTCX_LAUNCH(ctcx::LaunchNormTopClasses(logits_dev, ctcx::kInF32, (float*)(base + ws.off), (long long)chunk_time * B,
-                                           C, blank_index, W, (float*)(base + ws.srt_pl),
-                                           (unsigned short*)(base + ws.srt_cls), B, bp.tstride, stream));
-    CTCX_LAUNCH(ctcx::LaunchBeamWide(bp, ctcx::kInF32, stream));
-  } else {
-    CTCX_LAUNCH(ctcx::LaunchLogNorm(logits_dev, (float*)(base + ws.off), (long long)chunk_time * B, C, B, bp.tstride, stream));
-    CTCX_LAUNCH(ctcx::LaunchBeamGeneric(bp, stream));
-  }
-  return CTCX_OK;
+  const Path path = PathOf<float>(W, C, false);
+  if (path == kPathNarrow) CTCX_CUDA(cudaMemsetAsync(bp.queue, 0, 4, stream));  // the queue word, zero at launch
+  return BeamPass(path, Logits{logits_dev, ctcx::kInF32, (long long)B * C}, bp, ws, base, nullptr, stream);
 }
 
 int ctcx_stream_top_paths(void* workspace, int T_total, int B, int C, int W, int P, int merge_repeated,
@@ -1058,31 +1064,16 @@ int ctcx_stream_top_paths(void* workspace, int T_total, int B, int C, int W, int
   Workspace ws;
   ws.Init(T_total, B, C, W, P);
   unsigned char* base = (unsigned char*)workspace;
-  std::vector<unsigned char> h_res(4 * (size_t)P * 8 + kNStats * 4, 0);
-  int* h_stats = (int*)(h_res.data() + 4 * (size_t)P * 8);
-  h_stats[0] = 0;
-  for (int k = 1; k < 6; ++k) h_stats[k] = B;
+  std::vector<unsigned char> h_res(ResultBytes(P), 0);
+  InitStats((int*)(h_res.data() + StatsOffset(P)), B);
   if (B > 0) {
     CTCX_CUDA(cudaMemcpyAsync(base + ws.result, h_res.data(), h_res.size(), cudaMemcpyHostToDevice, stream));
-    ctcx::TraceParams tp;
-    tp.bp = base + ws.bp;
-    tp.seq_len = (const int*)(base + ws.t_done);  // frames consumed so far
-    tp.fin_kind = (const int*)(base + ws.fin_kind);
-    tp.fin_n = (const int*)(base + ws.fin_n);
-    tp.T = T_total; tp.B = B; tp.W = W; tp.P = P;
-    tp.merge_repeated = merge_repeated ? 1 : 0; tp.blank_label = blank_label;
-    tp.dec_len = (int*)(base + ws.dec_len); tp.dec = (int*)(base + ws.dec);
-    tp.ali_len = (int*)(base + ws.ali_len); tp.ali = (int*)(base + ws.ali);
-    ctcx::ScanParams sp;
-    sp.dec_len = tp.dec_len; sp.ali_len = tp.ali_len; sp.B = B; sp.P = P;
-    sp.dec_off = (long long*)(base + ws.dec_off); sp.ali_off = (long long*)(base + ws.ali_off);
-    sp.sizes = (long long*)(base + ws.result);
-    CTCX_LAUNCH(ctcx::LaunchTraceScanFlags(tp, ws.rec_bytes, sp, (const int*)(base + ws.flags),
-                                           (int*)(base + ws.result + 4 * (size_t)P * 8), stream, nullptr));
+    CTCX_RC(TraceScanFlags(ws, base, (const int*)(base + ws.t_done) /* frames consumed so far */, T_total, B, W, P,
+                           merge_repeated, blank_label, nullptr, stream));
     CTCX_CUDA(cudaMemcpyAsync(h_res.data(), base + ws.result, h_res.size(), cudaMemcpyDeviceToHost, stream));
     CTCX_CUDA(cudaStreamSynchronize(stream));
   }
-  return ReportSizes((const long long*)h_res.data(), h_stats, B, T_total, P, sizes, flags_out);
+  return ParseResult(h_res.data(), T_total, B, P, sizes, flags_out);
 }
 
 /* ---- measurement and test hooks (declared at the end of include/ctcx.h) ---- */
@@ -1102,9 +1093,9 @@ void ctcx_debug_set_cycles_buffer(long long* dev_buf) { g_dbg_cycles = dev_buf; 
  * the independent second implementation the parity tests compare with the fast ones. */
 void ctcx_debug_set_beam_impl(int impl) { g_force_generic.store(impl == 1 ? 1 : 0); }
 
-/* The normaliser pre-pass of a decode on its own, through the launchers the decode calls: route 0 the
- * generic path's (LaunchLogNorm; half inputs upcast first), route 1 the wide path's fused normaliser
- * and sorted-class list (LaunchNormTopClasses). */
+/* The normaliser pre-pass of a decode on its own: the decode's own PrePass, route 0 as the generic path
+ * runs it (LaunchLogNorm; half inputs upcast first), route 1 as the wide path does (the fused normaliser
+ * and sorted-class list, LaunchNormTopClasses). */
 int ctcx_debug_prepass(int route, const void* logits_dev, int in_dtype, int T, int B, int C, long long tstride,
                        int blank_index, int beam_width, void* off_dev, float* srt_pl_dev, uint16_t* srt_cls_dev,
                        int* ks_out, void* stream_v) {
@@ -1113,28 +1104,27 @@ int ctcx_debug_prepass(int route, const void* logits_dev, int in_dtype, int T, i
   if (T < 1 || B < 1 || C < 1 || C > kMaxClasses || blank_index < 0 || blank_index >= C ||
       tstride < (long long)B * C || ElemBytes(in_dtype) == 0 || logits_dev == nullptr || off_dev == nullptr)
     return CTCX_ERR_BAD_ARGUMENT;
-  const long long rows = (long long)T * B;
+  Logits x = {logits_dev, InDtypeOf(in_dtype), tstride};
   if (route == 0) {
     if (ks_out) *ks_out = 0;
     if (in_dtype == CTCX_F64)
-      return FromLaunch(ctcx::LaunchLogNorm((const double*)logits_dev, (double*)off_dev, rows, C, B, tstride, stream));
-    if (in_dtype == CTCX_F32)
-      return FromLaunch(ctcx::LaunchLogNorm((const float*)logits_dev, (float*)off_dev, rows, C, B, tstride, stream));
+      return PrePass<double>(kPathGeneric, x, T, B, C, blank_index, beam_width, (double*)off_dev, nullptr, nullptr,
+                             nullptr, stream);
+    // half inputs are widened into scratch of the hook's own (a decode has it in its workspace)
+    const bool half = (in_dtype != CTCX_F32);
     float* scratch = nullptr;
-    CTCX_CUDA(cudaMallocAsync((void**)&scratch, (size_t)rows * C * sizeof(float), stream));
-    int rc = FromLaunch(ctcx::LaunchUpcast(logits_dev, InDtypeOf(in_dtype), scratch, T, B, C, tstride, stream));
-    if (rc == CTCX_OK)
-      rc = FromLaunch(ctcx::LaunchLogNorm(scratch, (float*)off_dev, rows, C, B, (long long)B * C, stream));
-    if (!Check(cudaFreeAsync(scratch, stream), "cudaFreeAsync") && rc == CTCX_OK) rc = CTCX_ERR_CUDA;
+    if (half) CTCX_CUDA(cudaMallocAsync((void**)&scratch, (size_t)T * B * C * sizeof(float), stream));
+    int rc = PrePass<float>(kPathGeneric, x, T, B, C, blank_index, beam_width, (float*)off_dev, nullptr, nullptr,
+                            scratch, stream);
+    if (half && !Check(cudaFreeAsync(scratch, stream), "cudaFreeAsync") && rc == CTCX_OK) rc = CTCX_ERR_CUDA;
     return rc;
   }
   if (route != 1) return CTCX_ERR_BAD_ARGUMENT;
   if (in_dtype == CTCX_F64 || beam_width < 1 || !ctcx::WideFastShape(beam_width, C)) return CTCX_ERR_UNSUPPORTED;
   if (srt_pl_dev == nullptr || srt_cls_dev == nullptr) return CTCX_ERR_BAD_ARGUMENT;
   if (ks_out) *ks_out = ctcx::WideKs(beam_width, C);
-  return FromLaunch(ctcx::LaunchNormTopClasses(logits_dev, InDtypeOf(in_dtype), (float*)off_dev, rows, C, blank_index,
-                                               beam_width, srt_pl_dev, (unsigned short*)srt_cls_dev, B, tstride,
-                                               stream));
+  return PrePass<float>(kPathWide, x, T, B, C, blank_index, beam_width, (float*)off_dev, srt_pl_dev,
+                        (unsigned short*)srt_cls_dev, nullptr, stream);
 }
 
 /* y = f(x) element-wise with the exact device math; op 0 expf, 1 log1pf, 2 logf, 3 LogSumExp(x, 0),

@@ -38,6 +38,12 @@ int WideKs(int W, int C);  // row stride of the sorted arrays
 // 4-byte back-pointer records when every slot and label fits in a byte
 inline int RecBytes(int W, int C) { return (W <= 256 && C <= 256) ? 4 : 8; }
 
+// ---- shared by the launchers ----
+constexpr int kListCapMax = 4608;  // candidate-list entries kept in shared memory (8 B each)
+// beam tier (slots per CTA) of the fast kernels' instantiations
+inline int TierOf(int W) { return (W <= 32) ? 32 : (W <= 128) ? 128 : 256; }
+int SmCount();  // multiprocessors of the current device (cached per device)
+
 // ---- kernel 1 ----
 LaunchStatus LaunchLogNorm(const float* logits, float* off, long long rows, int C, int B, long long tstride,
                            cudaStream_t stream);
@@ -54,8 +60,8 @@ LaunchStatus LaunchUpcast(const void* in, int in_dtype, float* out, int T, int B
 LaunchStatus LaunchBeamNarrow(BeamParams& p, int in_dtype, cudaStream_t stream);
 LaunchStatus LaunchBeamNarrow(BeamParamsT<double>& p, cudaStream_t stream);  // float64 logits, double scores
 LaunchStatus LaunchBeamWide(BeamParams& p, int in_dtype, cudaStream_t stream);
-LaunchStatus LaunchBeamGeneric(BeamParamsT<float>& p, cudaStream_t stream);
-LaunchStatus LaunchBeamGeneric(BeamParamsT<double>& p, cudaStream_t stream);
+template <typename R>  // float or double scores
+LaunchStatus LaunchBeamGeneric(BeamParamsT<R>& p, cudaStream_t stream);
 
 // ---- kernels 3-5 ----
 // trace-back of the top paths, then per-path offsets / sizes and the reduction of the per-utterance

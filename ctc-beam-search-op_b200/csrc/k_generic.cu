@@ -10,15 +10,6 @@
 namespace ctcx {
 
 namespace {
-constexpr int kListCapMax = 4608;  // candidate-list entries kept in shared memory (8 B each)
-
-int SmCount() {
-  int sm_count = 148, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-  return sm_count;
-}
-
 struct Tier {
   int wmax, nt;
 };
@@ -93,42 +84,33 @@ LaunchStatus LaunchUpcast(const void* in, int in_dtype, float* out, int T, int B
 }
 
 // kernel 2, generic form
-LaunchStatus LaunchBeamGeneric(BeamParamsT<float>& bp, cudaStream_t stream) {
-  const int W = bp.W, C = bp.C;
-  bp.kid_words = (C + 31) / 32;
-  const long long full_list = (long long)W * C;
-  bp.cand_cap = (full_list <= kListCapMax) ? (int)full_list : 0;
-  const Tier tier = PickTier(W);
-  BeamSmem lay;
-  lay.Init(tier.wmax, tier.nt, C, bp.kid_words, bp.cand_cap, 4, W);
-  if (lay.bytes > 220 * 1024) return {kLaunchUnsupported, cudaSuccess, ""};
-  switch (tier.wmax) {
-    case 32: return LaunchOne<float, 32, 128>(bp, lay.bytes, stream);
-    case 128: return LaunchOne<float, 128, 256>(bp, lay.bytes, stream);
-    case 256: return LaunchOne<float, 256, 256>(bp, lay.bytes, stream);
-    default: return LaunchOne<float, 1024, 1024>(bp, lay.bytes, stream);
-  }
-}
-
-// T = double: the generic kernel instantiated for double scores (64-bit keys)
-LaunchStatus LaunchBeamGeneric(BeamParamsT<double>& bp, cudaStream_t stream) {
+template <typename R>
+LaunchStatus LaunchBeamGeneric(BeamParamsT<R>& bp, cudaStream_t stream) {
+  constexpr bool kF64 = (sizeof(R) == 8);
   const int W = bp.W, C = bp.C;
   bp.kid_words = (C + 31) / 32;
   const long long full_list = (long long)W * C;
   bp.cand_cap = (full_list <= kListCapMax) ? (int)full_list : 0;
   // double state is twice as wide: the largest tier that fits in shared memory holds 512 slots
   Tier tier = PickTier(W);
-  if (tier.wmax > 256) tier = (W <= 512) ? Tier{512, 512} : Tier{1024, 1024};
+  if (kF64 && tier.wmax > 256) tier = (W <= 512) ? Tier{512, 512} : Tier{1024, 1024};
   BeamSmem lay;
-  lay.Init(tier.wmax, tier.nt, C, bp.kid_words, bp.cand_cap, 8, W);
-  if (lay.bytes > 220 * 1024) return {kLaunchUnsupported, cudaSuccess, ""};  // beam_width > 512, or a very wide vocabulary
+  lay.Init(tier.wmax, tier.nt, C, bp.kid_words, bp.cand_cap, (int)sizeof(R), W);
+  // (double: beam_width > 512, or a very wide vocabulary)
+  if (lay.bytes > 220 * 1024) return {kLaunchUnsupported, cudaSuccess, ""};
   switch (tier.wmax) {
-    case 32: return LaunchOne<double, 32, 128>(bp, lay.bytes, stream);
-    case 128: return LaunchOne<double, 128, 256>(bp, lay.bytes, stream);
-    case 256: return LaunchOne<double, 256, 256>(bp, lay.bytes, stream);
-    case 512: return LaunchOne<double, 512, 512>(bp, lay.bytes, stream);
-    default: return {kLaunchUnsupported, cudaSuccess, ""};
+    case 32: return LaunchOne<R, 32, 128>(bp, lay.bytes, stream);
+    case 128: return LaunchOne<R, 128, 256>(bp, lay.bytes, stream);
+    case 256: return LaunchOne<R, 256, 256>(bp, lay.bytes, stream);
+  }
+  if constexpr (kF64) {
+    if (tier.wmax == 512) return LaunchOne<double, 512, 512>(bp, lay.bytes, stream);
+    return {kLaunchUnsupported, cudaSuccess, ""};
+  } else {
+    return LaunchOne<float, 1024, 1024>(bp, lay.bytes, stream);
   }
 }
+template LaunchStatus LaunchBeamGeneric<float>(BeamParamsT<float>& bp, cudaStream_t stream);
+template LaunchStatus LaunchBeamGeneric<double>(BeamParamsT<double>& bp, cudaStream_t stream);
 
 }  // namespace ctcx

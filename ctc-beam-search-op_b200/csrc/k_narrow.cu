@@ -4,11 +4,6 @@
 
 namespace ctcx {
 
-namespace {
-constexpr int kListCapMax = 4608;  // candidate-list entries kept in shared memory (8 B each)
-
-int TierOf(int W) { return (W <= 32) ? 32 : (W <= 128) ? 128 : 256; }
-
 int SmCount() {
   static int cached[64] = {0};
   int dev = 0, sms = 148;
@@ -19,6 +14,7 @@ int SmCount() {
   return sms;
 }
 
+namespace {
 // Launch configuration of one kernel instantiation on one device, computed once: the attribute and
 // occupancy queries cost tens of microseconds of host time that would otherwise sit between the
 // kernels of every decode. (A cache of immutable facts about the device, not decoder state.)
@@ -115,6 +111,15 @@ size_t SmemBytes(int wmax, int cand_cap, bool lm, bool f64 = false) {  // (the s
     default: return BeamSmemV4<256>::Bytes(cand_cap) + extra;
   }
 }
+
+// the preconditions both score types share, and the fields they derive; false = not this kernel's
+template <typename R>
+bool PrepareNarrow(BeamParamsT<R>& p) {
+  if (!NarrowFastShape(p.W, p.C) || p.queue == nullptr || p.bp32 == nullptr) return false;
+  p.cand_cap = p.W * p.C;
+  p.kid_words = 1;
+  return true;
+}
 }  // namespace
 
 bool NarrowFastShape(int W, int C) {
@@ -123,11 +128,8 @@ bool NarrowFastShape(int W, int C) {
 }
 
 LaunchStatus LaunchBeamNarrow(BeamParams& p, int in_dtype, cudaStream_t stream) {
-  if (!NarrowFastShape(p.W, p.C) || p.queue == nullptr || p.bp32 == nullptr) return {kLaunchUnsupported, cudaSuccess, ""};
-  p.cand_cap = p.W * p.C;
-  p.kid_words = 1;
+  if (!PrepareNarrow(p) || (p.lm != nullptr && in_dtype != kInF32)) return {kLaunchUnsupported, cudaSuccess, ""};
   const int wmax = TierOf(p.W);
-  if (p.lm != nullptr && in_dtype != kInF32) return {kLaunchUnsupported, cudaSuccess, ""};
   const size_t smem = SmemBytes(wmax, p.cand_cap, p.lm != nullptr);
   switch (in_dtype) {
     case kInF32: return LaunchTyped<float>(p, wmax, smem, stream);
@@ -137,16 +139,9 @@ LaunchStatus LaunchBeamNarrow(BeamParams& p, int in_dtype, cudaStream_t stream) 
   }
 }
 
-}  // namespace ctcx
-
-namespace ctcx {
-
 // float64 logits (the op's T = double registration): the same kernel computing in double, 64-bit keys
 LaunchStatus LaunchBeamNarrow(BeamParamsT<double>& p, cudaStream_t stream) {
-  if (!NarrowFastShape(p.W, p.C) || p.queue == nullptr || p.bp32 == nullptr || p.lm != nullptr)
-    return {kLaunchUnsupported, cudaSuccess, ""};
-  p.cand_cap = p.W * p.C;
-  p.kid_words = 1;
+  if (!PrepareNarrow(p) || p.lm != nullptr) return {kLaunchUnsupported, cudaSuccess, ""};
   p.state = nullptr;  // no time slices: whole utterances from the queue
   p.t_done = nullptr;
   const int wmax = TierOf(p.W);

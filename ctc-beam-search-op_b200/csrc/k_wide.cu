@@ -9,14 +9,6 @@
 namespace ctcx {
 
 namespace {
-int TierOf(int W) { return (W <= 32) ? 32 : (W <= 128) ? 128 : 256; }
-int SmCount() {
-  int sm_count = 148, dev = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sm_count, cudaDevAttrMultiProcessorCount, dev);
-  return sm_count;
-}
-
 template <typename IN, int NI>
 LaunchStatus TopClassesNI(const void* logits, float* off, long long rows, int C, int blank, int Ke, int Ks,
                           float* srt_pl, unsigned short* srt_cls, int B, long long tstride, cudaStream_t stream) {

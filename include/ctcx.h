@@ -304,8 +304,8 @@ int ctcx_debug_math_f32(int op, const float* x_dev, float* y_dev, int n, void* s
 int ctcx_debug_math_f64(int op, const double* x_dev, double* y_dev, int n, void* stream);
 
 /* The softmax-normaliser pre-pass of a decode, run alone on the T*B rows of a [T, B, C] tensor of
- * element type `in_dtype` (CTCX_F32 ... ; time stride `tstride` elements, 0 = B*C) with the launchers
- * the decode uses. off_dev[T*B] (double for CTCX_F64, float otherwise) receives max + log(sum exp).
+ * element type `in_dtype` (CTCX_F32 ... ; time stride `tstride` elements, 0 = B*C) through the same
+ * pre-pass function a decode calls. off_dev[T*B] (double for CTCX_F64, float otherwise) receives max + log(sum exp).
  * route 0: the generic path's normaliser (half inputs are upcast to float32 first).
  * route 1: the wide path's fused pre-pass (32 < C <= 2048, shapes the wide kernel takes, not CTCX_F64):
  *   also srt_pl_dev / srt_cls_dev[T*B, *ks_out] receive per row the first min(C-1, 2*beam_width+3)

@@ -63,6 +63,185 @@ def test_cabi_validation_without_device(lib):
     assert lib.ctcx_decode_f32(*args(5, 1, 3, 5000, 1, 0)) == 9  # beyond this build's limits
     assert lib.ctcx_decode_f32(*args(5, 1, 3, 2, 1, 0)) == 10    # no workspace
 
+    # Every other entry that validates before touching a device pointer. All device pointers are
+    # null: a call that got past its checks would return 10 (no workspace), never dereference one.
+    sz, fl = ctypes.byref(sizes), None
+    view = lambda dt, ts, T, B, C, W, P, blank: lib.ctcx_decode_view(  # noqa: E731
+        None, dt, ts, T, B, C, None, W, P, 0, blank, -1, None, 0, None, sz, fl)
+    assert view(7, 0, 5, 1, 3, 2, 1, 0) == 8          # no such dtype (before max_time)
+    assert view(7, 0, 0, 1, 3, 2, 1, 0) == 8
+    assert view(0, -1, 5, 1, 3, 2, 1, 0) == 8         # negative time stride
+    assert view(2, 0, 0, 1, 3, 2, 1, 0) == 2
+    assert view(3, 0, 0, 1, 3, 2, 1, 0) == 2
+    assert view(1, 0, 5, -1, 3, 2, 1, 0) == 8         # negative batch
+    assert view(0, 0, 5, 1, 0, 2, 1, 0) == 8          # no classes
+    assert view(3, 0, 5, 1, 3, 2, 0, 0) == 8          # top_paths < 1
+    assert view(2, 0, 5, 1, 3, 2, 1, -1) == 8         # negative blank
+    assert view(0, 0, 5, 1, 70000, 2, 1, 0) == 9      # more classes than this build takes
+    assert view(3, 0, 5, 1, 3, 1025, 1, 0) == 9
+    assert view(0, 5, 5, 2, 3, 2, 1, 0) == 8          # stride shorter than a frame (B * C = 6)
+    assert view(0, 6, 5, 2, 3, 2, 1, 0) == 10
+    assert view(3, 0, 5, 0, 3, 2, 1, 0) == 10         # an empty batch still needs its workspace
+    assert view(1, 0, 5, 1, 3, 1, 2, 0) == 10         # top_paths > beam_width: reported on the device
+    half = lambda dt, T, W, blank: lib.ctcx_decode_half(  # noqa: E731
+        None, dt, None, T, 1, 3, None, W, 1, 0, blank, -1, None, 0, None, sz, fl)
+    assert half(2, 0, 2, 0) == 2                      # unknown half type: max_time is checked first
+    assert half(2, 5, 2, 0) == 8
+    assert half(-1, 5, 2, 0) == 8
+    assert half(0, 0, 2, 0) == 2
+    assert half(1, 5, 0, 0) == 8
+    assert half(0, 5, 2, 3) == 8
+    assert half(1, 5, 2000, 0) == 9
+    assert half(0, 5, 2, 0) == 10
+    f64 = lambda T, C, W, P, blank: lib.ctcx_decode_f64(  # noqa: E731
+        None, T, 1, C, None, W, P, 0, blank, -1, None, 0, None, sz, fl)
+    assert f64(0, 3, 2, 1, 0) == 2
+    assert f64(-1, 3, 2, 1, 0) == 8
+    assert f64(5, 3, 2, 1, 3) == 8
+    assert f64(5, 65536, 2, 1, 0) == 9
+    assert f64(5, 3, 2, 1, 0) == 10
+    scorer = lambda T, C, W, blank: lib.ctcx_decode_scorer_f32(  # noqa: E731  (no table: the plain decode)
+        None, T, 1, C, None, W, 1, 0, blank, -1, None, None, 0, None, sz, fl)
+    assert scorer(0, 3, 2, 0) == 2
+    assert scorer(5, 3, 0, 0) == 8
+    assert scorer(5, 3, 2, 5) == 8
+    assert scorer(5, 3, 4096, 0) == 9
+    assert scorer(5, 3, 2, 0) == 10
+    hostin = lambda dt, ts, T, B, C, W, P, blank: lib.ctcx_decode_hostin(  # noqa: E731
+        None, dt, ts, T, B, C, None, W, P, 0, blank, -1, None, 0, None, 0, None, None, sz, fl)
+    assert hostin(9, 0, 0, 1, 3, 2, 1, 0) == 2        # max_time before the dtype here
+    assert hostin(9, 0, 5, 1, 3, 2, 1, 0) == 8
+    assert hostin(3, 0, 5, 1, 3, 0, 1, 0) == 8
+    assert hostin(0, 0, 5, 1, 3, 2, 1, 3) == 8
+    assert hostin(1, 0, 5, 1, 3, 1025, 1, 0) == 9
+    assert hostin(0, 2, 5, 1, 3, 2, 1, 0) == 8        # host stride shorter than a frame
+    assert hostin(0, 0, 5, 1, 3, 2, 1, 0) == 10       # workspace before staging, host pointers and streams
+    assert hostin(2, 9, 5, 3, 3, 2, 5, 0) == 10
+    reset = lambda T, B, C, W, P: lib.ctcx_stream_reset(None, 0, T, B, C, W, P, None)  # noqa: E731
+    assert reset(0, 1, 3, 2, 1) == 8
+    assert reset(5, -1, 3, 2, 1) == 8
+    assert reset(5, 1, 0, 2, 1) == 8
+    assert reset(5, 1, 3, 2, 0) == 8
+    assert reset(5, 1, 3, 1025, 1) == 9
+    assert reset(5, 1, 65536, 2, 1) == 9
+    assert reset(5, 1, 3, 2, 3) == 6                  # top_paths > beam_width, before the workspace
+    assert reset(5, 1, 3, 2, 1) == 10
+    assert reset(5, 0, 3, 2, 1) == 10
+    # the stream step and top_paths check the workspace before their arguments
+    assert lib.ctcx_stream_step_f32(None, 0, 1, 3, 2, 1, None, 0, None, 9, None) == 10
+    assert lib.ctcx_stream_step_f32(None, 5, 1, 3, 5000, 1, None, 1, None, 0, None) == 10
+    assert lib.ctcx_stream_top_paths(None, 0, 1, 3, 2, 1, 0, -1, None, sz, fl) == 10
+    assert lib.ctcx_stream_top_paths(None, 5, 1, 3, 5000, 1, 0, -1, None, None, fl) == 10
+    nul6 = [None] * 6
+    for pack in (lib.ctcx_pack_f32, lib.ctcx_pack_f64):
+        for T, B, P in ((5, 1, 1), (0, 1, 1), (5, -1, 1), (5, 1, 0), (5, 0, 1)):
+            assert pack(None, T, B, P, *nul6, None, None) == 10
+    for T, B, P, rb in ((5, 1, 1, 4), (5, 1, 1, 8), (5, 1, 1, 2), (0, 1, 1, 4), (5, 0, 1, 4), (5, 1, 0, 8)):
+        assert lib.ctcx_pack_compact(None, T, B, P, rb, None, 0, None) == 10
+    for T, B, P in ((5, 1, 1), (0, 1, 1), (5, -1, 1), (5, 1, 0), (5, 0, 1)):
+        assert lib.ctcx_finish(None, T, B, P, None, sz, fl) == 10
+        assert lib.ctcx_result_copy_async(None, T, B, P, None, 0, None) == 10
+    buf = ctypes.create_string_buffer(1024)
+    assert lib.ctcx_finish(None, 5, 1, 1, None, None, fl) == 10
+    assert lib.ctcx_result_copy_async(None, 5, 1, 1, buf, 1024, None) == 10
+    prep = lambda route, dt, T, B, C, ts, blank, W: lib.ctcx_debug_prepass(  # noqa: E731
+        route, None, dt, T, B, C, ts, blank, W, None, None, None, None, None)
+    for route in (0, 1, 2):
+        assert prep(route, 0, 2, 2, 40, 0, 0, 4) == 8    # no logits
+        assert prep(route, 0, 0, 2, 40, 0, 0, 4) == 8
+        assert prep(route, 3, 2, 2, 40, 0, 40, 4) == 8
+        assert prep(route, 5, 2, 2, 40, 0, 0, 4) == 8
+        assert prep(route, 1, 2, 2, 40, 79, 0, 4) == 8
+        assert prep(route, 2, 2, 2, 70000, 0, 0, 4) == 8
+
+
+# ctcx_workspace_bytes at shapes on both sides of every route and tier edge: the layout is part of the
+# ABI (a caller sizes its buffer from it), so these values do not change without a reason.
+WORKSPACE_BYTES = [
+    # narrow: beam tiers 32 / 128 / 256, the 4608-entry candidate list (32 x 144), C = 1, 2
+    ((50, 8, 29, 10, 3), 36352), ((50, 8, 32, 32, 1), 72448), ((50, 8, 32, 33, 2), 77568),
+    ((50, 8, 29, 128, 4), 265984), ((50, 8, 29, 129, 1), 258816), ((50, 8, 16, 256, 1), 502528),
+    ((50, 8, 16, 257, 1), 941312), ((50, 8, 32, 144, 1), 287488), ((50, 8, 32, 145, 1), 340736),
+    ((20, 3, 2, 1024, 7), 623616), ((10, 2, 1, 1, 1), 5120), ((1, 1, 3, 1, 1), 5120),
+    # wide: C = 33 and 2048 / 2049, beam tiers
+    ((40, 4, 33, 1, 1), 15360), ((40, 4, 33, 32, 2), 64256), ((40, 4, 33, 33, 1), 64000),
+    ((40, 4, 1000, 128, 1), 831232), ((40, 4, 1000, 129, 3), 835072), ((40, 4, 2048, 8, 1), 41472),
+    ((40, 4, 2048, 256, 2), 1687296), ((40, 4, 2048, 257, 1), 1687552), ((40, 4, 2049, 8, 1), 1329920),
+    # generic: beams up to 1024, C up to 65535, empty batches, a beam beyond the limits
+    ((7, 3, 300, 512, 5), 178176), ((7, 3, 300, 513, 1), 177920), ((7, 3, 300, 1024, 1024), 687616),
+    ((6, 2, 65535, 8, 2), 3151872), ((6, 2, 65535, 1024, 1), 3330816), ((6, 2, 5000, 100, 3), 262656),
+    ((10, 0, 29, 10, 1), 1024), ((10, 0, 5000, 300, 2), 1024), ((5, 1, 3, 5000, 1), 405248),
+]
+
+
+def test_workspace_bytes_table(lib):
+    for shape, want in WORKSPACE_BYTES:
+        assert lib.ctcx_workspace_bytes(*shape) == want, shape
+        assert lib.ctcx_stream_workspace_bytes(*shape) == want, shape
+    for bad in ((5, -1, 3, 2, 1), (5, 1, 0, 2, 1), (5, 1, 3, 0, 1), (5, 1, 3, 2, 0)):
+        assert lib.ctcx_workspace_bytes(*bad) == 0
+    assert [lib.ctcx_result_bytes(p) for p in (0, 1, 3)] == [0, 96, 160]
+
+
+def _result_block(P, sizes, stats):
+    """A result block as ctcx_result_copy_async delivers it: sizes [4, P] int64, then 16 status words."""
+    blk = np.zeros(4 * P * 2 + 8, np.int64)
+    blk[:4 * P] = np.asarray(sizes, np.int64).reshape(-1)
+    st = blk[4 * P:].view(np.int32)
+    st[:len(stats)] = stats
+    return blk
+
+
+def test_result_parse(lib):
+    """ctcx_result_parse reads the status words in a fixed order, then copies the sizes out."""
+    from ctc_beam_search_op_b200 import _lib
+    T, B, P = 9, 5, 3
+    sz = [[7, 0, 12], [4, 0, 6], [40, 40, 33], [9, 9, 8]]
+    ok = [0x3, B, B, B, B, B]
+
+    def parse(stats, P=P, flags=True, fields=(0, 1, 2, 3)):
+        blk = _result_block(P, sz if P == 3 else [[0] * P] * 4, stats)
+        got = [np.full(P, -7, np.int64) for _ in range(4)]
+        ptr = lambda a: a.ctypes.data_as(_lib._i64p)  # noqa: E731
+        s = _lib.CtcxSizes(*[ptr(got[k]) if k in fields else None for k in range(4)])
+        f = ctypes.c_int32(-7)
+        rc = lib.ctcx_result_parse(blk.ctypes.data, T, B, P, ctypes.byref(s), ctypes.byref(f) if flags else None)
+        return rc, [g.tolist() for g in got], f.value
+
+    rc, got, f = parse(ok)
+    assert rc == 0 and got == sz and f == 3
+    rc, got, _ = parse(ok, flags=False, fields=(1, 3))
+    assert rc == 0 and got == [[-7] * 3, sz[1], [-7] * 3, sz[3]]
+    assert parse([0, 1, B, B, B, B], P=1)[0] == 7  # P = 1 layout: status words right after 4 sizes
+    # one failing status word at a time, and which of two wins
+    assert parse(ok + [1])[0] == 10                               # compact pack: the buffer was too small
+    assert parse([0, 0, 0, 0, 0, 0, 1])[0] == 10                  # ... before everything else
+    rc = parse([0, B, B, B, B, 3])[0]                             # the input copy never delivered b = 3
+    assert rc == 11 and "utterance 3" in lib.ctcx_last_cuda_error().decode()
+    assert parse([0, 0, 0, 0, 0, 2])[0] == 11
+    rc = parse([0, B, 2, B, B, B])[0]                             # sequence_length(2) > T
+    assert rc == 5 and lib.ctcx_error_batch_index() == 2
+    assert lib.ctcx_strerror(5).decode() == "sequence_length(2) <= 9"
+    rc = parse([0, 0, 4, 0, 0, B])[0]
+    assert rc == 5 and lib.ctcx_error_batch_index() == 4
+    assert parse([0, B, B, 1, B, B])[0] == 8                      # negative sequence_length
+    assert parse([0, 0, B, 1, 0, B])[0] == 8
+    rc = parse([0, B, B, B, 3, B])[0]                             # stream fed past its frames
+    assert rc == 5 and lib.ctcx_error_batch_index() == 3
+    rc = parse([0, 0, B, B, 1, B])[0]
+    assert rc == 5 and lib.ctcx_error_batch_index() == 1
+    rc, got, f = parse([1, 0, B, B, B, B])                        # too few leaves
+    assert rc == 7 and got == [[-7] * 3] * 4 and f == -7
+    # argument errors
+    blk = _result_block(P, sz, ok)
+    s = _lib.CtcxSizes()
+    assert lib.ctcx_result_parse(None, T, B, P, ctypes.byref(s), None) == 8
+    assert lib.ctcx_result_parse(blk.ctypes.data, T, B, P, None, None) == 8
+    assert lib.ctcx_result_parse(blk.ctypes.data, 0, B, P, ctypes.byref(s), None) == 8
+    assert lib.ctcx_result_parse(blk.ctypes.data, T, -1, P, ctypes.byref(s), None) == 8
+    assert lib.ctcx_result_parse(blk.ctypes.data, T, B, 0, ctypes.byref(s), None) == 8
+    assert lib.ctcx_result_parse(blk.ctypes.data, T, 0, P, ctypes.byref(s), None) == 0  # empty batch
+
 
 def test_python_host_validation_order():
     import ctc_beam_search_op_b200 as op
