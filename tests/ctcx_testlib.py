@@ -389,7 +389,8 @@ def paper_logits(dtype=np.float64):
 MODEL_SRC = os.path.join(ROOT, "tests", "model", "ctcx_model.cc")
 MODEL_SO = os.path.join(ROOT, "tests", "model", "libctcx_model.so")
 MODEL_STATS = ("frames cands at_risk fp_iters fp_iters_max wiped wiped_with_cands anomalies cands_max "
-               "frames_wipe_matters queries radix_bits_sum").split()
+               "frames_wipe_matters queries radix_bits_sum fp_unwipes wiped_parents frames_at_risk "
+               "suspects_dropped").split()
 
 
 def build_model(force=False):
@@ -417,6 +418,36 @@ def model_decode(logits, seq_len, beam_width, top_paths, merge_repeated=False, b
                            7: "Less leaves in the beam search than requested."}.get(rc, "error %d" % rc))
     res = DenseResult(B, top_paths, T, dec_len, dec, ali_len, ali, logp)
     return (res, dict(zip(MODEL_STATS, st.tolist()))) if want_stats else res
+
+
+MODEL_VARIANTS = {"exact": 0, "count_wiped_rows": 1, "four_rounds": 2}
+
+
+def model_decode_utts(logits, seq_len, beam_width, top_paths, merge_repeated=False, blank_index=0,
+                      blank_label=-1, variant="exact"):
+    """model_decode with the statistics of every utterance: (DenseResult, [dict per utterance],
+    int32 [B, T] rounds of the revisit-wipe fixed point per frame, 0 where nobody is at risk).
+    variant: "exact", or a fixed point with a known mistake -- "count_wiped_rows" (the candidates of
+    wiped rows still count) or "four_rounds" (stops after 4 rounds) -- to show that a case exposes it."""
+    build_model()
+    lib = _load(MODEL_SO)
+    logits, seq_len = _check_inputs(logits, seq_len)
+    logits = logits.astype(np.float32, copy=False)
+    T, B, C = logits.shape
+    dec_len, dec, ali_len, ali, logp = _dense_out(B, top_paths, T, np.float32)
+    st = np.zeros((max(B, 1), 16), np.int64)
+    iters = np.zeros((max(B, 1), T), np.int32)
+    rc = lib.ctcx_model_decode_utts_f32(_ptr(logits, _c_float_p), T, B, C, _ptr(seq_len, _c_int_p),
+                                        beam_width, top_paths, int(bool(merge_repeated)), blank_index,
+                                        blank_label, _ptr(dec_len, _c_int_p), _ptr(dec, _c_int_p),
+                                        _ptr(ali_len, _c_int_p), _ptr(ali, _c_int_p), _ptr(logp, _c_float_p),
+                                        None, st.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)),
+                                        _ptr(iters, _c_int_p), MODEL_VARIANTS[variant])
+    if rc != 0:
+        raise OracleError({2: "max_time is 0", 6: "requested more paths than the beam width.",
+                           7: "Less leaves in the beam search than requested."}.get(rc, "error %d" % rc))
+    res = DenseResult(B, top_paths, T, dec_len, dec, ali_len, ali, logp)
+    return res, [dict(zip(MODEL_STATS, row)) for row in st[:B].tolist()], iters[:B]
 
 
 def same_result(a, b, bitwise=True):
@@ -476,3 +507,31 @@ class Golden:
             x = np.asarray(rows, np.float32)[:, None, :]
             out.append((name, x, np.asarray([sl], np.int32), W, P, merge, blank, bl))
         return out
+
+
+# ----------------------------------------------------------------------------------------------
+# Revisit-wipe cases found by a search on the CPU model (tests/golden/make_wipe_cases.py)
+WIPE_NPZ = os.path.join(ROOT, "tests", "golden", "wipe_cases.npz")
+
+
+class WipeCase:
+    """One utterance of wipe_cases.npz: logits k/16 (float32, [T, 1, C]), decode attributes, and the
+    model's statistics (dict over MODEL_STATS) and fixed-point rounds per frame recorded for it."""
+
+    def __init__(self, arr, name):
+        k = arr[name + "/k"]
+        self.name = name
+        self.x = np.where(k == -32768, -np.inf, k.astype(np.float32) / 16).astype(np.float32)[:, None, :]
+        self.T, _, self.C = self.x.shape
+        self.W, self.blank, merge, self.P, exposes = (int(v) for v in arr[name + "/attrs"])
+        self.merge = bool(merge)
+        # the mistaken fixed point (a model_decode_utts variant) under which this case decodes differently
+        self.exposes = {v: k for k, v in MODEL_VARIANTS.items()}[exposes] if exposes else None
+        self.stats = dict(zip(MODEL_STATS, arr[name + "/stats"].tolist()))
+        self.iters = arr[name + "/iters"].astype(np.int32)
+        self.sl = np.array([self.T], np.int32)
+
+
+def wipe_cases():
+    arr = np.load(WIPE_NPZ)
+    return [WipeCase(arr, str(n)) for n in arr["names"]]

@@ -21,7 +21,11 @@ const float kNegInf = -INFINITY;
 
 struct Stats {
   long long frames, cands, at_risk, fp_iters, fp_iters_max, wiped, wiped_with_cands, anomalies,
-      cands_max, frames_wipe_matters, queries, radix_bits_sum;
+      cands_max, frames_wipe_matters, queries, radix_bits_sum,
+      fp_unwipes,        // verdicts that flip from wiped back to kept in a later round of the fixed point
+      wiped_parents,     // at-risk members whose parent is wiped in the final verdict
+      frames_at_risk,    // frames with at least one at-risk member
+      suspects_dropped;  // members whose parent's re-score beats their own total and that leave the beam
 };
 
 inline float Lse(float a, float b) {  // util/ctc_loss_util.h:33-41
@@ -56,8 +60,13 @@ struct Cand {
   unsigned char an_kind;
 };
 
+// Variants of the revisit-wipe fixed point with a known mistake, for the test fixture: a case that
+// guards against the mistake must decode differently under it (tests/golden/make_wipe_cases.py).
+enum { kExact = 0, kCountWipedRows = 1, kFourRounds = 2 };
+
 struct Beam {
   int W, C, blank, blank_label;
+  int variant = kExact;
   int n;
   std::vector<float> total, blk, lab, ab, an;
   std::vector<int> label;
@@ -75,7 +84,8 @@ struct Beam {
     bp.clear();
   }
 
-  void Step(const float* x, Stats* st) {
+  // Returns the rounds the revisit-wipe fixed point ran in this frame (the last one changes nothing).
+  int Step(const float* x, Stats* st) {
     // decoder.h:71-80
     float mx = x[0];
     for (int j = 1; j < C; ++j) mx = x[j] > mx ? x[j] : mx;
@@ -181,13 +191,16 @@ struct Beam {
           int cnt = 0;
           const int end_full = row_begin[b];
           for (int k = 0; k < end_full; ++k)
-            if (!wiped[cands[k].row] && cands[k].s > nt[m]) ++cnt;
+            if ((variant == kCountWipedRows || !wiped[cands[k].row]) && cands[k].s > nt[m]) ++cnt;
           for (int k = row_begin[b]; k < row_begin[b + 1]; ++k)
             if (cands[k].label < label[m] && cands[k].s > nt[m]) ++cnt;
           if (rank[m] + cnt >= W) nw[m] = 1;
         }
         if (nw == wiped) break;
+        if (st)
+          for (int m = 0; m < n; ++m) st->fp_unwipes += (wiped[m] && !nw[m]) ? 1 : 0;
         wiped.swap(nw);
+        if (variant == kFourRounds && iters == 4) break;
       }
     }
     if (st) {
@@ -205,6 +218,8 @@ struct Beam {
         if (s > nt[m]) st->anomalies++;
       }
       st->frames_wipe_matters += matters;
+      st->frames_at_risk += at_risk.empty() ? 0 : 1;
+      for (size_t q = 0; q < at_risk.size(); ++q) st->wiped_parents += wiped[pslot[at_risk[q]]] ? 1 : 0;
     }
 
     // (7) stable top-W over members (first, slot order) and live candidates (visiting order)
@@ -215,6 +230,16 @@ struct Beam {
       if (!wiped[cands[k].row]) items.push_back(Item{cands[k].s, n + (int)k});
     std::stable_sort(items.begin(), items.end(), [](const Item& a, const Item& b) { return a.s > b.s; });
     const int n_new = std::min<int>((int)items.size(), W);
+    if (st) {  // the kernels' rounding-anomaly report (DESIGN.md section 8), exactly as the generic kernel decides it
+      std::vector<char> kept(n, 0);
+      for (int k = 0; k < n_new; ++k) if (items[k].idx < n) kept[items[k].idx] = 1;
+      for (int m = 0; m < n; ++m) {
+        const int b = pslot[m];
+        if (b < 0 || kept[m]) continue;
+        const float p = x[label[m]] - off;
+        if (((label[m] == label[b]) ? p + blk[b] : p + total[b]) > nt[m]) st->suspects_dropped++;
+      }
+    }
 
     // (8) write the new beam (sorted) and this frame's back-pointers
     std::vector<float> t2(W, kNegInf), b2(W, kNegInf), l2(W, kNegInf), ab2(W, kNegInf), an2(W, kNegInf);
@@ -240,6 +265,7 @@ struct Beam {
     hash.swap(h2); phash.swap(ph2);
     n = n_new;
     bp.push_back(recs);
+    return iters;
   }
 
   // decoder.h:229-261 + entry.h:123-152, from the back-pointers
@@ -276,18 +302,29 @@ struct Beam {
 
 }  // namespace
 
-extern "C" int ctcx_model_decode_f32(const float* logits, int T, int B, int C, const int* seq_len,
-                                     int W, int P, int merge_repeated, int blank_index,
-                                     int blank_label, int* dec_len, int* dec, int* ali_len, int* ali,
-                                     float* logp, long long* stats_out) {
+// stats_out: the statistics summed over the batch (maxima for *_max); utt_stats_out: optional [B,16],
+// the same per utterance; iters_out: optional [B,T], the fixed-point rounds of every frame (0 past the
+// utterance's length). variant: kExact, or one of the mistaken fixed points above.
+extern "C" int ctcx_model_decode_utts_f32(const float* logits, int T, int B, int C, const int* seq_len,
+                                          int W, int P, int merge_repeated, int blank_index,
+                                          int blank_label, int* dec_len, int* dec, int* ali_len, int* ali,
+                                          float* logp, long long* stats_out, long long* utt_stats_out,
+                                          int* iters_out, int variant) {
+  static_assert(sizeof(Stats) <= 16 * sizeof(long long), "the stats array has 16 slots");
   if (T == 0) return 2;
   for (int b = 0; b < B; ++b) if (!(seq_len[b] <= T)) return 5;
   Stats st; std::memset(&st, 0, sizeof(st));
   Beam beam; beam.W = W; beam.C = C; beam.blank = blank_index; beam.blank_label = blank_label;
+  beam.variant = variant;
   std::vector<int> d, a;
   for (int b = 0; b < B; ++b) {
+    Stats us; std::memset(&us, 0, sizeof(us));
     beam.Reset();
-    for (int t = 0; t < seq_len[b]; ++t) beam.Step(logits + ((size_t)t * B + b) * C, &st);
+    for (int t = 0; t < seq_len[b]; ++t) {
+      const int it = beam.Step(logits + ((size_t)t * B + b) * C, &us);
+      if (iters_out) iters_out[(size_t)b * T + t] = it;
+    }
+    if (iters_out) for (int t = seq_len[b]; t < T; ++t) iters_out[(size_t)b * T + t] = 0;
     if (P > W) return 6;
     if (P > beam.n) return 7;
     for (int p = 0; p < P; ++p) {
@@ -298,7 +335,26 @@ extern "C" int ctcx_model_decode_f32(const float* logits, int T, int B, int C, c
       for (size_t i = 0; i < d.size(); ++i) dec[row * T + i] = d[i];
       for (size_t i = 0; i < a.size(); ++i) ali[row * T + i] = a[i];
     }
+    if (utt_stats_out) {
+      std::memset(utt_stats_out + (size_t)b * 16, 0, 16 * sizeof(long long));
+      std::memcpy(utt_stats_out + (size_t)b * 16, &us, sizeof(us));
+    }
+    const long long iters_max = std::max(st.fp_iters_max, us.fp_iters_max);
+    const long long cands_max = std::max(st.cands_max, us.cands_max);
+    long long* acc = reinterpret_cast<long long*>(&st);
+    const long long* u = reinterpret_cast<const long long*>(&us);
+    for (size_t i = 0; i < sizeof(Stats) / sizeof(long long); ++i) acc[i] += u[i];
+    st.fp_iters_max = iters_max;
+    st.cands_max = cands_max;
   }
   if (stats_out) std::memcpy(stats_out, &st, sizeof(st));
   return 0;
+}
+
+extern "C" int ctcx_model_decode_f32(const float* logits, int T, int B, int C, const int* seq_len,
+                                     int W, int P, int merge_repeated, int blank_index,
+                                     int blank_label, int* dec_len, int* dec, int* ali_len, int* ali,
+                                     float* logp, long long* stats_out) {
+  return ctcx_model_decode_utts_f32(logits, T, B, C, seq_len, W, P, merge_repeated, blank_index, blank_label,
+                                    dec_len, dec, ali_len, ali, logp, stats_out, nullptr, nullptr, kExact);
 }
