@@ -34,6 +34,7 @@ EXPORTS = ("ctcx_strerror", "ctcx_last_cuda_error", "ctcx_error_batch_index", "c
            "ctcx_decode_half", "ctcx_decode_view", "ctcx_hostin_staging_bytes", "ctcx_decode_hostin",
            "ctcx_pack_f32", "ctcx_pack_f64", "ctcx_pack_compact", "ctcx_finish", "ctcx_result_bytes", "ctcx_result_copy_async", "ctcx_result_parse", "ctcx_decode_host_f32", "ctcx_decode_host_f64", "ctcx_free_host",
            "ctcx_stream_workspace_bytes", "ctcx_stream_reset", "ctcx_stream_step_f32", "ctcx_stream_top_paths",
+           "ctcx_stream_workspace_bytes_v", "ctcx_stream_reset_v", "ctcx_stream_step_v",
            # measurement and test hooks
            "ctcx_workspace_views", "ctcx_profile_enable", "ctcx_profile_get", "ctcx_debug_set_cycles_buffer",
            "ctcx_debug_set_beam_impl", "ctcx_debug_math_f32", "ctcx_debug_math_f64", "ctcx_debug_prepass")
@@ -109,6 +110,11 @@ def load():
     lib.ctcx_stream_workspace_bytes.argtypes = [ctypes.c_int] * 5
     lib.ctcx_stream_reset.argtypes = [_vp, ctypes.c_size_t] + [ctypes.c_int] * 5 + [_vp]
     lib.ctcx_stream_step_f32.argtypes = [_vp] + [ctypes.c_int] * 5 + [_vp, ctypes.c_int, _vp, ctypes.c_int, _vp]
+    lib.ctcx_stream_workspace_bytes_v.restype = ctypes.c_size_t
+    lib.ctcx_stream_workspace_bytes_v.argtypes = [ctypes.c_int] * 6
+    lib.ctcx_stream_reset_v.argtypes = [_vp, ctypes.c_size_t] + [ctypes.c_int] * 6 + [_vp]
+    lib.ctcx_stream_step_v.argtypes = [_vp, ctypes.c_size_t] + [_i] * 5 + [_vp, _i, ctypes.c_int64, _i, _vp, _i,
+                                                                            _vp, _vp]
     lib.ctcx_stream_top_paths.argtypes = [_vp] + [ctypes.c_int] * 5 + [ctypes.c_int, ctypes.c_int, _vp,
                                                                       ctypes.POINTER(CtcxSizes),
                                                                       ctypes.POINTER(ctypes.c_int32)]

@@ -51,6 +51,8 @@ constexpr int kMaxBeamWidth = 1024;
 constexpr int kMaxClasses = 65535;
 constexpr uint32_t kMagic = 0x43544359u;  // "CTCY": workspace layout of this build
 constexpr int kNStats = 16;
+// control word (Workspace::ctrl) set when a scorer table with a positive entry was passed
+constexpr int kCtrlTablePositive = 8;
 
 size_t Align256(size_t v) { return (v + 255) / 256 * 256; }
 
@@ -113,7 +115,8 @@ struct Workspace {
     ali = o; o += Align256(b * pp * t * 4);
     return o;
   }
-  void Init(int T, int B, int C, int W, int P) {
+  // score_bytes: 8 = room for a float64 stream (the double state blocks after the float ones)
+  void Init(int T, int B, int C, int W, int P, int score_bytes = 4) {
     size_t o = InitPack(T, B, P);
     const size_t b = (size_t)B, t = (size_t)T, w = (size_t)W;
     seq = o; o += Align256(b * 4);                               // sequence_length of host-input decodes
@@ -121,7 +124,6 @@ struct Workspace {
     fin_n = o; o += Align256(b * 4);
     flags = o; o += Align256(b * 4);
     t_done = o; o += Align256(b * 4);                            // streaming: frames consumed so far
-    state = o; o += Align256(b * ctcx::StreamStateBytes(W));     // streaming: beam between chunks
     const bool narrow = ctcx::NarrowFastShape(W, C), wide = ctcx::WideFastShape(W, C);
     off = o; o += Align256(t * b * 8);                           // float or double (unused by the narrow kernel, which normalises itself)
     rec_bytes = ctcx::RecBytes(W, C);
@@ -132,11 +134,14 @@ struct Workspace {
     // shapes served by the generic kernel only: room to upcast half-precision logits (the fast kernels
     // read them directly)
     scratch = o; o += (narrow || wide) ? 0 : Align256(t * b * (size_t)C * 4);
+    // streaming: the beam between chunks (last, so that no other offset depends on the score type)
+    state = o; o += Align256(b * ctcx::StreamStateBytes(W));
+    if (score_bytes == 8) o += Align256(b * ctcx::StreamStateBytes<double>(W));  // at ctcx::StreamState64
     bytes = o;
   }
   // the upcast room, or null where a fast kernel takes the shape (even with the generic kernel forced:
   // the layout does not depend on the test hook)
-  float* Scratch(unsigned char* base) const { return bytes > scratch ? (float*)(base + scratch) : nullptr; }
+  float* Scratch(unsigned char* base) const { return state > scratch ? (float*)(base + scratch) : nullptr; }
 };
 
 thread_local int g_err_batch = -1;
@@ -302,6 +307,22 @@ int BeamPass(Path path, Logits x, ctcx::BeamParamsT<R>& bp, const Workspace& ws,
   else if (path == kPathNarrow) CTCX_LAUNCH(ctcx::LaunchBeamNarrow(bp, x.in_dtype, stream));
   else CTCX_LAUNCH(ctcx::LaunchBeamWide(bp, x.in_dtype, stream));
   return CTCX_OK;
+}
+
+// One Step() of a streamed decode with R scores: up to chunk_len[b] frames of the chunk `x` for every
+// utterance, the beam carried in from and out to the state blocks. `lm`: scorer table (float), or null.
+template <typename R>
+int StreamStep(const Workspace& ws, unsigned char* base, int T_total, int B, int C, int W, int P, const Logits& x,
+               int chunk_time, const int32_t* chunk_len_dev, int blank_index, const float* lm, cudaStream_t stream) {
+  ctcx::BeamParamsT<R> bp = BeamParamsOf<R>(ws, base, T_total, B, C, W, P, blank_index,
+                                            chunk_len_dev);  // frames of THIS chunk to consume, per utterance
+  bp.T = chunk_time;
+  bp.t_done = (int*)(base + ws.t_done);
+  bp.state = base + ws.state;
+  bp.lm = (const R*)lm;
+  const Path path = PathOf<R>(W, C, lm != nullptr);
+  if (path == kPathNarrow) CTCX_CUDA(cudaMemsetAsync(bp.queue, 0, 4, stream));  // the queue word, zero at launch
+  return BeamPass(path, x, bp, ws, base, nullptr, stream);
 }
 
 // Trace-back of the top paths over the first seq_len[b] frames, then the sparse offsets and sizes and the
@@ -644,7 +665,7 @@ int ctcx_decode_scorer_f32(const float* logits_dev, int T, int B, int C, const i
     Workspace ws;
     ws.Init(T > 0 ? T : 1, B > 0 ? B : 0, C, W > 0 ? W : 1, P > 0 ? P : 1);
     if (workspace_bytes < ws.bytes) return CTCX_ERR_WORKSPACE;
-    int* d_flag = (int*)((unsigned char*)workspace + ws.ctrl) + 8;
+    int* d_flag = (int*)((unsigned char*)workspace + ws.ctrl) + kCtrlTablePositive;
     CTCX_CUDA(cudaMemsetAsync(d_flag, 0, 4, stream));
     CTCX_LAUNCH(ctcx::LaunchPositive(expansion_scores_dev, (long long)(C + 1) * C, d_flag, stream));
     int h_flag = 0;
@@ -1006,25 +1027,35 @@ size_t ctcx_stream_workspace_bytes(int max_time_total, int B, int C, int W, int 
   return ctcx_workspace_bytes(max_time_total, B, C, W, P);
 }
 
-int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int T_total, int B, int C, int W, int P,
-                      void* stream_v) {
+size_t ctcx_stream_workspace_bytes_v(int score_dtype, int max_time_total, int B, int C, int W, int P) {
+  if (score_dtype != CTCX_F32 && score_dtype != CTCX_F64) return 0;
+  if (max_time_total <= 0 || B < 0 || C <= 0 || W <= 0 || P <= 0) return 0;
+  Workspace ws;
+  ws.Init(max_time_total, B, C, W, P, (int)ElemBytes(score_dtype));
+  return ws.bytes;
+}
+
+int ctcx_stream_reset_v(void* workspace, size_t workspace_bytes, int score_dtype, int T_total, int B, int C, int W,
+                        int P, void* stream_v) {
   cudaStream_t stream = (cudaStream_t)stream_v;
+  if (score_dtype != CTCX_F32 && score_dtype != CTCX_F64) return CTCX_ERR_BAD_ARGUMENT;
   if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1) return CTCX_ERR_BAD_ARGUMENT;
   if (W > kMaxBeamWidth || C > kMaxClasses) return CTCX_ERR_UNSUPPORTED;
   if (P > W) return CTCX_ERR_TOO_MANY_PATHS;
+  const int score_bytes = (int)ElemBytes(score_dtype);
   Workspace ws;
-  ws.Init(T_total, B, C, W, P);
+  ws.Init(T_total, B, C, W, P, score_bytes);
   if (workspace == nullptr || workspace_bytes < ws.bytes || ((uintptr_t)workspace & 255u))
     return CTCX_ERR_WORKSPACE;
   unsigned char* base = (unsigned char*)workspace;
-  Workspace::Header hdr = {kMagic, T_total, B, C, W, P, 4};
-  InitBlock init(ws, hdr, B);
+  Workspace::Header hdr = {kMagic, T_total, B, C, W, P, score_bytes};
+  InitBlock init(ws, hdr, B);  // (zeroes the control words: no table with a positive entry yet)
   CTCX_CUDA(cudaMemcpyAsync(base, init.bytes.data(), ws.dec_len, cudaMemcpyHostToDevice, stream));
   if (B > 0) {
     // decoder.h:212-227: with zero frames consumed the kernels start from the root; TopPaths before
     // the first Step() sees the root itself: one leaf, log-probability 0 (ln 1), empty sequences
     CTCX_CUDA(cudaMemsetAsync(base + ws.t_done, 0, (size_t)B * 4, stream));
-    CTCX_CUDA(cudaMemsetAsync(base + ws.state, 0, (size_t)B * ctcx::StreamStateBytes(W), stream));
+    CTCX_LAUNCH(ctcx::LaunchStreamReset(base + ws.state, B, W, score_bytes, stream));
     CTCX_CUDA(cudaMemsetAsync(base + ws.fin_total, 0, (size_t)B * P * 8, stream));
     CTCX_CUDA(cudaMemsetAsync(base + ws.fin_kind, 0, (size_t)B * P * 4, stream));
     std::vector<int> ones((size_t)B, 1), fl((size_t)B, (P > 1) ? 2 : 0);  // fewer leaves than top_paths
@@ -1034,25 +1065,46 @@ int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int T_total, int 
   return CTCX_OK;  // (copies from pageable memory are staged before the calls return)
 }
 
-int ctcx_stream_step_f32(void* workspace, int T_total, int B, int C, int W, int P, const float* logits_dev,
-                         int chunk_time, const int32_t* chunk_len_dev, int blank_index, void* stream_v) {
+int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int T_total, int B, int C, int W, int P,
+                      void* stream_v) {
+  return ctcx_stream_reset_v(workspace, workspace_bytes, CTCX_F32, T_total, B, C, W, P, stream_v);
+}
+
+int ctcx_stream_step_v(void* workspace, size_t workspace_bytes, int T_total, int B, int C, int W, int P,
+                       const void* logits_dev, int dtype, int64_t time_stride, int chunk_time,
+                       const int32_t* chunk_len_dev, int blank_index, const float* expansion_scores_dev,
+                       void* stream_v) {
   cudaStream_t stream = (cudaStream_t)stream_v;
   if (workspace == nullptr || ((uintptr_t)workspace & 255u)) return CTCX_ERR_WORKSPACE;
+  if (ElemBytes(dtype) == 0 || time_stride < 0) return CTCX_ERR_BAD_ARGUMENT;
   if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1 || W > kMaxBeamWidth || C > kMaxClasses || P > W ||
       chunk_time <= 0 || chunk_time > T_total || chunk_len_dev == nullptr || blank_index < 0 || blank_index >= C)
     return CTCX_ERR_BAD_ARGUMENT;
-  if (B == 0) return CTCX_OK;
+  const long long tstride = time_stride ? time_stride : (long long)B * C;
+  if (tstride < (long long)B * C) return CTCX_ERR_BAD_ARGUMENT;
+  const bool f64 = (dtype == CTCX_F64);
+  if (f64 && expansion_scores_dev != nullptr) return CTCX_ERR_BAD_ARGUMENT;  // tables hold float32 scores
   Workspace ws;
-  ws.Init(T_total, B, C, W, P);
+  ws.Init(T_total, B, C, W, P, f64 ? 8 : 4);
+  if (workspace_bytes < ws.bytes) return CTCX_ERR_WORKSPACE;
+  if (B == 0) return CTCX_OK;
   unsigned char* base = (unsigned char*)workspace;
-  ctcx::BeamParams bp = BeamParamsOf<float>(ws, base, T_total, B, C, W, P, blank_index,
-                                            chunk_len_dev);  // frames of THIS chunk to consume, per utterance
-  bp.T = chunk_time;
-  bp.t_done = (int*)(base + ws.t_done);
-  bp.state = base + ws.state;
-  const Path path = PathOf<float>(W, C, false);
-  if (path == kPathNarrow) CTCX_CUDA(cudaMemsetAsync(bp.queue, 0, 4, stream));  // the queue word, zero at launch
-  return BeamPass(path, Logits{logits_dev, ctcx::kInF32, (long long)B * C}, bp, ws, base, nullptr, stream);
+  int* d_ctrl = (int*)(base + ws.ctrl);
+  // a table with a positive entry: sticky until the next reset, reported by ctcx_stream_top_paths
+  if (expansion_scores_dev != nullptr)
+    CTCX_LAUNCH(ctcx::LaunchPositive(expansion_scores_dev, (long long)(C + 1) * C, d_ctrl + kCtrlTablePositive, stream));
+  const Logits x = {logits_dev, InDtypeOf(dtype), tstride};
+  return f64 ? StreamStep<double>(ws, base, T_total, B, C, W, P, x, chunk_time, chunk_len_dev, blank_index, nullptr,
+                                  stream)
+             : StreamStep<float>(ws, base, T_total, B, C, W, P, x, chunk_time, chunk_len_dev, blank_index,
+                                 expansion_scores_dev, stream);
+}
+
+int ctcx_stream_step_f32(void* workspace, int T_total, int B, int C, int W, int P, const float* logits_dev,
+                         int chunk_time, const int32_t* chunk_len_dev, int blank_index, void* stream_v) {
+  // (no size argument: the workspace is taken to be the float stream's)
+  return ctcx_stream_step_v(workspace, ctcx_stream_workspace_bytes(T_total, B, C, W, P), T_total, B, C, W, P,
+                            logits_dev, CTCX_F32, 0, chunk_time, chunk_len_dev, blank_index, nullptr, stream_v);
 }
 
 int ctcx_stream_top_paths(void* workspace, int T_total, int B, int C, int W, int P, int merge_repeated,
@@ -1070,6 +1122,9 @@ int ctcx_stream_top_paths(void* workspace, int T_total, int B, int C, int W, int
     CTCX_CUDA(cudaMemcpyAsync(base + ws.result, h_res.data(), h_res.size(), cudaMemcpyHostToDevice, stream));
     CTCX_RC(TraceScanFlags(ws, base, (const int*)(base + ws.t_done) /* frames consumed so far */, T_total, B, W, P,
                            merge_repeated, blank_label, nullptr, stream));
+    // score types mixed since the reset, or a table with a positive entry: CTCX_ERR_BAD_ARGUMENT
+    CTCX_LAUNCH(ctcx::LaunchStreamCheck(base + ws.state, B, W, (const int*)(base + ws.ctrl) + kCtrlTablePositive,
+                                        (int*)(base + ws.stats), stream));
     CTCX_CUDA(cudaMemcpyAsync(h_res.data(), base + ws.result, h_res.size(), cudaMemcpyDeviceToHost, stream));
     CTCX_CUDA(cudaStreamSynchronize(stream));
   }

@@ -349,7 +349,8 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
     }
     const int L = min(Lall, t0 + p.slice_frames) - t0;  // frames of this task
     const bool last_slice = (t0 + L == Lall);
-    const bool resume = (p.state != nullptr) && (t_done > 0 || slice > 0);
+    bool resume = (p.state != nullptr) && (t_done > 0 || slice > 0);
+    if constexpr (kF64) resume = resume && StreamResumable64(p.state, B, W, b);
     const size_t row0 = (size_t)b * C;  // element offset of (t = 0, b) in the logits tensor
     if (slice > 0) {  // wait for the previous slice of this utterance (acquire), then read its state
       if (tid == 0) {
@@ -509,8 +510,8 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
     }
     __syncthreads();
     int carried = 0;  // flag bits handed on from the previous slice / call
-    if constexpr (!kF64) if (resume) {  // beam as the previous slice left it (buffer 0: local frame 0 reads buffer 0)
-      StreamView sv(p.state + (size_t)b * StreamStateBytes(W), W);
+    if (resume) {  // beam as the previous slice left it (buffer 0: local frame 0 reads buffer 0)
+      const StreamViewT<R> sv = StreamBlock<R>(p.state, B, W, b);
       n = __ldcg(&sv.hdr->n);
       carried = __ldcg(&sv.hdr->flags);
       for (int i = tid; i < n; i += NT) {  // (L2 loads: another SM wrote the block)
@@ -1232,8 +1233,8 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
         }
       }
       // ---- carry the beam (and the score-range prediction) to the next slice / the next call ----
-      if constexpr (!kF64) if (p.state != nullptr && (!last_slice || p.t_done != nullptr)) {
-        StreamView sv(p.state + (size_t)b * StreamStateBytes(W), W);
+      if (p.state != nullptr && (!last_slice || p.t_done != nullptr)) {
+        const StreamViewT<R> sv = StreamBlock<R>(p.state, B, W, b);
         for (int i = tid; i < n; i += NT) {
           sv.total[i] = s_total[cur * WMAX + i]; sv.blk[i] = s_blk[cur * WMAX + i];
           sv.lab[i] = s_lab[cur * WMAX + i]; sv.ab[i] = s_ab[cur * WMAX + i];
@@ -1244,6 +1245,10 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
           sv.hdr->n = n;
           sv.hdr->gap = s_keys[kV4KGap];
           sv.hdr->flags = (sci[kV2Anomaly] ? 1 : 0) | overflow | lost | (carried & 4);
+          if constexpr (kF64) {
+            sv.hdr->type = 8;
+            StreamMarkF64Step(p.state, W, b);
+          }
         }
       }
       if (p.t_done != nullptr && tid == 0) p.t_done[b] = t_done + t_end;

@@ -66,6 +66,28 @@ __device__ __forceinline__ unsigned long long HashChild(unsigned long long h, in
   return z;
 }
 
+// Streamed float64 decodes (see StreamHdrT): the double block of utterance b, or null where the double
+// kernel starts from the root -- it resumes only a block that a double kernel wrote after the reset of a
+// float64 stream, so that a stream stepped with both score types never feeds it foreign bytes.
+__device__ __forceinline__ StreamViewT<double> StreamBlock64(unsigned char* state, int B, int W, int b) {
+  return StreamViewT<double>(StreamState64(state, B, W) + (size_t)b * StreamStateBytes<double>(W), W);
+}
+// the block of utterance b that the kernels with R scores carry their beam in
+template <typename R>
+__device__ __forceinline__ StreamViewT<R> StreamBlock(unsigned char* state, int B, int W, int b) {
+  if constexpr (sizeof(R) == 4) return StreamViewT<R>(state + (size_t)b * StreamStateBytes(W), W);
+  else return StreamBlock64(state, B, W, b);
+}
+__device__ __forceinline__ bool StreamResumable64(unsigned char* state, int B, int W, int b) {
+  const StreamView fv(state + (size_t)b * StreamStateBytes(W), W);
+  return __ldcg(&fv.hdr->type) == 8 && __ldcg(&StreamBlock64(state, B, W, b).hdr->type) == 8;
+}
+// after a double kernel saved block b: a float stream gets the mark that ctcx_stream_top_paths reports
+__device__ __forceinline__ void StreamMarkF64Step(unsigned char* state, int W, int b) {
+  const StreamView fv(state + (size_t)b * StreamStateBytes(W), W);
+  if (fv.hdr->type != 8) fv.hdr->type |= kStreamF64Stepped;
+}
+
 // element i of the caller's logits tensor as the decoder's score type (exact: float16 / bfloat16 ->
 // float32 is a widening). The loads bypass L1: the narrow fast kernel may run while a host->device
 // copy of later frames is still in flight (BeamParamsT::ready).
@@ -479,7 +501,7 @@ __global__ void __launch_bounds__(NT) BeamKernelT(BeamParamsT<R> p) {
   using Ops = RealOps<R>;
   using Key = typename Ops::Key;
   using Comp = typename Ops::Comp;
-  constexpr bool kIsF32 = (sizeof(R) == 4);  // streaming state blocks exist for float only
+  constexpr bool kIsF32 = (sizeof(R) == 4);
   extern __shared__ __align__(16) unsigned char smem[];
   constexpr int NWARP = NT / 32;
   constexpr int TS = 2 * WMAX;  // hash-table slots (power of two)
@@ -490,7 +512,8 @@ __global__ void __launch_bounds__(NT) BeamKernelT(BeamParamsT<R> p) {
   // streaming: frames already consumed by earlier chunks; this chunk contributes L more
   const int t_done = (p.t_done != nullptr) ? p.t_done[b] : 0;
   const int L = max(0, min(p.seq_len[b], p.Tcap - t_done));
-  const bool resume = kIsF32 && (p.state != nullptr) && t_done > 0;
+  bool resume = (p.state != nullptr) && t_done > 0;
+  if constexpr (!kIsF32) resume = resume && StreamResumable64(p.state, B, W, b);
 
   BeamSmem lay;
   lay.Init(WMAX, NT, C, KW, p.cand_cap, (int)sizeof(R), W);
@@ -545,17 +568,15 @@ __global__ void __launch_bounds__(NT) BeamKernelT(BeamParamsT<R> p) {
     sci[kScAnomaly] = 0;
   }
   int n = 1;  // members in the beam (uniform across the CTA)
-  if constexpr (kIsF32) {
-    if (resume) {  // beam as the previous chunk left it (buffer 0: local frame 0 reads buffer 0)
-      StreamView sv(p.state + (size_t)b * StreamStateBytes(W), W);
-      n = sv.hdr->n;
-      for (int i = tid; i < n; i += NT) {
-        s_total[i] = sv.total[i]; s_blk[i] = sv.blk[i]; s_lab[i] = sv.lab[i];
-        s_ab[i] = sv.ab[i]; s_an[i] = sv.an[i]; s_label[i] = sv.label[i];
-        s_hash[i] = sv.hash[i]; s_phash[i] = sv.phash[i];
-      }
-      if (tid == 0) sci[kScAnomaly] = sv.hdr->flags & 1;
+  if (resume) {  // beam as the previous chunk left it (buffer 0: local frame 0 reads buffer 0)
+    const StreamViewT<R> sv = StreamBlock<R>(p.state, B, W, b);
+    n = sv.hdr->n;
+    for (int i = tid; i < n; i += NT) {
+      s_total[i] = sv.total[i]; s_blk[i] = sv.blk[i]; s_lab[i] = sv.lab[i];
+      s_ab[i] = sv.ab[i]; s_an[i] = sv.an[i]; s_label[i] = sv.label[i];
+      s_hash[i] = sv.hash[i]; s_phash[i] = sv.phash[i];
     }
+    if (tid == 0) sci[kScAnomaly] = sv.hdr->flags & 1;
   }
   // row 0 of the logits
   if (L > 0) {
@@ -1038,19 +1059,21 @@ __global__ void __launch_bounds__(NT) BeamKernelT(BeamParamsT<R> p) {
       p.fin_n[b] = n;
       p.flags[b] = (sci[kScAnomaly] ? 1 : 0) | ((p.P > n) ? 2 : 0) | overflow;
     }
-    if constexpr (kIsF32) {
-      if (p.state != nullptr) {  // carry the beam to the next chunk
-        StreamView sv(p.state + (size_t)b * StreamStateBytes(W), W);
-        for (int i = tid; i < n; i += NT) {
-          sv.total[i] = s_total[cur * WMAX + i]; sv.blk[i] = s_blk[cur * WMAX + i];
-          sv.lab[i] = s_lab[cur * WMAX + i]; sv.ab[i] = s_ab[cur * WMAX + i];
-          sv.an[i] = s_an[cur * WMAX + i]; sv.label[i] = s_label[cur * WMAX + i];
-          sv.hash[i] = s_hash[cur * WMAX + i]; sv.phash[i] = s_phash[cur * WMAX + i];
-        }
-        if (tid == 0) {
-          sv.hdr->n = n;
-          sv.hdr->gap = 0u;
-          sv.hdr->flags = (sci[kScAnomaly] ? 1 : 0) | overflow | (resume ? (sv.hdr->flags & 4) : 0);
+    if (p.state != nullptr) {  // carry the beam to the next chunk
+      const StreamViewT<R> sv = StreamBlock<R>(p.state, B, W, b);
+      for (int i = tid; i < n; i += NT) {
+        sv.total[i] = s_total[cur * WMAX + i]; sv.blk[i] = s_blk[cur * WMAX + i];
+        sv.lab[i] = s_lab[cur * WMAX + i]; sv.ab[i] = s_ab[cur * WMAX + i];
+        sv.an[i] = s_an[cur * WMAX + i]; sv.label[i] = s_label[cur * WMAX + i];
+        sv.hash[i] = s_hash[cur * WMAX + i]; sv.phash[i] = s_phash[cur * WMAX + i];
+      }
+      if (tid == 0) {
+        sv.hdr->n = n;
+        sv.hdr->gap = 0u;
+        sv.hdr->flags = (sci[kScAnomaly] ? 1 : 0) | overflow | (resume ? (sv.hdr->flags & 4) : 0);
+        if constexpr (!kIsF32) {
+          sv.hdr->type = 8;
+          StreamMarkF64Step(p.state, W, b);
         }
       }
     }

@@ -74,6 +74,11 @@ LaunchStatus LaunchPack(const PackParams& pp, cudaStream_t stream);
 LaunchStatus LaunchPackTable(const long long* sizes, int B, int P, int real_bytes, long long* buf,
                              unsigned long long buf_elems, long long** ptrs, int* overflow, cudaStream_t stream);
 LaunchStatus LaunchPositive(const float* v, long long n, int* flag, cudaStream_t stream);
+// streamed decodes (StreamHdrT): the state blocks of a reset stream with score_bytes (4 or 8) scores, and
+// the check before TopPaths -- stats[3] = 0 (a bad argument) if *table_flag is set or score types were mixed
+LaunchStatus LaunchStreamReset(unsigned char* state, int B, int W, int score_bytes, cudaStream_t stream);
+LaunchStatus LaunchStreamCheck(unsigned char* state, int B, int W, const int* table_flag, int* stats,
+                               cudaStream_t stream);
 // out[b] = frames of utterance b inside the time chunk [t0, t0 + len) (lengths clamped to [0, T])
 LaunchStatus LaunchChunkLen(const int* seq_len, int B, int T, int t0, int len, int* out, cudaStream_t stream);
 LaunchStatus LaunchMathTest(int op, const float* x, float* y, int n, cudaStream_t stream);

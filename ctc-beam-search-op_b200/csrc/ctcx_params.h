@@ -54,30 +54,65 @@ struct BeamParamsT {
 };
 using BeamParams = BeamParamsT<float>;
 
-// Beam state of one utterance between two chunks of a streamed decode.
-struct StreamHdr {
+// Beam state of one utterance between two chunks of a streamed decode, for R scores. A streamed
+// workspace holds [B] float blocks, and for a float64 stream [B] double blocks after them
+// (StreamState64): the float kernels always find a valid beam in their own blocks, whichever score
+// type stepped the stream, and the two header words below tell the type of every step since the reset.
+template <typename R>
+struct StreamHdrT;
+template <>
+struct StreamHdrT<float> {
   int n;         // members in the beam
   unsigned gap;  // score-range prediction of the fast kernel
-  int flags;     // bit0 rounding anomaly, bit2 more frames than the stream was sized for
-  int pad;
+  int flags;     // bit0 rounding anomaly, bit2 more frames than the stream was sized for, kStreamNoF32Step
+  int type;      // score bytes of the stream, set by the reset (the float kernels leave it alone);
+                 // kStreamF64Stepped is or-ed in by a float64 step
 };
+template <>
+struct StreamHdrT<double> {
+  int n;
+  int flags;
+  int type;  // 8 once a double kernel has written the block (0 after a reset)
+  int pad;
+  unsigned long long gap;  // the fast kernel's 64-bit key
+};
+using StreamHdr = StreamHdrT<float>;
+// float header flag set by the reset and dropped by every float step (each one rewrites the flags)
+constexpr int kStreamNoF32Step = 1 << 30;
+// float header type bit: a float64 step ran on a stream reset for float scores
+constexpr int kStreamF64Stepped = 1 << 8;
+
+template <typename R = float>
 __host__ __device__ inline size_t StreamStateBytes(int W) {
-  return (sizeof(StreamHdr) + (size_t)W * 40 + 15) / 16 * 16;  // 5 x f32 + label + 2 x u64 per slot
+  // 5 scores + label + 2 x u64 per slot: 16 + 40 W bytes for float, 24 + 60 W for double
+  return (sizeof(StreamHdrT<R>) + (size_t)W * (5 * sizeof(R) + 20) + 15) / 16 * 16;
 }
-struct StreamView {
-  StreamHdr* hdr;
-  float *total, *blk, *lab, *ab, *an;
+// the double blocks of a float64 stream: right after the [B] float blocks (256-byte aligned)
+__host__ __device__ inline unsigned char* StreamState64(unsigned char* state, int B, int W) {
+  return state + ((size_t)B * StreamStateBytes<float>(W) + 255) / 256 * 256;
+}
+template <typename R>
+struct StreamViewT {
+  StreamHdrT<R>* hdr;
+  R *total, *blk, *lab, *ab, *an;
   int* label;
   unsigned long long *hash, *phash;
-  __host__ __device__ StreamView(unsigned char* base, int W) {
-    hdr = reinterpret_cast<StreamHdr*>(base);
-    total = reinterpret_cast<float*>(base + sizeof(StreamHdr));
+  __host__ __device__ StreamViewT(unsigned char* base, int W) {
+    hdr = reinterpret_cast<StreamHdrT<R>*>(base);
+    total = reinterpret_cast<R*>(base + sizeof(StreamHdrT<R>));
     blk = total + W; lab = blk + W; ab = lab + W; an = ab + W;
-    label = reinterpret_cast<int*>(an + W);
-    hash = reinterpret_cast<unsigned long long*>(label + W);
-    phash = hash + W;
+    if constexpr (sizeof(R) == 4) {
+      label = reinterpret_cast<int*>(an + W);
+      hash = reinterpret_cast<unsigned long long*>(label + W);
+      phash = hash + W;
+    } else {  // the 8-byte arrays first: aligned for any W
+      hash = reinterpret_cast<unsigned long long*>(an + W);
+      phash = hash + W;
+      label = reinterpret_cast<int*>(phash + W);
+    }
   }
 };
+using StreamView = StreamViewT<float>;
 
 
 // Kernel 3: trace-back

@@ -142,8 +142,9 @@ LaunchStatus LaunchBeamNarrow(BeamParams& p, int in_dtype, cudaStream_t stream) 
 // float64 logits (the op's T = double registration): the same kernel computing in double, 64-bit keys
 LaunchStatus LaunchBeamNarrow(BeamParamsT<double>& p, cudaStream_t stream) {
   if (!PrepareNarrow(p) || p.lm != nullptr) return {kLaunchUnsupported, cudaSuccess, ""};
-  p.state = nullptr;  // no time slices: whole utterances from the queue
-  p.t_done = nullptr;
+  // one-shot decodes take whole utterances from the queue (no time slices); a streamed step
+  // (t_done set) carries the beam in the double blocks of the state
+  if (p.t_done == nullptr) p.state = nullptr;
   const int wmax = TierOf(p.W);
   const size_t smem = SmemBytes(wmax, p.cand_cap, false, true);
   // (~90 KB of shared memory at beam 100: two CTAs per SM in either regime, 128 registers)

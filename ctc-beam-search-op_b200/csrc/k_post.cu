@@ -31,6 +31,36 @@ __global__ void PositiveKernel(const float* v, long long n, int* flag) {
     if (!(v[i] <= 0.0f)) *flag = 1;
 }
 
+// Every float block holds the root (what a float kernel resumes if a float64 step advanced the frame
+// count: a valid beam, never foreign bytes), marked "no float step yet" and tagged with the stream's
+// score type; the double blocks of a float64 stream are marked unwritten.
+__global__ void StreamResetKernel(unsigned char* state, int B, int W, int score_bytes) {
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
+    const StreamView fv(state + (size_t)b * StreamStateBytes(W), W);
+    fv.hdr->n = 1;
+    fv.hdr->gap = 0u;
+    fv.hdr->flags = kStreamNoF32Step;
+    fv.hdr->type = score_bytes;
+    fv.total[0] = 0.0f; fv.blk[0] = 0.0f; fv.lab[0] = NegInf(); fv.ab[0] = 0.0f; fv.an[0] = NegInf();
+    fv.label[0] = -1; fv.hash[0] = kRootHash; fv.phash[0] = 0ull;
+    if (score_bytes == 8) {
+      const StreamViewT<double> dv = StreamBlock64(state, B, W, b);
+      dv.hdr->n = 0;
+      dv.hdr->type = 0;
+    }
+  }
+}
+
+// A float64 step on a float stream marks the float header's type; a float step on a float64 stream drops
+// the "no float step yet" flag (float kernels rewrite the flags of every block they step).
+__global__ void StreamCheckKernel(const unsigned char* state, int B, int W, const int* table_flag, int* stats) {
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
+    const StreamHdr* h = reinterpret_cast<const StreamHdr*>(state + (size_t)b * StreamStateBytes(W));
+    const bool mixed = (h->type & kStreamF64Stepped) || (h->type == 8 && !(h->flags & kStreamNoF32Step));
+    if (mixed || (b == 0 && *table_flag != 0)) atomicMin(&stats[3], 0);
+  }
+}
+
 // frames of utterance b inside the time chunk [t0, t0 + len) of a decode that is run chunk by chunk
 __global__ void ChunkLenKernel(const int* seq_len, int B, int T, int t0, int len, int* out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -100,6 +130,17 @@ LaunchStatus LaunchChunkLen(const int* seq_len, int B, int T, int t0, int len, i
 LaunchStatus LaunchPositive(const float* v, long long n, int* flag, cudaStream_t stream) {
   PositiveKernel<<<(unsigned)std::min<long long>((n + 255) / 256, 1024), 256, 0, stream>>>(v, n, flag);
   return LaunchFrom(cudaGetLastError(), "PositiveKernel launch");
+}
+
+LaunchStatus LaunchStreamReset(unsigned char* state, int B, int W, int score_bytes, cudaStream_t stream) {
+  StreamResetKernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(state, B, W, score_bytes);
+  return LaunchFrom(cudaGetLastError(), "StreamResetKernel launch");
+}
+
+LaunchStatus LaunchStreamCheck(unsigned char* state, int B, int W, const int* table_flag, int* stats,
+                               cudaStream_t stream) {
+  StreamCheckKernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(state, B, W, table_flag, stats);
+  return LaunchFrom(cudaGetLastError(), "StreamCheckKernel launch");
 }
 
 LaunchStatus LaunchMathTest(int op, const float* x, float* y, int n, cudaStream_t stream) {

@@ -426,12 +426,19 @@ def ctc_ext_beam_search_decoder(inputs, sequence_length, beam_width, top_paths,
     return out
 
 
+def _torch_dtype(dtype):
+    """torch dtype of a torch or numpy dtype (np.float64, "float64", ...)."""
+    if isinstance(dtype, torch.dtype):
+        return dtype
+    return torch.from_numpy(np.empty(0, dtype=np.dtype(dtype))).dtype
+
+
 class CTCExtBeamSearchDecoderStream:
     """Streaming form of the decoder: the reference's `Step / TopPaths / Reset`
     (cc/util/ctc_ext_beam_search_decoder.h:39-53) for a whole batch, with the beam kept on the
     device between calls. Feeding the frames of an utterance in any chunking gives bit-identical
-    results to one `ctc_ext_beam_search_decoder` call on the concatenation. float32 scores only
-    (float16 / bfloat16 chunks are widened; float64 chunks are refused).
+    results to one `ctc_ext_beam_search_decoder` call on the concatenation with the same score type
+    and table.
 
         dec = CTCExtBeamSearchDecoderStream(batch_size=B, num_classes=C, beam_width=100, top_paths=1,
                                             max_time=3000, merge_repeated=True, blank_index=C - 1)
@@ -439,48 +446,86 @@ class CTCExtBeamSearchDecoderStream:
             dec.step(chunk)                   # or dec.step(chunk, lengths) for ragged chunks
             decoded, alignment, logp = dec.top_paths()   # any time; does not disturb the state
         dec.reset()
+
+    dtype             score type of the stream (torch or numpy dtype): float32 (default) takes float32,
+                      float16 and bfloat16 chunks (half chunks are read in place, as the one-shot decode
+                      reads them); float64 takes float64 chunks, computes in float64 and returns float64
+                      log_probability. Other chunk types raise TypeError.
+    expansion_scores  optional scorer table, as for `ctc_ext_beam_search_decoder_raw` ([num_classes + 1,
+                      num_classes], entries <= 0; float32 streams only), checked once here.
     """
 
     def __init__(self, batch_size, num_classes, beam_width, top_paths, max_time, merge_repeated=False,
-                 blank_index=0, blank_label=-1, device=None):
+                 blank_index=0, blank_label=-1, device=None, dtype=torch.float32, expansion_scores=None):
         if int(beam_width) < 1 or int(top_paths) < 1:
             raise ValueError("beam_width and top_paths must be >= 1")
-        if not torch.cuda.is_available():
-            raise RuntimeError("ctcx: no CUDA device available and there is no CPU fallback")
+        self.dtype = _torch_dtype(dtype)
+        if self.dtype not in (torch.float32, torch.float64):
+            raise TypeError("the streaming decoder computes in float32 or float64, not %s" % self.dtype)
+        self._f64 = self.dtype == torch.float64
         self._lib = _lib.load()
         self.B, self.C, self.W, self.P, self.T = (int(batch_size), int(num_classes), int(beam_width),
                                                   int(top_paths), int(max_time))
+        es = None
+        if expansion_scores is not None:
+            if self._f64:
+                raise TypeError("expansion_scores is supported for float32 inputs only")
+            es, _ = _as_tensor(expansion_scores)
+            if tuple(es.shape) != (self.C + 1, self.C):
+                raise InvalidArgumentError(8, "expansion_scores must have shape [num_classes + 1, num_classes]")
+            es = es.to(dtype=torch.float32)
+            if not bool((es.cpu() <= 0).all()):  # log-probabilities (NaN fails too)
+                raise InvalidArgumentError(8, self._lib.ctcx_strerror(8).decode())
+        if not torch.cuda.is_available():
+            raise RuntimeError("ctcx: no CUDA device available and there is no CPU fallback")
         self.merge_repeated, self.blank_index, self.blank_label = (bool(merge_repeated), int(blank_index),
                                                                    int(blank_label))
         self.device = (torch.device(device) if device is not None
                        else torch.device("cuda", torch.cuda.current_device()))
-        nbytes = self._lib.ctcx_stream_workspace_bytes(self.T, self.B, self.C, self.W, self.P)
+        self._score_code = _lib.F64 if self._f64 else _lib.F32
+        nbytes = self._lib.ctcx_stream_workspace_bytes_v(self._score_code, self.T, self.B, self.C, self.W, self.P)
         if nbytes == 0:
             raise InvalidArgumentError(8, self._lib.ctcx_strerror(8).decode())
         self._nbytes = nbytes
         self._ws = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=self.device)
+        self._esd = None if es is None else es.to(device=self.device).contiguous()
         self.reset()
 
     def _stream(self):
         return torch.cuda.current_stream(self.device).cuda_stream
 
+    def _chunk_dtypes(self):
+        return (torch.float64,) if self._f64 else (torch.float32, torch.float16, torch.bfloat16)
+
     def reset(self):
         """Reset() (decoder.h:212-227): back to the empty prefix for every utterance."""
         with torch.cuda.device(self.device):
-            rc = self._lib.ctcx_stream_reset(self._ws.data_ptr(), self._nbytes, self.T, self.B, self.C,
-                                             self.W, self.P, self._stream())
+            rc = self._lib.ctcx_stream_reset_v(self._ws.data_ptr(), self._nbytes, self._score_code, self.T, self.B,
+                                               self.C, self.W, self.P, self._stream())
         if rc != 0:
             _raise(self._lib, rc)
 
+    def _step(self, x, ln):
+        """ctcx_stream_step_v on a frame-strided device chunk and device lengths; returns the code."""
+        tstride = int(x.stride(0)) if int(x.shape[0]) > 1 else self.B * self.C
+        return self._lib.ctcx_stream_step_v(
+            self._ws.data_ptr(), self._nbytes, self.T, self.B, self.C, self.W, self.P, x.data_ptr(),
+            _DTYPE_CODE[x.dtype], tstride, int(x.shape[0]), ln.data_ptr(), self.blank_index,
+            None if self._esd is None else self._esd.data_ptr(), self._stream())
+
     def step(self, inputs, sequence_length=None):
         """Step() over a chunk: inputs [chunk_time, batch, num_classes]; sequence_length[b] = how many
-        leading frames of the chunk utterance b consumes (default: all)."""
+        leading frames of the chunk utterance b consumes (default: all). A device chunk that is a batch
+        shard `x[:, b0:b1, :]` of a contiguous tensor is read in place."""
         x, _ = _as_tensor(inputs)
         if x.dim() != 3:
             raise InvalidArgumentError(1, self._lib.ctcx_strerror(1).decode())
-        if x.dtype == torch.float64:
+        if self._f64 and x.dtype != torch.float64:
+            raise TypeError("a float64 stream takes float64 chunks, got %s" % x.dtype)
+        if not self._f64 and x.dtype == torch.float64:
             raise TypeError("the streaming decoder computes in float32; float64 chunks would not be "
-                            "bit-identical to a one-shot float64 decode -- cast explicitly if that is intended")
+                            "bit-identical to a one-shot float64 decode -- cast explicitly, or make the "
+                            "stream with dtype=torch.float64")
         Tc, B, C = (int(v) for v in x.shape)
         if B != self.B or C != self.C:
             raise InvalidArgumentError(8, "chunk shape %s does not match the stream (batch %d, classes %d)"
@@ -488,7 +533,10 @@ class CTCExtBeamSearchDecoderStream:
         if Tc == 0:
             return
         with torch.cuda.device(self.device):
-            xd = x.to(device=self.device, dtype=torch.float32, non_blocking=True).contiguous()
+            dt = x.dtype if x.dtype in self._chunk_dtypes() else torch.float32
+            xd = x.to(device=self.device, dtype=dt, non_blocking=True)
+            if not _frame_strided(xd):
+                xd = xd.contiguous()
             if sequence_length is None:
                 ld = torch.full((B,), Tc, dtype=torch.int32, device=self.device)
             else:
@@ -499,9 +547,12 @@ class CTCExtBeamSearchDecoderStream:
                 if bool((l.to("cpu") > Tc).any()) or bool((l.to("cpu") < 0).any()):
                     raise FailedPreconditionError(5, "sequence_length(b) <= %d" % Tc)
                 ld = l.to(device=self.device, dtype=torch.int32).contiguous()
-            rc = self._lib.ctcx_stream_step_f32(self._ws.data_ptr(), self.T, self.B, self.C, self.W, self.P,
-                                                xd.data_ptr(), Tc, ld.data_ptr(), self.blank_index,
-                                                self._stream())
+            rc = self._step(xd, ld)
+            if rc == 9 and xd.dtype in (torch.float16, torch.bfloat16):
+                # a table with half-precision chunks where the kernel has no room to widen them (as in the
+                # one-shot decode), or the test hook's generic kernel forced onto a fast-path shape
+                xd = xd.float().contiguous()
+                rc = self._step(xd, ld)
             # the kernels read xd / ld asynchronously on this stream; keep them alive until then
             xd.record_stream(torch.cuda.current_stream(self.device))
             ld.record_stream(torch.cuda.current_stream(self.device))
@@ -509,27 +560,27 @@ class CTCExtBeamSearchDecoderStream:
             _raise(self._lib, rc)
 
     def step_device(self, inputs_dev, lengths_dev):
-        """Step() on buffers that already live on the device -- float32 [chunk_time, batch, num_classes]
-        and int32 [batch], both contiguous -- without any conversion, allocation or synchronisation: the
-        call only enqueues kernels on the current stream, so it can be captured into a CUDA graph
+        """Step() on buffers that already live on the device -- a [chunk_time, batch, num_classes] chunk of
+        one of the stream's chunk types (contiguous, or a batch shard of a contiguous tensor) and int32
+        [batch] lengths -- without any conversion, allocation or synchronisation: the call only enqueues
+        kernels on the current stream, so it can be captured into a CUDA graph
         (`with torch.cuda.graph(g): dec.step_device(x_static, len_static)`) and replayed per chunk,
-        which removes the launch overhead that dominates small chunks."""
+        which removes the launch overhead that dominates small chunks. Half-precision chunks with a
+        scorer table raise UnsupportedError where `step()` would widen them."""
         x, ln = inputs_dev, lengths_dev
-        if not (x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 3 and
+        if not (x.is_cuda and x.dtype in self._chunk_dtypes() and x.dim() == 3 and _frame_strided(x) and
                 int(x.shape[1]) == self.B and int(x.shape[2]) == self.C):
-            raise InvalidArgumentError(8, "step_device needs a contiguous CUDA float32 [chunk_time, %d, %d] tensor"
-                                       % (self.B, self.C))
+            raise InvalidArgumentError(8, "step_device needs a frame-strided CUDA %s [chunk_time, %d, %d] tensor"
+                                       % ("/".join(str(d) for d in self._chunk_dtypes()), self.B, self.C))
         if not (ln.is_cuda and ln.dtype == torch.int32 and ln.is_contiguous() and tuple(ln.shape) == (self.B,)):
             raise InvalidArgumentError(8, "step_device needs a contiguous CUDA int32 [%d] tensor" % self.B)
-        rc = self._lib.ctcx_stream_step_f32(self._ws.data_ptr(), self.T, self.B, self.C, self.W, self.P,
-                                            x.data_ptr(), int(x.shape[0]), ln.data_ptr(), self.blank_index,
-                                            self._stream())
+        rc = self._step(x, ln)
         if rc != 0:
             _raise(self._lib, rc)
 
     def top_paths_raw(self):
         """TopPaths() (decoder.h:229-261) of the frames consumed so far, as the raw 7 output groups
-        (device tensors)."""
+        (device tensors; log_probability in the stream's score type)."""
         P = self.P
         arr = ctypes.c_int64 * P
         n_dec, max_dec, n_ali, max_ali = arr(), arr(), arr(), arr()
@@ -542,7 +593,7 @@ class CTCExtBeamSearchDecoderStream:
             if rc != 0:
                 _raise(self._lib, rc)
             groups, logp, _ = _pack(self._lib, self._ws, self.T, self.B, P, (n_dec, n_ali), self.device,
-                                    self._stream())
+                                    self._stream(), self._f64)
         res = CTCExtBeamSearchDecoder(*groups, logp)
         res.flags = int(flags.value)
         return res

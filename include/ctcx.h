@@ -254,10 +254,12 @@ int ctcx_decode_scorer_f32(const float* logits_dev, int max_time, int batch, int
  *   ctcx_stream_reset(...)                       Reset():    decoder.h:212-227
  *   ctcx_stream_step_f32(..., chunk, lens ...)   Step() x lens[b] frames: decoder.h:67-210
  *   ctcx_stream_top_paths(...) + ctcx_pack_f32   TopPaths(): decoder.h:229-261 (does not disturb the state)
- * Feeding the same frames in any chunking gives bit-identical results to one ctcx_decode_f32 call.
+ * Feeding the same frames in any chunking gives bit-identical results to one one-shot decode of the
+ * same score type (ctcx_decode_view / ctcx_decode_f64 / ctcx_decode_scorer_f32 with the same table).
  * max_time_total bounds the frames per utterance over the whole stream (feeding more is reported by
  * ctcx_stream_top_paths as CTCX_ERR_SEQ_LEN_RANGE). The shape arguments must be the same in every
- * call on one workspace. None of the step calls synchronises. ---- */
+ * call on one workspace. None of the step calls synchronises. The un-suffixed entries are the float32
+ * stream of the _v entries (same workspace size). ---- */
 size_t ctcx_stream_workspace_bytes(int max_time_total, int batch, int num_classes, int beam_width,
                                    int top_paths);
 int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int max_time_total, int batch,
@@ -267,8 +269,27 @@ int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int max_time_tota
 int ctcx_stream_step_f32(void* workspace, int max_time_total, int batch, int num_classes,
                          int beam_width, int top_paths, const float* logits_dev, int chunk_time,
                          const int32_t* chunk_len_dev, int blank_index, void* stream);
+/* A stream with score_dtype scores: CTCX_F32 (float32 / float16 / bfloat16 chunks) or CTCX_F64 (float64
+ * chunks, double scores; pack with ctcx_pack_f64). workspace_bytes 0 = bad arguments. */
+size_t ctcx_stream_workspace_bytes_v(int score_dtype, int max_time_total, int batch, int num_classes,
+                                     int beam_width, int top_paths);
+int ctcx_stream_reset_v(void* workspace, size_t workspace_bytes, int score_dtype, int max_time_total,
+                        int batch, int num_classes, int beam_width, int top_paths, void* stream);
+/* One Step() of a chunk of element type `dtype` (CTCX_F32 / F16 / BF16 step a float32 stream, CTCX_F64 a
+ * float64 one), row (t, b) at element t * time_stride + b * num_classes (0 = batch * num_classes: a batch
+ * shard [:, b0:b1, :] of a wider tensor is stepped in place). expansion_scores_dev: the scorer table of
+ * ctcx_decode_scorer_f32 (float32 streams; NULL = the default scorer); with float16 / bfloat16 chunks it
+ * returns CTCX_ERR_UNSUPPORTED wherever ctcx_decode_scorer_f32 would not take them (widen the chunk).
+ * Errors: CTCX_ERR_WORKSPACE when workspace_bytes is short of the chunk's score type; unknown dtype or a
+ * stride shorter than a frame: CTCX_ERR_BAD_ARGUMENT. A table entry > 0, or float32 and float64 steps
+ * since the last reset, make the next ctcx_stream_top_paths return CTCX_ERR_BAD_ARGUMENT. */
+int ctcx_stream_step_v(void* workspace, size_t workspace_bytes, int max_time_total, int batch,
+                       int num_classes, int beam_width, int top_paths, const void* logits_dev, int dtype,
+                       int64_t time_stride, int chunk_time, const int32_t* chunk_len_dev, int blank_index,
+                       const float* expansion_scores_dev, void* stream);
 /* Leaves the dense result in the workspace and reports the sparse sizes; follow with
- * ctcx_pack_f32(workspace, max_time_total, batch, top_paths, ...). Synchronises `stream` once. */
+ * ctcx_pack_f32(workspace, max_time_total, batch, top_paths, ...) (ctcx_pack_f64 for a float64
+ * stream). Synchronises `stream` once. */
 int ctcx_stream_top_paths(void* workspace, int max_time_total, int batch, int num_classes,
                           int beam_width, int top_paths, int merge_repeated, int blank_label,
                           void* stream, ctcx_sizes* sizes, int32_t* flags_out);
