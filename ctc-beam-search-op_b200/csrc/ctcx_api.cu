@@ -70,6 +70,7 @@ void InitStats(int* stats, int B) {
 std::atomic<int> g_force_generic{0};
 // measurement hook (ctcx_debug_set_cycles_buffer)
 thread_local long long* g_dbg_cycles = nullptr;
+thread_local int g_dbg_slots = 24;
 
 enum Path { kPathNarrow, kPathWide, kPathGeneric };
 // which beam kernel (and with it which pre-pass) decodes this shape with R scores
@@ -418,6 +419,7 @@ int DecodeImpl(const void* logits_dev, int T, int B, int C, const int32_t* seq_l
     bp.lm = (const R*)opt.lm;
     bp.ready = opt.ready;
     bp.dbg_cycles = g_dbg_cycles;
+    bp.dbg_slots = g_dbg_slots;
     const Logits x = {logits_dev, opt.in_dtype, tstride};
     if (path == kPathWide && opt.n_slabs > 0) {
       // Host feed of a wide-vocabulary batch: the copy (hundreds of MB) takes longer than the decode, so
@@ -1142,7 +1144,14 @@ void ctcx_profile_get(float* out_ms) {
 
 /* device buffer [B,24] int64 receiving per-phase clock64 cycles of the fast beam kernels (thread 0
  * of every CTA, summed over frames) for this thread's decodes; NULL switches it off. */
-void ctcx_debug_set_cycles_buffer(long long* dev_buf) { g_dbg_cycles = dev_buf; }
+void ctcx_debug_set_cycles_buffer(long long* dev_buf) { ctcx_debug_set_cycles_buffer_n(dev_buf, 24); }
+
+/* the same with [B,slots] rows (slots >= 24; smaller values count as 24): the narrow kernel also
+ * fills its revisit-wipe event counters 24-26 where the row has room for them. */
+void ctcx_debug_set_cycles_buffer_n(long long* dev_buf, int slots) {
+  g_dbg_cycles = dev_buf;
+  g_dbg_slots = slots > 24 ? slots : 24;
+}
 
 /* 0 = dispatch by shape (default); 1 = route every decode of the process to the generic beam kernel,
  * the independent second implementation the parity tests compare with the fast ones. */

@@ -81,9 +81,9 @@ struct BeamSmemV4 {
   static constexpr size_t m_rec = m_key + w * rb;         // u32 [WMAX]
   static constexpr size_t m_pslot = m_rec + w * 4;        // i32 [WMAX]
   static constexpr size_t risk = m_pslot + w * 4;         // i32 [WMAX]
-  static constexpr size_t risk_new = risk + w * 4;        // i32 [WMAX]
-  static constexpr size_t wiped = risk_new + w * 4;       // u32 [WMAX]
-  static constexpr size_t qcnt = wiped + w * 4;           // i32 [WMAX]   revisit-wipe queries: items ranking before the member
+  static constexpr size_t con = risk + w * 4;             // i32 [WMAX]   contested at-risk members (PC)
+  static constexpr size_t wiped = con + w * 4;            // u32 [WMAX]
+  static constexpr size_t qcnt = wiped + w * 4;           // i32 [WMAX]   per contested member: items ranking before it
   static constexpr size_t qchg = qcnt + w * 4;            // u32 [WMAX]   rows whose wiped state changed in this round: (row << 1) | new state
   static constexpr size_t htab = qchg + w * 4;            // u32 [8*WMAX]  (hash tag << 10 | slot), 0xffffffff = empty
   static constexpr size_t hist = htab + 8 * w * 4;        // u32 [kBinsV2]
@@ -208,7 +208,12 @@ __device__ __forceinline__ unsigned long long ReachOf(unsigned long long gap) {
   return (gap > (1ull << 62)) ? ~0ull : gap + gap / 4ull + 64ull;
 }
 
-enum { kV4Utt = 23, kV4Abort = 24, kV4NChg = 25 };  // scalar slots in addition to the kV2* / kV3* ones
+// scalar slots in addition to the kV2* / kV3* ones. PC: kV4NChg and kV4MinWiped are pairs, one word per
+// round parity (a round reads the pair's one half and writes the other); kV4NAtRisk counts at-risk
+// members for the timing build's event counters only.
+enum { kV4Utt = 23, kV4Abort = 24, kV4NChg = 25, kV4MinWiped = 27, kV4MaxParent = 29, kV4NAtRisk = 30 };
+// timing build: clock64 phase slots 0-19, event counters 20-26 (tools/phase_cycles.py names them)
+constexpr int kV4DbgSlots = 27;
 
 // MINB = resident CTAs per SM the register allocation is tuned for: 4 (64 registers) for batches that
 // fill the machine, 2 (128 registers: more loads in flight, no re-materialisation) for the latency
@@ -261,7 +266,7 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
   unsigned* m_rec = (unsigned*)(smem + lay::m_rec);
   int* m_pslot = (int*)(smem + lay::m_pslot);
   int* s_risk = (int*)(smem + lay::risk);
-  int* s_risk_new = (int*)(smem + lay::risk_new);
+  int* s_con = (int*)(smem + lay::con);
   unsigned* s_wiped = (unsigned*)(smem + lay::wiped);
   int* s_qcnt = (int*)(smem + lay::qcnt);
   unsigned* s_qchg = (unsigned*)(smem + lay::qchg);
@@ -312,7 +317,7 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
   const int pg_slot = tid % WMAX, pg_role = tid / WMAX;
 
   // optional per-phase clock64 instrumentation (thread 0), compiled out of the production kernel
-  long long cyc[TIMING ? 24 : 1] = {0};
+  long long cyc[TIMING ? kV4DbgSlots : 1] = {0};
   long long tprev = 0;
   const bool timing = TIMING && (p.dbg_cycles != nullptr) && tid == 0;
 #define CTCX_TICK(i)                      \
@@ -490,6 +495,10 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
       sci[kV2Anomaly] = 0;
       sci[kV2NCand] = 0;
       sci[kV2NRisk] = 0;
+      sci[kV4NChg] = 0;
+      sci[kV4MinWiped] = 0x7fffffff;
+      sci[kV4MaxParent] = -1;
+      sci[kV4NAtRisk] = 0;
       s_keys[kV4KMin] = Ops::kKeyMax;
       s_keys[kV4KMax] = (Key)0;
       sci[kV2NBnd] = 0;
@@ -633,8 +642,17 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
         if (pslot >= 0) {
           atomicOr(Rec::MaskPtr(&s_row[pslot]), 1u << lbl);
           if (pslot < i) {
-            const int q = atomicAdd(&sci[kV2NRisk], 1);
-            s_risk[q] = i;
+            atomicMax(&sci[kV4MaxParent], pslot);
+            if constexpr (TIMING) atomicAdd(&sci[kV4NAtRisk], 1);
+            // A wipe query counts the members ranking before this one (fewer than n <= W) plus the
+            // children above v_nt. No child can be: a child's base is a row's old total, or its old blank
+            // mass, which is never above it; row 0 holds the largest old total; fp addition is monotone.
+            // So a member above lp_max + o_total[0] is never wiped and is not listed. (The scorer's
+            // table adds an entry to the base; its sign is not checked on every path, so LM lists all.)
+            if (LM || !(v_nt > Ops::Add(s_fsc[cur * 4 + 1], o_total[0]))) {
+              const int q = atomicAdd(&sci[kV2NRisk], 1);
+              s_risk[q] = i;
+            }
           }
         }
       }
@@ -731,7 +749,13 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
       // per member). When verdicts wipe rows, the counts are not recomputed: a later round only adds or
       // removes the contribution of the rows whose state CHANGED -- one thread per (member, changed row)
       // pair -- and re-derives the verdicts; a handful of candidate tests instead of a full sweep each.
+      int fp_contested = 0, fp_rounds = 0;  // timing build: contested members, verdict derivations
       if (__builtin_expect(n_risk > 0, 0)) {
+        // Round 1 counts with no row wiped; a later round only subtracts wiped rows or adds restored ones
+        // back, so no count ever exceeds its round-1 value. A member whose round-1 count is below W is
+        // therefore a final survivor and its row never changes state. Only the others, the contested
+        // members, take part in later rounds: round 1 wipes them all (no parent is wiped yet), lists them
+        // as the rows that changed, and thread k owns the verdict of contested member k from then on.
         for (int q = warp; q < n_risk; q += NWARP) {  // round 1: one warp per at-risk member (nothing is wiped yet)
           const int m = s_risk[q];
           const int pslot = m_pslot[m];
@@ -754,59 +778,60 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
             }
           }
           cnt = __reduce_add_sync(kFull, cnt);
-          if (lane == 0) {
-            s_qcnt[q] = cnt;
-            s_risk_new[q] = (cnt >= W) ? 1 : 0;
+          if (lane == 0 && cnt >= W) {
+            const int k = atomicAdd(&sci[kV4NChg], 1);
+            s_con[k] = m;
+            s_qcnt[k] = cnt;
+            s_qchg[k] = ((unsigned)m << 1) | 1u;
+            s_wiped[m] = 1u;  // (round 1 reads no wiped state)
+            atomicMin(&sci[kV4MinWiped], m);
           }
         }
-        for (;;) {
-          __syncthreads();
-          // every thread inspects the (few) verdicts itself: no flag, no extra barrier when nothing
-          // changes -- the common case
-          bool changed = false;
-          int min_wiped = 0x7fffffff, max_parent = -1;
-          for (int q = 0; q < n_risk; ++q) {
-            const int m = s_risk[q];
-            const unsigned v = (unsigned)s_risk_new[q];
-            changed |= (s_wiped[m] != v);
-            if (v) min_wiped = min(min_wiped, m);
-            max_parent = max(max_parent, m_pslot[m]);
-          }
-          if (!changed) break;
-          __syncthreads();  // all reads of s_wiped are done
-          if (tid == 0) sci[kV4NChg] = 0;
-          __syncthreads();
-          for (int q = tid; q < n_risk; q += NT) {  // apply the verdicts, list the rows that changed
-            const int m = s_risk[q];
-            const unsigned nv = (unsigned)s_risk_new[q];
-            if (s_wiped[m] != nv) {
-              s_wiped[m] = nv;
-              s_qchg[atomicAdd(&sci[kV4NChg], 1)] = ((unsigned)m << 1) | nv;
-            }
-          }
-          __syncthreads();
+        __syncthreads();
+        const int n_con = sci[kV4NChg];
+        if (TIMING) {
+          fp_contested = n_con;
+          fp_rounds = 1;
+        }
+        // Rounds after the first. Words [par] hold the last round's changes; the apply step writes [par ^ 1].
+        for (int par = 0;; par ^= 1) {
           // a query only counts rows up to its parent's: if every wiped row lies beyond every parent
-          // row, no count (and no parent) is affected and the verdicts are final
-          if (min_wiped > max_parent) break;
-          const int n_chg = sci[kV4NChg];
-          for (int pr = tid; pr < n_risk * n_chg; pr += NT) {  // one (member, changed row) pair per thread
-            const int q = pr / n_chg, c = pr - q * n_chg;
+          // row, no count (and no parent) is affected and the verdicts are final (no contested member: no
+          // wiped row)
+          if (sci[kV4MinWiped + par] > sci[kV4MaxParent]) break;  // (max over every at-risk member, listed or not)
+          const int n_chg = sci[kV4NChg + par];
+          const bool parent_wiped = (tid < n_con) && s_wiped[m_pslot[s_con[tid]]] != 0u;
+          for (int pr = tid; pr < n_con * n_chg; pr += NT) {  // one (contested member, changed row) pair per thread
+            const int k = pr / n_chg, c = pr - k * n_chg;
             const unsigned e = s_qchg[c];
             const int r = (int)(e >> 1);
-            const int m = s_risk[q];
+            const int m = s_con[k];
             const int pslot = m_pslot[m];
             if (r <= pslot) {
               unsigned mk = cand_mask(s_row[r], m_nt[m]);
               if (r == pslot) mk &= (1u << o_label[m]) - 1u;
               const int d = __popc(mk);
-              if (d) atomicAdd(&s_qcnt[q], (e & 1u) ? -d : d);  // wiped rows stop counting, restored ones count again
+              if (d) atomicAdd(&s_qcnt[k], (e & 1u) ? -d : d);  // wiped rows stop counting, restored ones count again
             }
           }
-          __syncthreads();
-          for (int q = tid; q < n_risk; q += NT) {  // a wiped parent never sweeps (decoder.h:167)
-            const int pslot = m_pslot[s_risk[q]];
-            s_risk_new[q] = (!s_wiped[pslot] && s_qcnt[q] >= W) ? 1 : 0;
+          if (tid == 0) {  // nobody reads these words again before the next barrier
+            sci[kV4NChg + (par ^ 1)] = 0;
+            sci[kV4MinWiped + (par ^ 1)] = 0x7fffffff;
           }
+          __syncthreads();
+          if (TIMING) ++fp_rounds;
+          bool changed = false;
+          if (tid < n_con) {  // re-derive the verdict, apply it, list the row if it changed
+            const int m = s_con[tid];  // (only this thread writes s_wiped[m] after round 1)
+            const unsigned nv = (!parent_wiped && s_qcnt[tid] >= W) ? 1u : 0u;  // a wiped parent never sweeps (decoder.h:167)
+            if (nv != s_wiped[m]) {
+              changed = true;
+              s_wiped[m] = nv;
+              s_qchg[atomicAdd(&sci[kV4NChg + (par ^ 1)], 1)] = ((unsigned)m << 1) | nv;
+            }
+            if (nv) atomicMin(&sci[kV4MinWiped + (par ^ 1)], m);
+          }
+          if (!__syncthreads_or(changed)) break;
         }
       }
       CTCX_TICK(2)  // PC
@@ -968,17 +993,21 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
       }
       const bool member_in = !clamped || my_key > lo_key;
       const int bstar = sc[kV2Bstar], k_rem = sc[kV2KRem], e_b = sc[kV2E], n_new = sc[kV2NNew];
-      if (TIMING && timing) {  // event counters (slots 20-23): how selective would a "below the cut" filter be?
+      if (TIMING && timing) {  // event counters (slots 20-26): how selective would a "below the cut" filter be?
         int below = 0, wiped = 0;
-        for (int q = 0; q < n_risk; ++q) {
+        for (int q = 0; q < n_risk; ++q) {  // (the members PA listed; the others are never wiped)
           const int m = s_risk[q];
           below += (bucket_of(m_key[m]) <= bstar || (clamped && m_key[m] <= lo_key)) ? 1 : 0;
           wiped += s_wiped[m] ? 1 : 0;
         }
-        cyc[TIMING ? 20 : 0] += n_risk;
+        const int at_risk = sci[kV4NAtRisk];
+        cyc[TIMING ? 20 : 0] += at_risk;
         cyc[TIMING ? 21 : 0] += below;
         cyc[TIMING ? 22 : 0] += wiped;
-        cyc[TIMING ? 23 : 0] += (n_risk > 0) ? 1 : 0;
+        cyc[TIMING ? 23 : 0] += (at_risk > 0) ? 1 : 0;
+        cyc[TIMING ? 24 : 0] += n_risk;                                   // listed by PA
+        cyc[TIMING ? 25 : 0] += fp_contested;
+        cyc[TIMING ? 26 : 0] += fp_rounds;
       }
       // a suspect member (see PA) that is not certain to stay in the beam: report the utterance
       if (__builtin_expect(suspect, 0) && (!member_in || bucket_of(my_key) <= bstar)) sci[kV2Anomaly] = 1;
@@ -1130,6 +1159,10 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
         if (tid == 0) {
           sci[kV2NCand] = 0;
           sci[kV2NRisk] = 0;
+          sci[kV4NChg] = 0;
+          sci[kV4MinWiped] = 0x7fffffff;
+          sci[kV4MaxParent] = -1;
+          if (TIMING) sci[kV4NAtRisk] = 0;
           s_keys[kV4KMin] = Ops::kKeyMax;
           s_keys[kV4KMax] = (Key)0;
           sci[kV2NBnd] = 0;
@@ -1207,8 +1240,8 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
       }
     }
     if (TIMING && timing)
-      for (int i = 0; i < (TIMING ? 24 : 1); ++i) {
-        atomicAdd(reinterpret_cast<unsigned long long*>(p.dbg_cycles + (size_t)b * 24 + i), (unsigned long long)cyc[i]);
+      for (int i = 0; i < (TIMING ? kV4DbgSlots : 1); ++i) {
+        if (i < p.dbg_slots) atomicAdd(reinterpret_cast<unsigned long long*>(p.dbg_cycles + (size_t)b * p.dbg_slots + i), (unsigned long long)cyc[i]);
         cyc[TIMING ? i : 0] = 0;
       }
 

@@ -988,7 +988,7 @@ __global__ void __launch_bounds__(NT, ((NT <= 256 && !TIMING) ? 4 : 1)) BeamKern
     n = n_new;
   }
   if (TIMING && timing)
-    for (int i = 0; i < (TIMING ? 24 : 1); ++i) p.dbg_cycles[(size_t)b * 24 + i] = cyc[i];
+    for (int i = 0; i < (TIMING ? 24 : 1); ++i) p.dbg_cycles[(size_t)b * p.dbg_slots + i] = cyc[i];
 #undef CTCX_TICK
 
   // ---- final beam (decoder.h:229-261): sorted, the first P slots are the top paths ----

@@ -24,7 +24,8 @@ struct BeamParamsT {
   int* flags;        // [B]   bit0 rounding anomaly, bit1 fewer leaves than top_paths
   R* dbg_totals;      // optional [B,T,W]
   int* dbg_n;         // optional [B,T]
-  long long* dbg_cycles;  // optional [B,24]: clock64 cycles per phase (thread 0), summed over frames
+  long long* dbg_cycles;  // optional [B,dbg_slots]: clock64 cycles per phase (thread 0), summed over frames
+  int dbg_slots;          // row length of dbg_cycles (>= 24)
   // streaming (Step / TopPaths / Reset, decoder.h:39-53); all null / T for a one-shot decode
   int Tcap;               // frames per utterance the back-pointer array can hold (its row stride)
   int* t_done;            // [B] frames already consumed per utterance (updated by the kernel), or null

@@ -311,8 +311,11 @@ void ctcx_profile_get(float* out_ms);
 
 /* Device buffer [batch, 24] int64 receiving per-phase clock64 cycles of the fast beam kernels (thread
  * 0 of every CTA, summed over frames; a separately compiled timing build of the kernel is launched
- * while it is set) for the calling thread's decodes; NULL switches it off. tools/phase_cycles.py. */
+ * while it is set) for the calling thread's decodes; NULL switches it off. tools/phase_cycles.py.
+ * The _n form takes rows of `slots` >= 24 entries; the narrow kernel fills its revisit-wipe event
+ * counters 24-26 (at-risk members listed, contested members, fixed-point rounds) where they fit. */
 void ctcx_debug_set_cycles_buffer(long long* dev_buf);
+void ctcx_debug_set_cycles_buffer_n(long long* dev_buf, int slots);
 
 /* 0 = dispatch by shape (default); 1 = route every decode of the process to the generic beam kernel,
  * the independently written second implementation the parity tests compare with the fast kernels. */

@@ -22,7 +22,8 @@ x = torch.from_numpy(L.make_logits(kind, T, B, C, BLANK, 1)).cuda()
 if len(sys.argv) > 4 and sys.argv[4] == "bf16":  # bfloat16-rounded values (many exact ties), float32 kernel
     x = x.bfloat16().float()
 sl = torch.full((B,), T, dtype=torch.int32).cuda()
-buf = torch.zeros((B, 24), dtype=torch.int64, device="cuda")
+NS = 27  # the narrow kernel also fills its revisit-wipe event counters 24-26
+buf = torch.zeros((B, NS), dtype=torch.int64, device="cuda")
 kw = dict(beam_width=W, top_paths=1, merge_repeated=MERGE, blank_index=BLANK)
 if len(sys.argv) > 4 and sys.argv[4] == "scorer":  # the bench's random label-bigram table
     kw["expansion_scores"] = torch.from_numpy(
@@ -34,7 +35,7 @@ ms = (ctypes.c_float * 5)()
 op.ctc_ext_beam_search_decoder_raw(x, sl, **kw)
 lib.ctcx_profile_get(ms)
 prod_ms = ms[1]
-lib.ctcx_debug_set_cycles_buffer(buf.data_ptr())
+lib.ctcx_debug_set_cycles_buffer_n(buf.data_ptr(), NS)
 op.ctc_ext_beam_search_decoder_raw(x, sl, **kw)
 torch.cuda.synchronize()
 lib.ctcx_profile_get(ms)
@@ -43,7 +44,8 @@ print("beam kernel: production build %.3f ms, timing build %.3f ms" % (prod_ms, 
 c = buf.cpu().numpy().astype(np.float64) / T
 names = ["PA(end)", "PB(end)", "PC", "PD", "PE", "PF", "PG(end)", "setup", "PA.lookup", "PA.lse1", "PA.lse2",
          "PA.store", "PA.minmax", "PG.rank", "PG.barrier", "PG.write", "PB.range", "PB.pass1", "PB.scan",
-         "PB.pass2+bar"] + (["ev.n_risk", "ev.risk_below_cut", "ev.wiped", "ev.frames_with_risk"] if cfg == "cfg2"
+         "PB.pass2+bar"] + (["ev.n_risk", "ev.risk_below_cut", "ev.wiped", "ev.frames_with_risk", "ev.listed",
+                                  "ev.contested", "ev.fp_rounds"] if cfg == "cfg2"
                                  else ["ev.slowcut", "ev.fullrange", "ev.capped", "ev.ncand"])
 m = c.mean(axis=0)
 tot = c[:, :20].sum(axis=1)
