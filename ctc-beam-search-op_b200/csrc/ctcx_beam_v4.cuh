@@ -1,6 +1,6 @@
 // Beam kernel, fourth generation: the fast path for num_classes <= 32 (all of BASELINE's char-CTC
-// shapes). Bit-identical results to the generic BeamKernel (ctcx_kernels.cuh); what changed against the
-// third generation (round 1) is how the kernel is fed and scheduled:
+// shapes). Bit-identical results to the generic BeamKernelT (ctcx_beam_generic.cuh); what changed against
+// the third generation (round 1) is how the kernel is fed and scheduled:
 //
 //   * persistent CTAs: the grid is sized to the machine (resident CTAs per SM x SM count) and every
 //     CTA pulls utterances from a queue until it is empty -- no tail wave, ragged lengths balance
@@ -1205,7 +1205,6 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
             }
             w_label[r] = lbl;
             p.bp32[((size_t)b * p.Tcap + (t_done + t0 + t)) * W + r] = rec;
-            if (p.dbg_totals) p.dbg_totals[((size_t)b * T + t0 + t) * W + r] = w_total[r];
           }
           if (PGS == 1 || pg_role == 1) {  // prefix hash, row info of the next frame, parent look-up table
             unsigned long long hsh;
@@ -1228,7 +1227,6 @@ __global__ void __launch_bounds__(NT, (TIMING ? 1 : MINB)) BeamKernelV4(BeamPara
             while (atomicCAS(&s_htab[h], 0xffffffffu, entry) != 0xffffffffu) h = (h + 1) & (TS - 1);
           }
         }
-        if (p.dbg_n && tid == 0) p.dbg_n[(size_t)b * T + t0 + t] = n_new;
         CTCX_TICK(15)  // PG: state write
       }
       __syncthreads();

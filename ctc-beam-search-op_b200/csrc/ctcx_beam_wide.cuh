@@ -1,6 +1,7 @@
 // Beam kernel for WIDE vocabularies (32 < num_classes <= 2048: BASELINE's Conformer-BPE shape
-// C=1024, W=16). Derived from BeamKernelV3 (ctcx_beam_v3.cuh): same phases, same total order,
-// bit-identical results as the generic BeamKernel. What differs is how candidates are found: the
+// C=1024, W=16). Derived from the third generation of the narrow kernel (since grown into BeamKernelV4,
+// ctcx_beam_v4.cuh): same phases, same total order, bit-identical results as the generic BeamKernelT
+// (ctcx_beam_generic.cuh). What differs is how candidates are found: the
 // pre-pass (NormTopClassesKernel) orders every frame's best classes by log-prob; the children of a row
 // above ANY threshold are then a PREFIX of that order (fp addition is monotone), whose length an
 // exact binary search finds in ~log2(Kc) steps -- instead of scoring W*C children and issuing W*C
@@ -104,7 +105,7 @@ __global__ void __launch_bounds__(NT, ((NT <= 256 && !TIMING) ? 4 : 1)) BeamKern
   constexpr int TS = 8 * WMAX;  // parent look-up table slots (load factor <= 1/8: ~97% of the look-ups miss)
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int b = blockIdx.x;
-  const int W = p.W, C = p.C, T = p.T, B = p.B, blank = p.blank_index;
+  const int W = p.W, C = p.C, B = p.B, blank = p.blank_index;
   // streaming: frames already consumed by earlier chunks; this chunk contributes L more
   const int t_done = (p.t_done != nullptr) ? p.t_done[b] : 0;
   const int L = max(0, min(p.seq_len[b], p.Tcap - t_done));
@@ -254,7 +255,7 @@ __global__ void __launch_bounds__(NT, ((NT <= 256 && !TIMING) ? 4 : 1)) BeamKern
     if (warp == NWARP - 1 && t + 1 < L) {
       const size_t r1 = (size_t)(t + 1) * B + b;
       const size_t g0 = (size_t)(t + 1) * (size_t)p.tstride + (size_t)b * C;
-      if (sizeof(IN) != 4) {
+      if constexpr (sizeof(IN) != 4) {
         // half-precision logits: widened in registers on the way to shared memory. 16-byte loads (eight
         // elements per lane, all in flight together) where the row is aligned; this warp is idle during PA.
         const IN* g = reinterpret_cast<const IN*>(p.logits) + g0;
@@ -974,12 +975,10 @@ __global__ void __launch_bounds__(NT, ((NT <= 256 && !TIMING) ? 4 : 1)) BeamKern
           p.bp32[((size_t)b * p.Tcap + (t_done + t)) * W + r] = Rec64To32(rec, (unsigned)lbl);
         else
           p.bp[((size_t)b * p.Tcap + (t_done + t)) * W + r] = make_uint2(rec, (unsigned)lbl);
-        if (p.dbg_totals) p.dbg_totals[((size_t)b * T + t) * W + r] = nt_;
         unsigned h = (unsigned)hsh & (TS - 1);
         const unsigned entry = ((unsigned)(hsh >> 42) << 10) | (unsigned)r;
         while (atomicCAS(&s_htab[h], 0xffffffffu, entry) != 0xffffffffu) h = (h + 1) & (TS - 1);
       }
-      if (p.dbg_n && tid == 0) p.dbg_n[(size_t)b * T + t] = n_new;
       CTCX_TICK(15)  // PG: state write
     }
     asm volatile("cp.async.wait_all;\n" ::);

@@ -1,8 +1,12 @@
-// Host-side launch interface of the kernel translation units (k_narrow.cu, k_wide.cu, k_generic.cu,
-// k_post.cu). ctcx_api.cu -- validation, workspace carve-up, stream choreography -- sees the kernels
-// only through these functions, so each family of kernels compiles in its own translation unit.
+// Host-side launch interface of the kernel translation units, each of which holds one family of
+// kernels and their launchers: k_narrow.cu (BeamKernelV4), k_wide.cu (NormTopClassesKernel,
+// BeamKernelWide), k_generic.cu (the LogNorm normalisers, BeamKernelT) and k_post.cu (trace-back, scan,
+// pack). ctcx_api.cu -- validation, workspace carve-up, stream choreography -- sees the kernels only
+// through these functions.
 #pragma once
 #include <cuda_runtime.h>
+
+#include <atomic>
 
 #include "ctcx_params.h"
 
@@ -42,7 +46,65 @@ inline int RecBytes(int W, int C) { return (W <= 256 && C <= 256) ? 4 : 8; }
 constexpr int kListCapMax = 4608;  // candidate-list entries kept in shared memory (8 B each)
 // beam tier (slots per CTA) of the fast kernels' instantiations
 inline int TierOf(int W) { return (W <= 32) ? 32 : (W <= 128) ? 128 : 256; }
-int SmCount();  // multiprocessors of the current device (cached per device)
+
+// Facts about a device are cached for the first kMaxDevices device ordinals (queried anew on others).
+// The attribute and occupancy queries cost tens of microseconds of host time that would otherwise sit
+// between the kernels of every decode. Every cached fact is one atomic word, so concurrent callers
+// never see a half-written entry; callers racing on a first query store the same value.
+constexpr int kMaxDevices = 64;
+
+// multiprocessors of the current device
+inline int SmCount() {
+  static std::atomic<int> cached[kMaxDevices];
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const bool keep = dev >= 0 && dev < kMaxDevices;
+  int sms = keep ? cached[dev].load(std::memory_order_relaxed) : 0;
+  if (sms > 0) return sms;
+  sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (keep) cached[dev].store(sms, std::memory_order_relaxed);
+  return sms;
+}
+
+// Launch set-up of one kernel instantiation; its launcher keeps one as a function-local static.
+class KernelSetup {
+ public:
+  // Raises the kernel's dynamic shared-memory limit to `max_smem`, once per device: the most that any
+  // shape reaching the instantiation requests. The limit belongs to the function and the whole
+  // process, so it is never set lower, and no launch depends on what another host thread set.
+  cudaError_t RaiseSmemLimit(const void* kern, size_t max_smem) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const bool keep = dev >= 0 && dev < kMaxDevices;
+    if (keep && raised_[dev].load(std::memory_order_acquire)) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)max_smem);
+    if (e == cudaSuccess && keep) raised_[dev].store(true, std::memory_order_release);
+    return e;
+  }
+  // CTAs of the kernel (`threads` each, `smem` bytes of dynamic shared memory) that the current device
+  // keeps resident, remembered for the last `smem` asked about
+  cudaError_t Resident(const void* kern, int threads, size_t smem, long long* ctas) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const bool keep = dev >= 0 && dev < kMaxDevices;
+    const unsigned long long seen = keep ? resident_[dev].load(std::memory_order_relaxed) : 0ull;
+    if (seen != 0ull && (seen >> 32) == smem) {
+      *ctas = (long long)(seen & 0xffffffffull);
+      return cudaSuccess;
+    }
+    int per_sm = 1;
+    const cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem);
+    if (e != cudaSuccess) return e;
+    *ctas = (long long)SmCount() * (per_sm > 0 ? per_sm : 1);
+    if (keep) resident_[dev].store((unsigned long long)smem << 32 | (unsigned long long)*ctas, std::memory_order_relaxed);
+    return cudaSuccess;
+  }
+
+ private:
+  std::atomic<bool> raised_[kMaxDevices] = {};
+  std::atomic<unsigned long long> resident_[kMaxDevices] = {};  // smem << 32 | CTAs, 0 = not known yet
+};
 
 // ---- kernel 1 ----
 LaunchStatus LaunchLogNorm(const float* logits, float* off, long long rows, int C, int B, long long tstride,

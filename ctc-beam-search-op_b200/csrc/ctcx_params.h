@@ -22,8 +22,6 @@ struct BeamParamsT {
   int* fin_kind;     // [B,P] 1 = best alignment ends in blank
   int* fin_n;        // [B]   members in the final beam
   int* flags;        // [B]   bit0 rounding anomaly, bit1 fewer leaves than top_paths
-  R* dbg_totals;      // optional [B,T,W]
-  int* dbg_n;         // optional [B,T]
   long long* dbg_cycles;  // optional [B,dbg_slots]: clock64 cycles per phase (thread 0), summed over frames
   int dbg_slots;          // row length of dbg_cycles (>= 24)
   // streaming (Step / TopPaths / Reset, decoder.h:39-53); all null / T for a one-shot decode

@@ -4,47 +4,20 @@
 
 namespace ctcx {
 
-int SmCount() {
-  static int cached[64] = {0};
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  if (dev >= 0 && dev < 64 && cached[dev] > 0) return cached[dev];
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (dev >= 0 && dev < 64) cached[dev] = sms;
-  return sms;
-}
-
 namespace {
-// Launch configuration of one kernel instantiation on one device, computed once: the attribute and
-// occupancy queries cost tens of microseconds of host time that would otherwise sit between the
-// kernels of every decode. (A cache of immutable facts about the device, not decoder state.)
-struct LaunchCfg {
-  size_t smem = 0;   // dynamic shared memory the attribute was raised to
-  int resident = 0;  // CTAs the device keeps resident at that size
-};
-constexpr int kMaxDevices = 64;
+constexpr size_t kNarrowSmemMax = 220 * 1024;  // the most NarrowFastShape admits
 constexpr int kMinSliceFrames = 32;  // shorter slices would not amortise the hand-over
 
 template <typename IN, int WMAX, bool TIMING, int MINB, bool LM = false>
 LaunchStatus LaunchOne(BeamParamsT<typename ScoreOf<IN>::type>& p, size_t smem, cudaStream_t stream) {
   auto kern = BeamKernelV4<IN, WMAX, 256, TIMING, MINB, LM>;
-  static LaunchCfg cfgs[kMaxDevices];
-  int dev = 0;
-  cudaGetDevice(&dev);
-  LaunchCfg local;
-  LaunchCfg& cfg = (dev >= 0 && dev < kMaxDevices) ? cfgs[dev] : local;
-  if (cfg.resident == 0 || cfg.smem != smem) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return LaunchFrom(e, "cudaFuncSetAttribute(BeamKernelV4)");
-    // persistent CTAs: as many as the device keeps resident, each pulls utterances from p.queue
-    int per_sm = 1, sms = 148;
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, smem);
-    if (e != cudaSuccess) return LaunchFrom(e, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(BeamKernelV4)");
-    cfg.smem = smem;
-    cfg.resident = sms * (per_sm > 0 ? per_sm : 1);
-  }
-  const long long resident = cfg.resident;
+  static KernelSetup setup;
+  cudaError_t e = setup.RaiseSmemLimit((const void*)kern, kNarrowSmemMax);
+  if (e != cudaSuccess) return LaunchFrom(e, "shared-memory limit of BeamKernelV4");
+  // persistent CTAs: as many as the device keeps resident, each pulls utterances from p.queue
+  long long resident = 0;
+  e = setup.Resident((const void*)kern, 256, smem, &resident);
+  if (e != cudaSuccess) return LaunchFrom(e, "cudaOccupancyMaxActiveBlocksPerMultiprocessor(BeamKernelV4)");
   const unsigned grid = (unsigned)(p.B < resident ? p.B : resident);
   // Batches beyond the resident CTAs: cut every utterance into time slices so that the queue keeps all
   // CTAs busy to the end (the beam travels between slices through the state block in HBM, ~4 KB).
@@ -124,7 +97,7 @@ bool PrepareNarrow(BeamParamsT<R>& p) {
 
 bool NarrowFastShape(int W, int C) {
   if (C > 32 || W > 256 || (long long)W * C > kListCapMax) return false;
-  return SmemBytes(TierOf(W), W * C, true) <= 220 * 1024 && SmemBytes(TierOf(W), W * C, false, true) <= 220 * 1024;
+  return SmemBytes(TierOf(W), W * C, true) <= kNarrowSmemMax && SmemBytes(TierOf(W), W * C, false, true) <= kNarrowSmemMax;
 }
 
 LaunchStatus LaunchBeamNarrow(BeamParams& p, int in_dtype, cudaStream_t stream) {

@@ -1,6 +1,5 @@
 // Translation unit of the kernels after the beam search: trace-back of the top paths, prefix sums of
 // the sparse sizes, reduction of the per-utterance flags, sparse packing; plus the math test hooks.
-#define CTCX_WITH_POST
 #include "ctcx_kernels.cuh"
 #include "ctcx_launch.h"
 
@@ -8,6 +7,382 @@
 #include <cstdint>
 
 namespace ctcx {
+
+// ---------------------------------------------------------------------------------------------
+// Kernel 3: trace-back. One thread per (utterance, path) walks the back-pointer records from the
+// last frame to the first, emitting the alignment (entry.h:137-152) and the decoded labels
+// (entry.h:123-136, with optional repeat merging).
+// ---------------------------------------------------------------------------------------------
+// Back-pointer record formats: the generic / wide kernels write 8-byte records {packed word, label}
+// (PackRec), the narrow fast kernel 4-byte ones (PackRec32, ctcx_beam_v4.cuh).
+struct RecFields {
+  unsigned prev_self, an_src, ab_kind, an_kind;
+  int label;
+};
+__device__ __forceinline__ RecFields UnpackRec(const uint2 r) {
+  return {r.x & 0x7ffu, (r.x >> 11) & 0x7ffu, (r.x >> 22) & 1u, (r.x >> 23) & 3u, (int)r.y};
+}
+__device__ __forceinline__ RecFields UnpackRec(const unsigned r) {
+  return {r & 0xffu, (r >> 8) & 0xffu, (r >> 16) & 1u, (r >> 17) & 3u, (int)(r >> 24)};
+}
+
+
+template <typename REC>
+__global__ void __launch_bounds__(128) TraceKernel(TraceParams p) {
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= p.B * p.P) return;
+  const int b = idx / p.P, path = idx - b * p.P;
+  const int L = max(0, min(p.seq_len[b], p.T));  // out-of-range lengths are reported by the host, not walked
+  int* ali = p.ali + (size_t)idx * p.T;
+  int* dec = p.dec + (size_t)idx * p.T;
+  if (path >= p.fin_n[b] || L <= 0) {
+    p.dec_len[idx] = 0;
+    p.ali_len[idx] = 0;
+    return;
+  }
+  int slot = path;
+  int kind_ab = p.fin_kind[idx];
+  const REC* bp = reinterpret_cast<const REC*>(p.bp) + (size_t)b * p.T * p.W;
+  for (int t = L - 1; t >= 0; --t) {
+    const RecFields r = UnpackRec(bp[(size_t)t * p.W + min(slot, p.W - 1)]);
+    if (kind_ab) {
+      ali[t] = p.blank_label;
+      dec[t] = -1;
+      kind_ab = (r.ab_kind == kAbFromAb) ? 1 : 0;
+      slot = (int)r.prev_self;
+    } else {
+      ali[t] = r.label;
+      if (r.an_kind == kAnSelfAn) {
+        dec[t] = -1;
+        slot = (int)r.prev_self;
+      } else {
+        dec[t] = r.label;  // a new label was emitted at this frame
+        slot = (int)r.an_src;
+        kind_ab = (r.an_kind == kAnParAb) ? 1 : 0;
+      }
+    }
+  }
+  int pos = 0, prev = -1;
+  for (int t = 0; t < L; ++t) {
+    const int v = dec[t];
+    if (v >= 0) {
+      if (!p.merge_repeated || v != prev) dec[pos++] = v;
+      prev = v;
+    }
+  }
+  p.dec_len[idx] = pos;
+  p.ali_len[idx] = L;
+}
+
+// Warp-cooperative trace-back (used when there are too few walks to hide latency by themselves;
+// TraceKernel above is the simple form). One warp per (utterance, path). The walk is a dependent
+// chain (the slot at frame t-1 comes out of the record at frame t), but WHICH ROWS are needed next is
+// known in advance: the warp streams blocks of `rows` consecutive back-pointer rows [rows x W x 8 B,
+// contiguous in memory] into a double buffer in shared memory with cp.async, one block ahead of the
+// walk, so a step is one shared-memory broadcast read plus a few ALU operations instead of a
+// dependent trip to L2/HBM. Symbols are collected 32 frames at a time in registers and written as
+// coalesced rows; the decoded labels are compacted with warp ballots.
+// When a row of records is a multiple of 16 bytes (beam 100 with 4-byte records: 400 B) a block of rows is
+// ONE contiguous, 16-byte aligned span of HBM: it is fetched by a single bulk-copy instruction
+// (cp.async.bulk, the TMA unit's 1-D form) issued by one lane and signalled on an mbarrier, instead
+// of one 4-byte cp.async per record (3 200 per block).
+template <typename REC, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32) TraceWarpKernel(TraceParams p, int rows_log2, int use_bulk) {
+  extern __shared__ __align__(16) unsigned char tsm[];
+  __shared__ __align__(8) unsigned long long s_mbar[WARPS][2];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int idx = blockIdx.x * WARPS + warp;
+  if (idx >= p.B * p.P) return;
+  const int b = idx / p.P, path = idx - b * p.P;
+  const int L = max(0, min(p.seq_len[b], p.T));  // out-of-range lengths are reported by the host, not walked
+  int* ali = p.ali + (size_t)idx * p.T;
+  int* dec = p.dec + (size_t)idx * p.T;
+  if (path >= p.fin_n[b] || L <= 0) {
+    if (lane == 0) {
+      p.dec_len[idx] = 0;
+      p.ali_len[idx] = 0;
+    }
+    return;
+  }
+  const int W = p.W;
+  const int R = 1 << rows_log2;
+  REC* buf = reinterpret_cast<REC*>(tsm) + (size_t)warp * 2 * R * W;
+  const REC* bp = reinterpret_cast<const REC*>(p.bp) + (size_t)b * p.T * W;
+  const unsigned mbar0 = (unsigned)__cvta_generic_to_shared(&s_mbar[warp][0]);
+  if (use_bulk) {
+    if (lane == 0) {
+      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"(mbar0));
+      asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n" ::"r"(mbar0 + 8u));
+      asm volatile("fence.mbarrier_init.release.cluster;\n" ::: "memory");
+    }
+    __syncwarp();
+  }
+  // block k holds frames [k*R, min(L, (k+1)*R)); blocks are walked from the last one down
+  auto fetch_block = [&](int k) {
+    if (k >= 0) {
+      const int t0 = k << rows_log2;
+      const int nrec = (min(L, t0 + R) - t0) * W;
+      const REC* src = bp + (size_t)t0 * W;
+      const unsigned dst = (unsigned)__cvta_generic_to_shared(buf + (size_t)(k & 1) * R * W);
+      if (use_bulk) {
+        if (lane == 0) {
+          const unsigned bytes = (unsigned)nrec * (unsigned)sizeof(REC);
+          const unsigned mbar = mbar0 + 8u * (unsigned)(k & 1);
+          // the buffer was last read through ordinary loads (two blocks ago): order them before the
+          // asynchronous-proxy write
+          asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
+          asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;\n" ::"r"(mbar), "r"(bytes) : "memory");
+          asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];\n" ::"r"(dst),
+                       "l"(src), "r"(bytes), "r"(mbar)
+                       : "memory");
+        }
+      } else {
+        for (int i = lane; i < nrec; i += 32)
+          asm volatile("cp.async.ca.shared.global [%0], [%1], %2;\n" ::"r"(dst + (unsigned)sizeof(REC) * (unsigned)i),
+                       "l"(src + i), "n"(sizeof(REC)));
+      }
+    }
+    if (!use_bulk) asm volatile("cp.async.commit_group;\n" ::);
+  };
+  // wait until block k has landed (bulk path: the k-th use of its buffer flips the barrier's phase)
+  const int last_block = (L - 1) >> rows_log2;
+  auto wait_block = [&](int k) {
+    if (use_bulk) {
+      const unsigned mbar = mbar0 + 8u * (unsigned)(k & 1);
+      const unsigned parity = (unsigned)(((last_block - k) >> 1) & 1);
+      unsigned done = 0;
+      while (!done) {
+        asm volatile(
+            "{\n .reg .pred p;\n mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n selp.u32 %0, 1, 0, p;\n}\n"
+            : "=r"(done)
+            : "r"(mbar), "r"(parity)
+            : "memory");
+      }
+    } else {
+      asm volatile("cp.async.wait_group 1;\n" ::);
+    }
+  };
+  fetch_block(last_block);
+  int slot = path;
+  int kind_ab = p.fin_kind[idx];
+  int a_val = 0, d_val = -1;  // this lane's symbols of the current 32-frame store block
+  for (int k = last_block; k >= 0; --k) {
+    fetch_block(k - 1);  // next block in flight while this one is walked
+    wait_block(k);       // block k has landed
+    __syncwarp();
+    const REC* blk = buf + (size_t)(k & 1) * R * W;
+    const int t_lo = k << rows_log2;
+    for (int t = min(L, t_lo + R) - 1; t >= t_lo; --t) {
+      const RecFields r = UnpackRec(blk[(t - t_lo) * W + min(slot, W - 1)]);
+      int sym_a, sym_d = -1;
+      if (kind_ab) {  // entry.h:133-136: a blank frame
+        sym_a = p.blank_label;
+        kind_ab = (r.ab_kind == kAbFromAb) ? 1 : 0;
+        slot = (int)r.prev_self;
+      } else {
+        sym_a = r.label;
+        if (r.an_kind == kAnSelfAn) {
+          slot = (int)r.prev_self;
+        } else {
+          sym_d = r.label;  // a new label was emitted at this frame
+          slot = (int)r.an_src;
+          kind_ab = (r.an_kind == kAnParAb) ? 1 : 0;
+        }
+      }
+      if (lane == (t & 31)) {
+        a_val = sym_a;
+        d_val = sym_d;
+      }
+      if ((t & 31) == 0) {  // frames [t, t+32) complete: coalesced store
+        const int tt = t + lane;
+        if (tt < L) {
+          ali[tt] = a_val;
+          dec[tt] = d_val;
+        }
+      }
+    }
+    __syncwarp();  // buffer (k & 1) is refilled two iterations from now
+  }
+  __syncwarp();
+  // forward compaction of the new labels (entry.h:123-136, optional repeat merging)
+  int base = 0, carry = -1;
+  for (int t0 = 0; t0 < L; t0 += 32) {
+    const int tt = t0 + lane;
+    const int v = (tt < L) ? dec[tt] : -1;
+    const unsigned mask = __ballot_sync(kFull, v >= 0);
+    const unsigned pm = mask & ((1u << lane) - 1u);
+    const int prev_lane = pm ? (31 - __clz(pm)) : 0;
+    int prev_val = __shfl_sync(kFull, v, prev_lane);
+    if (!pm) prev_val = carry;
+    const bool keep = (v >= 0) && (!p.merge_repeated || v != prev_val);
+    const unsigned kmask = __ballot_sync(kFull, keep);
+    __syncwarp();
+    if (keep) dec[base + __popc(kmask & ((1u << lane) - 1u))] = v;
+    base += __popc(kmask);
+    if (mask) carry = __shfl_sync(kFull, v, 31 - __clz(mask));
+  }
+  if (lane == 0) {
+    p.dec_len[idx] = base;
+    p.ali_len[idx] = L;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Kernels 4/5: sparse packing (kernels.cc:163-257). ScanKernel: per path, exclusive prefix sums of
+// the lengths over the batch + totals + maxima. PackKernel: indices [b,pos], values, shapes.
+// ---------------------------------------------------------------------------------------------
+
+static __global__ void __launch_bounds__(1024) ScanKernel(ScanParams p) {
+  __shared__ long long s_sum[2][32];
+  __shared__ int s_max[2][32];
+  const int path = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const int per = (p.B + 1023) / 1024;
+  const int b0 = min(p.B, tid * per), b1 = min(p.B, b0 + per);
+  long long sum[2] = {0, 0};
+  int mx[2] = {0, 0};
+  for (int b = b0; b < b1; ++b) {
+    const int d = p.dec_len[(size_t)b * p.P + path], a = p.ali_len[(size_t)b * p.P + path];
+    sum[0] += d; sum[1] += a;
+    mx[0] = max(mx[0], d); mx[1] = max(mx[1], a);
+  }
+  long long incl[2];
+#pragma unroll
+  for (int w = 0; w < 2; ++w) {
+    long long v = sum[w];
+    int m = mx[w];
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const long long u = __shfl_up_sync(kFull, v, o);
+      if (lane >= o) v += u;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(kFull, m, o));
+    incl[w] = v;
+    if (lane == 31) s_sum[w][warp] = v;
+    if (lane == 0) s_max[w][warp] = m;
+  }
+  __syncthreads();
+  if (warp == 0) {
+#pragma unroll
+    for (int w = 0; w < 2; ++w) {
+      long long v = s_sum[w][lane];
+      int m = s_max[w][lane];
+#pragma unroll
+      for (int o = 1; o < 32; o <<= 1) {
+        const long long u = __shfl_up_sync(kFull, v, o);
+        if (lane >= o) v += u;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) m = max(m, __shfl_xor_sync(kFull, m, o));
+      s_sum[w][lane] = v;  // inclusive over warps
+      if (lane == 31) p.sizes[(w * 2) * p.P + path] = v;
+      if (lane == 0) p.sizes[(w * 2 + 1) * p.P + path] = m;
+    }
+  }
+  __syncthreads();
+#pragma unroll
+  for (int w = 0; w < 2; ++w) {
+    long long base = incl[w] - sum[w] + (warp > 0 ? s_sum[w][warp - 1] : 0);
+    long long* out = (w == 0 ? p.dec_off : p.ali_off) + (size_t)path * p.B;
+    for (int b = b0; b < b1; ++b) {
+      out[b] = base;
+      base += (w == 0) ? p.dec_len[(size_t)b * p.P + path] : p.ali_len[(size_t)b * p.P + path];
+    }
+  }
+}
+
+
+// Pointer table of the COMPACT output layout: all outputs of a decode as consecutive slices of one
+// int64 buffer -- per path: decoded indices [n,2], values [n], shape [2], alignment indices, values,
+// shape; then log_probability [B,P] (float32 pairs or float64 in int64 slots) -- computed on the device
+// from the sizes the scan left there, so that the pack can be enqueued before the host knows them.
+static __global__ void PackTableKernel(const long long* sizes, int B, int P, int real_bytes, long long* buf,
+                                       unsigned long long buf_elems, long long** ptrs, int* overflow) {
+  if (threadIdx.x != 0 || blockIdx.x != 0) return;
+  unsigned long long o = 0;
+  for (int p = 0; p < P; ++p) {
+    const unsigned long long nd = (unsigned long long)sizes[0 * P + p], na = (unsigned long long)sizes[2 * P + p];
+    ptrs[0 * P + p] = buf + o; o += 2 * nd;
+    ptrs[1 * P + p] = buf + o; o += nd;
+    ptrs[2 * P + p] = buf + o; o += 2;
+    ptrs[3 * P + p] = buf + o; o += 2 * na;
+    ptrs[4 * P + p] = buf + o; o += na;
+    ptrs[5 * P + p] = buf + o; o += 2;
+  }
+  ptrs[6 * P] = buf + o;
+  o += (real_bytes == 8) ? (unsigned long long)B * P : ((unsigned long long)B * P + 1) / 2;
+  if (o > buf_elems) *overflow = 1;
+}
+
+static __global__ void __launch_bounds__(128) PackKernel(PackParams p) {
+  if (p.skip != nullptr && *p.skip != 0) return;
+  const int b = blockIdx.x, path = blockIdx.y;
+  const size_t row = (size_t)b * p.P + path;
+  {
+    const int n = p.dec_len[row];
+    const long long o = p.dec_off[(size_t)path * p.B + b];
+    long long* idx = p.ptrs[0 * p.P + path];
+    long long* val = p.ptrs[1 * p.P + path];
+    const int* src = p.dec + row * p.T;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      idx[2 * (o + i)] = b;
+      idx[2 * (o + i) + 1] = i;
+      val[o + i] = src[i];
+    }
+  }
+  {
+    const int n = p.ali_len[row];
+    const long long o = p.ali_off[(size_t)path * p.B + b];
+    long long* idx = p.ptrs[3 * p.P + path];
+    long long* val = p.ptrs[4 * p.P + path];
+    const int* src = p.ali + row * p.T;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+      idx[2 * (o + i)] = b;
+      idx[2 * (o + i) + 1] = i;
+      val[o + i] = src[i];
+    }
+  }
+  if (threadIdx.x == 0) {
+    void* lp = (p.log_prob != nullptr) ? p.log_prob : (void*)p.ptrs[6 * p.P];
+    if (p.real_bytes == 8)  // kernels.cc:87-89
+      ((double*)lp)[row] = ((const double*)p.fin_total)[row];
+    else
+      ((float*)lp)[row] = ((const float*)p.fin_total)[row];
+    if (b == 0) {
+      long long* ds = p.ptrs[2 * p.P + path];
+      long long* as = p.ptrs[5 * p.P + path];
+      ds[0] = p.B; ds[1] = p.sizes[1 * p.P + path];  // kernels.cc:236-237
+      as[0] = p.B; as[1] = p.sizes[3 * p.P + path];  // kernels.cc:253-254
+    }
+  }
+}
+
+// Test hook: element-wise evaluation of the exact math functions.
+// op 0: expf, 1: log1pf, 2: logf, 3: LogSumExp(x, 0), 4: LogSumExp(0, x)
+static __global__ void MathTestKernel(int op, const float* x, float* y, int n) {
+  __shared__ unsigned long long s_tab[32];
+  LoadExpTable(s_tab, threadIdx.x, blockDim.x);
+  __syncthreads();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const float v = x[i];
+  y[i] = (op == 0) ? ExpfExact(v, s_tab) : (op == 1) ? Log1pfExact(v) : (op == 2) ? LogfExact(v)
+       : (op == 3) ? LogSumExp(v, 0.0f, s_tab) : LogSumExp(0.0f, v, s_tab);
+}
+
+// op 0: exp (x <= 0), 1: log (x >= 1), 2: LogSumExp(x, 0) of the double path
+static __global__ void MathTestKernelF64(int op, const double* x, double* y, int n) {
+  __shared__ unsigned long long s_tab[256];
+  __shared__ unsigned long long s_tabf[32];
+  for (int i = threadIdx.x; i < 256; i += blockDim.x) s_tab[i] = kCtcxExpTab[i];
+  LoadExpTable(s_tabf, threadIdx.x, blockDim.x);
+  __syncthreads();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double v = x[i];
+  y[i] = (op == 0) ? ExpExactD(v, s_tab) : (op == 1) ? LogExactD(v) : LogSumExp(v, 0.0, s_tabf);
+}
 
 namespace {
 // Reduces the per-utterance flags to stats[0..5] = {OR of anomaly bits, first b with too few leaves (or
@@ -77,14 +452,16 @@ LaunchStatus LaunchTrace(const TraceParams& tp, cudaStream_t stream) {
     TraceKernel<REC><<<(unsigned)((walks + 127) / 128), 128, 0, stream>>>(tp);
   } else {
     // one warp per (utterance, path); two blocks of 2^rows_log2 back-pointer rows per warp in
-    // shared memory (about 26 KB per block)
+    // shared memory (at most 26 KB per block: a single row of records, 8 KB at beam width 1024, is less)
     constexpr int kTraceWarps = 2;
+    constexpr size_t kBlockBytes = 26 * 1024;
     int rows_log2 = 5;
-    while (rows_log2 > 0 && ((size_t)W << rows_log2) * sizeof(REC) > 26 * 1024) --rows_log2;
+    while (rows_log2 > 0 && ((size_t)W << rows_log2) * sizeof(REC) > kBlockBytes) --rows_log2;
     const size_t tsm = (size_t)kTraceWarps * 2 * ((size_t)W << rows_log2) * sizeof(REC);
     auto tk = TraceWarpKernel<REC, kTraceWarps>;
-    cudaError_t e = cudaFuncSetAttribute(tk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsm);
-    if (e != cudaSuccess) return LaunchFrom(e, "cudaFuncSetAttribute(TraceWarpKernel)");
+    static KernelSetup setup;
+    const cudaError_t e = setup.RaiseSmemLimit((const void*)tk, kTraceWarps * 2 * kBlockBytes);
+    if (e != cudaSuccess) return LaunchFrom(e, "shared-memory limit of TraceWarpKernel");
     // a row of records that is a multiple of 16 bytes makes every block of rows one aligned span: bulk copies
     const int use_bulk = (((size_t)W * sizeof(REC)) % 16 == 0 && (reinterpret_cast<uintptr_t>(tp.bp) & 15u) == 0) ? 1 : 0;
     tk<<<(unsigned)((walks + kTraceWarps - 1) / kTraceWarps), kTraceWarps * 32, tsm, stream>>>(tp, rows_log2, use_bulk);

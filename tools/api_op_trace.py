@@ -1,7 +1,7 @@
 """What each C-ABI entry enqueues: one small call of every entry and route under torch.profiler (CUDA
-activities), printed per call as the ordered kernels (normalised names), memcpys (kind, bytes) and
-memsets (bytes), stream by stream, with the call's return code. Two builds of the library that should
-enqueue the same work print the same text:
+activities), printed per call as the ordered kernels (normalised names, grid, block, shared memory),
+memcpys (kind, bytes) and memsets (bytes), stream by stream, with the call's return code. Two builds of
+the library that should enqueue the same work print the same text:
 
     python tools/api_op_trace.py [--lib path/to/libctcx.so] > ops.txt
 
@@ -45,7 +45,8 @@ def gpu_ops(prof):
     for e in events:
         cat, a = e.get("cat", ""), e.get("args", {})
         if cat == "kernel":
-            text = "kernel " + norm_kernel(e["name"])
+            text = "kernel %s grid %s block %s smem %s" % (norm_kernel(e["name"]), a.get("grid"), a.get("block"),
+                                                         a.get("shared memory"))
         elif cat == "gpu_memcpy":
             text = "%s %d B" % (e["name"], a.get("bytes", -1))
         elif cat == "gpu_memset":

@@ -4,7 +4,9 @@
   python tools/sass_opcode_diff.py before.cubin after.cubin [kernel name substring]
 Prints, per kernel present in both, "same" or the opcodes whose counts differ. Operands (register
 numbers, constant-bank offsets, branch targets) are not compared: a change that only moves data
-leaves the histogram alone, one that adds or removes work does not."""
+leaves the histogram alone, one that adds or removes work does not. Names in an anonymous namespace
+carry a hash of their file's contents; it is dropped, so a kernel still pairs with itself after an edit
+elsewhere in that file."""
 import collections
 import re
 import subprocess
@@ -17,7 +19,7 @@ def histograms(cubin):
     for ln in out.split("\n"):
         m = re.match(r"\s*Function : (\S+)", ln)
         if m:
-            cur = m.group(1)
+            cur = re.sub(r"_GLOBAL__N__[0-9a-f]+_", "_GLOBAL__N__", m.group(1))
             hist[cur] = collections.Counter()
             continue
         m = re.match(r"\s*/\*[0-9a-f]{4,}\*/\s+(@!?U?P\w+\s+)?([A-Z][A-Z0-9_.]*)", ln)
