@@ -35,6 +35,7 @@ EXPORTS = ("ctcx_strerror", "ctcx_last_cuda_error", "ctcx_error_batch_index", "c
            "ctcx_pack_f32", "ctcx_pack_f64", "ctcx_pack_compact", "ctcx_finish", "ctcx_result_bytes", "ctcx_result_copy_async", "ctcx_result_parse", "ctcx_decode_host_f32", "ctcx_decode_host_f64", "ctcx_free_host",
            "ctcx_stream_workspace_bytes", "ctcx_stream_reset", "ctcx_stream_step_f32", "ctcx_stream_top_paths",
            "ctcx_stream_workspace_bytes_v", "ctcx_stream_reset_v", "ctcx_stream_step_v",
+           "ctcx_stream_reset_slots", "ctcx_stream_top_paths_slots",
            # measurement and test hooks
            "ctcx_workspace_views", "ctcx_profile_enable", "ctcx_profile_get", "ctcx_debug_set_cycles_buffer",
            "ctcx_debug_set_cycles_buffer_n",
@@ -119,6 +120,9 @@ def load():
     lib.ctcx_stream_top_paths.argtypes = [_vp] + [ctypes.c_int] * 5 + [ctypes.c_int, ctypes.c_int, _vp,
                                                                       ctypes.POINTER(CtcxSizes),
                                                                       ctypes.POINTER(ctypes.c_int32)]
+    lib.ctcx_stream_reset_slots.argtypes = [_vp, ctypes.c_size_t] + [_i] * 6 + [_vp, _vp]
+    lib.ctcx_stream_top_paths_slots.argtypes = [_vp] + [_i] * 7 + [_vp, _vp, ctypes.POINTER(CtcxSizes),
+                                                                    ctypes.POINTER(ctypes.c_int32)]
     lib.ctcx_profile_enable.argtypes = [ctypes.c_int]
     lib.ctcx_profile_enable.restype = None
     lib.ctcx_profile_get.argtypes = [ctypes.POINTER(ctypes.c_float)]

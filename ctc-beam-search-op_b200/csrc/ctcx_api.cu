@@ -327,9 +327,11 @@ int StreamStep(const Workspace& ws, unsigned char* base, int T_total, int B, int
 }
 
 // Trace-back of the top paths over the first seq_len[b] frames, then the sparse offsets and sizes and the
-// status words into the result block.
+// status words into the result block. `mask`: optional [B] device words, non-zero = utterance traced and
+// checked; the others contribute lengths 0.
 int TraceScanFlags(const Workspace& ws, unsigned char* base, const int* seq_len, int T, int B, int W, int P,
-                   int merge_repeated, int blank_label, cudaEvent_t after_trace, cudaStream_t stream) {
+                   int merge_repeated, int blank_label, cudaEvent_t after_trace, cudaStream_t stream,
+                   const int* mask = nullptr) {
   ctcx::TraceParams tp;
   tp.bp = base + ws.bp; tp.seq_len = seq_len;
   tp.fin_kind = (const int*)(base + ws.fin_kind); tp.fin_n = (const int*)(base + ws.fin_n);
@@ -337,6 +339,7 @@ int TraceScanFlags(const Workspace& ws, unsigned char* base, const int* seq_len,
   tp.merge_repeated = merge_repeated ? 1 : 0; tp.blank_label = blank_label;
   tp.dec_len = (int*)(base + ws.dec_len); tp.dec = (int*)(base + ws.dec);
   tp.ali_len = (int*)(base + ws.ali_len); tp.ali = (int*)(base + ws.ali);
+  tp.mask = mask;
   ctcx::ScanParams sp;
   sp.dec_len = tp.dec_len; sp.ali_len = tp.ali_len; sp.B = B; sp.P = P;
   sp.dec_off = (long long*)(base + ws.dec_off); sp.ali_off = (long long*)(base + ws.ali_off);
@@ -586,6 +589,47 @@ size_t ElemBytes(int dtype) {
 }
 int InDtypeOf(int dtype) {
   return dtype == CTCX_F16 ? ctcx::kInF16 : dtype == CTCX_BF16 ? ctcx::kInBF16 : ctcx::kInF32;
+}
+
+// argument checks of a stream reset (full or per slot), before any CUDA call; lays out *ws
+int CheckStreamReset(const void* workspace, size_t workspace_bytes, int score_dtype, int T_total, int B, int C, int W,
+                     int P, Workspace* ws) {
+  if (score_dtype != CTCX_F32 && score_dtype != CTCX_F64) return CTCX_ERR_BAD_ARGUMENT;
+  if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1) return CTCX_ERR_BAD_ARGUMENT;
+  if (W > kMaxBeamWidth || C > kMaxClasses) return CTCX_ERR_UNSUPPORTED;
+  if (P > W) return CTCX_ERR_TOO_MANY_PATHS;
+  ws->Init(T_total, B, C, W, P, (int)ElemBytes(score_dtype));
+  if (workspace == nullptr || workspace_bytes < ws->bytes || ((uintptr_t)workspace & 255u))
+    return CTCX_ERR_WORKSPACE;
+  return CTCX_OK;
+}
+
+// TopPaths() of a stream for the utterances `mask` selects (null = all), after the checks of its entry:
+// trace-back, sparse sizes and status words into the result block. sizes == NULL: only enqueued, completed
+// like a deferred decode; otherwise one synchronisation and the reference's checks.
+int StreamTopPaths(void* workspace, int T_total, int B, int C, int W, int P, int merge_repeated, int blank_label,
+                   const int* mask, cudaStream_t stream, ctcx_sizes* sizes, int32_t* flags_out) {
+  Workspace ws;
+  ws.Init(T_total, B, C, W, P);
+  unsigned char* base = (unsigned char*)workspace;
+  std::vector<unsigned char> h_res(ResultBytes(P), 0);
+  InitStats((int*)(h_res.data() + StatsOffset(P)), B);
+  const bool defer = (sizes == nullptr);
+  if (B > 0 || defer)  // (a deferred result is read from the device: it must hold the empty batch's too)
+    CTCX_CUDA(cudaMemcpyAsync(base + ws.result, h_res.data(), h_res.size(), cudaMemcpyHostToDevice, stream));
+  if (B > 0) {
+    CTCX_RC(TraceScanFlags(ws, base, (const int*)(base + ws.t_done) /* frames consumed so far */, T_total, B, W, P,
+                           merge_repeated, blank_label, nullptr, stream, mask));
+    // score types mixed since the reset, or a table with a positive entry: CTCX_ERR_BAD_ARGUMENT
+    CTCX_LAUNCH(ctcx::LaunchStreamCheck(base + ws.state, B, W, (const int*)(base + ws.ctrl) + kCtrlTablePositive,
+                                        (int*)(base + ws.stats), mask, stream));
+  }
+  if (defer) return CTCX_OK;
+  if (B > 0) {
+    CTCX_CUDA(cudaMemcpyAsync(h_res.data(), base + ws.result, h_res.size(), cudaMemcpyDeviceToHost, stream));
+    CTCX_CUDA(cudaStreamSynchronize(stream));
+  }
+  return ParseResult(h_res.data(), T_total, B, P, sizes, flags_out);
 }
 
 }  // namespace
@@ -1040,15 +1084,9 @@ size_t ctcx_stream_workspace_bytes_v(int score_dtype, int max_time_total, int B,
 int ctcx_stream_reset_v(void* workspace, size_t workspace_bytes, int score_dtype, int T_total, int B, int C, int W,
                         int P, void* stream_v) {
   cudaStream_t stream = (cudaStream_t)stream_v;
-  if (score_dtype != CTCX_F32 && score_dtype != CTCX_F64) return CTCX_ERR_BAD_ARGUMENT;
-  if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1) return CTCX_ERR_BAD_ARGUMENT;
-  if (W > kMaxBeamWidth || C > kMaxClasses) return CTCX_ERR_UNSUPPORTED;
-  if (P > W) return CTCX_ERR_TOO_MANY_PATHS;
-  const int score_bytes = (int)ElemBytes(score_dtype);
   Workspace ws;
-  ws.Init(T_total, B, C, W, P, score_bytes);
-  if (workspace == nullptr || workspace_bytes < ws.bytes || ((uintptr_t)workspace & 255u))
-    return CTCX_ERR_WORKSPACE;
+  CTCX_RC(CheckStreamReset(workspace, workspace_bytes, score_dtype, T_total, B, C, W, P, &ws));
+  const int score_bytes = (int)ElemBytes(score_dtype);
   unsigned char* base = (unsigned char*)workspace;
   Workspace::Header hdr = {kMagic, T_total, B, C, W, P, score_bytes};
   InitBlock init(ws, hdr, B);  // (zeroes the control words: no table with a positive entry yet)
@@ -1065,6 +1103,27 @@ int ctcx_stream_reset_v(void* workspace, size_t workspace_bytes, int score_dtype
     CTCX_CUDA(cudaMemcpyAsync(base + ws.flags, fl.data(), (size_t)B * 4, cudaMemcpyHostToDevice, stream));
   }
   return CTCX_OK;  // (copies from pageable memory are staged before the calls return)
+}
+
+int ctcx_stream_reset_slots(void* workspace, size_t workspace_bytes, int score_dtype, int T_total, int B, int C,
+                            int W, int P, const int32_t* slot_mask_dev, void* stream_v) {
+  Workspace ws;
+  CTCX_RC(CheckStreamReset(workspace, workspace_bytes, score_dtype, T_total, B, C, W, P, &ws));
+  if (slot_mask_dev == nullptr) return CTCX_ERR_BAD_ARGUMENT;
+  if (B == 0) return CTCX_OK;
+  unsigned char* base = (unsigned char*)workspace;
+  ctcx::StreamSlotsParams sp;
+  sp.state = base + ws.state;
+  sp.mask = slot_mask_dev;
+  sp.t_done = (int*)(base + ws.t_done);
+  sp.fin_total = base + ws.fin_total;
+  sp.fin_kind = (int*)(base + ws.fin_kind);
+  sp.fin_n = (int*)(base + ws.fin_n);
+  sp.flags = (int*)(base + ws.flags);
+  sp.B = B; sp.W = W; sp.P = P;
+  sp.score_bytes = (int)ElemBytes(score_dtype);
+  CTCX_LAUNCH(ctcx::LaunchStreamResetSlots(sp, (cudaStream_t)stream_v));
+  return CTCX_OK;
 }
 
 int ctcx_stream_reset(void* workspace, size_t workspace_bytes, int T_total, int B, int C, int W, int P,
@@ -1111,26 +1170,23 @@ int ctcx_stream_step_f32(void* workspace, int T_total, int B, int C, int W, int 
 
 int ctcx_stream_top_paths(void* workspace, int T_total, int B, int C, int W, int P, int merge_repeated,
                           int blank_label, void* stream_v, ctcx_sizes* sizes, int32_t* flags_out) {
-  cudaStream_t stream = (cudaStream_t)stream_v;
   if (workspace == nullptr || sizes == nullptr || ((uintptr_t)workspace & 255u)) return CTCX_ERR_WORKSPACE;
   if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1 || W > kMaxBeamWidth || C > kMaxClasses)
     return CTCX_ERR_BAD_ARGUMENT;
-  Workspace ws;
-  ws.Init(T_total, B, C, W, P);
-  unsigned char* base = (unsigned char*)workspace;
-  std::vector<unsigned char> h_res(ResultBytes(P), 0);
-  InitStats((int*)(h_res.data() + StatsOffset(P)), B);
-  if (B > 0) {
-    CTCX_CUDA(cudaMemcpyAsync(base + ws.result, h_res.data(), h_res.size(), cudaMemcpyHostToDevice, stream));
-    CTCX_RC(TraceScanFlags(ws, base, (const int*)(base + ws.t_done) /* frames consumed so far */, T_total, B, W, P,
-                           merge_repeated, blank_label, nullptr, stream));
-    // score types mixed since the reset, or a table with a positive entry: CTCX_ERR_BAD_ARGUMENT
-    CTCX_LAUNCH(ctcx::LaunchStreamCheck(base + ws.state, B, W, (const int*)(base + ws.ctrl) + kCtrlTablePositive,
-                                        (int*)(base + ws.stats), stream));
-    CTCX_CUDA(cudaMemcpyAsync(h_res.data(), base + ws.result, h_res.size(), cudaMemcpyDeviceToHost, stream));
-    CTCX_CUDA(cudaStreamSynchronize(stream));
-  }
-  return ParseResult(h_res.data(), T_total, B, P, sizes, flags_out);
+  return StreamTopPaths(workspace, T_total, B, C, W, P, merge_repeated, blank_label, nullptr, (cudaStream_t)stream_v,
+                        sizes, flags_out);
+}
+
+int ctcx_stream_top_paths_slots(void* workspace, int T_total, int B, int C, int W, int P, int merge_repeated,
+                                int blank_label, const int32_t* slot_mask_dev, void* stream_v, ctcx_sizes* sizes,
+                                int32_t* flags_out) {
+  if (workspace == nullptr || ((uintptr_t)workspace & 255u)) return CTCX_ERR_WORKSPACE;
+  if (T_total <= 0 || B < 0 || C <= 0 || W < 1 || P < 1 || W > kMaxBeamWidth || C > kMaxClasses)
+    return CTCX_ERR_BAD_ARGUMENT;
+  if (P > W) return CTCX_ERR_TOO_MANY_PATHS;
+  if (slot_mask_dev == nullptr) return CTCX_ERR_BAD_ARGUMENT;
+  return StreamTopPaths(workspace, T_total, B, C, W, P, merge_repeated, blank_label, slot_mask_dev,
+                        (cudaStream_t)stream_v, sizes, flags_out);
 }
 
 /* ---- measurement and test hooks (declared at the end of include/ctcx.h) ---- */

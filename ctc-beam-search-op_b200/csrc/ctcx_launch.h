@@ -127,7 +127,7 @@ LaunchStatus LaunchBeamGeneric(BeamParamsT<R>& p, cudaStream_t stream);
 
 // ---- kernels 3-5 ----
 // trace-back of the top paths, then per-path offsets / sizes and the reduction of the per-utterance
-// flags into `stats` (see FlagsKernel in k_post.cu)
+// flags into `stats` (see FlagsKernel in k_post.cu); with tp.mask set, over the selected utterances only
 LaunchStatus LaunchTraceScanFlags(const TraceParams& tp, int rec_bytes, const ScanParams& sp, const int* flags,
                                   int* stats, cudaStream_t stream, cudaEvent_t after_trace);
 LaunchStatus LaunchFlagsOnly(const int* seq_len, int B, int T, int* stats, cudaStream_t stream);
@@ -138,9 +138,12 @@ LaunchStatus LaunchPackTable(const long long* sizes, int B, int P, int real_byte
 LaunchStatus LaunchPositive(const float* v, long long n, int* flag, cudaStream_t stream);
 // streamed decodes (StreamHdrT): the state blocks of a reset stream with score_bytes (4 or 8) scores, and
 // the check before TopPaths -- stats[3] = 0 (a bad argument) if *table_flag is set or score types were mixed
+// (mask: optional [B], non-zero = utterance checked; null = all)
 LaunchStatus LaunchStreamReset(unsigned char* state, int B, int W, int score_bytes, cudaStream_t stream);
+// the reset of the utterances selected by p.mask only, entirely on the device
+LaunchStatus LaunchStreamResetSlots(const StreamSlotsParams& p, cudaStream_t stream);
 LaunchStatus LaunchStreamCheck(unsigned char* state, int B, int W, const int* table_flag, int* stats,
-                               cudaStream_t stream);
+                               const int* mask, cudaStream_t stream);
 // out[b] = frames of utterance b inside the time chunk [t0, t0 + len) (lengths clamped to [0, T])
 LaunchStatus LaunchChunkLen(const int* seq_len, int B, int T, int t0, int len, int* out, cudaStream_t stream);
 LaunchStatus LaunchMathTest(int op, const float* x, float* y, int n, cudaStream_t stream);

@@ -126,6 +126,20 @@ struct TraceParams {
   int* dec;      // [B,P,T]
   int* ali_len;  // [B,P]
   int* ali;      // [B,P,T]
+  const int* mask;  // optional [B]: non-zero = walk utterance b, zero = lengths 0 (null = every utterance)
+};
+
+// Reset() of selected utterances of a streamed decode (StreamResetSlotsKernel)
+struct StreamSlotsParams {
+  unsigned char* state;  // [B] state blocks (and the double blocks of a float64 stream)
+  const int* mask;       // [B] non-zero = reset utterance b
+  int* t_done;           // [B]
+  void* fin_total;       // [B,P] float or double
+  int* fin_kind;         // [B,P]
+  int* fin_n;            // [B]
+  int* flags;            // [B]
+  int B, W, P;
+  int score_bytes;       // 4 or 8
 };
 
 // Kernels 4/5: sparse packing

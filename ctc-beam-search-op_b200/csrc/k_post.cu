@@ -27,11 +27,35 @@ __device__ __forceinline__ RecFields UnpackRec(const unsigned r) {
 }
 
 
+// The trace kernels take their record type as TAG: REC itself, or Masked<REC> for the form that walks
+// only the utterances TraceParams::mask selects (the others get lengths 0 and load nothing else). The
+// one-shot decodes' instantiations thereby keep both their code and their names.
 template <typename REC>
+struct Masked {};
+template <typename TAG>
+struct TraceTag {
+  using Rec = TAG;
+  static constexpr bool kMasked = false;
+};
+template <typename REC>
+struct TraceTag<Masked<REC>> {
+  using Rec = REC;
+  static constexpr bool kMasked = true;
+};
+
+template <typename TAG>
 __global__ void __launch_bounds__(128) TraceKernel(TraceParams p) {
+  using REC = typename TraceTag<TAG>::Rec;
   const int idx = blockIdx.x * blockDim.x + threadIdx.x;
   if (idx >= p.B * p.P) return;
   const int b = idx / p.P, path = idx - b * p.P;
+  if constexpr (TraceTag<TAG>::kMasked) {
+    if (p.mask[b] == 0) {
+      p.dec_len[idx] = 0;
+      p.ali_len[idx] = 0;
+      return;
+    }
+  }
   const int L = max(0, min(p.seq_len[b], p.T));  // out-of-range lengths are reported by the host, not walked
   int* ali = p.ali + (size_t)idx * p.T;
   int* dec = p.dec + (size_t)idx * p.T;
@@ -86,14 +110,24 @@ __global__ void __launch_bounds__(128) TraceKernel(TraceParams p) {
 // ONE contiguous, 16-byte aligned span of HBM: it is fetched by a single bulk-copy instruction
 // (cp.async.bulk, the TMA unit's 1-D form) issued by one lane and signalled on an mbarrier, instead
 // of one 4-byte cp.async per record (3 200 per block).
-template <typename REC, int WARPS>
+template <typename TAG, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32) TraceWarpKernel(TraceParams p, int rows_log2, int use_bulk) {
+  using REC = typename TraceTag<TAG>::Rec;
   extern __shared__ __align__(16) unsigned char tsm[];
   __shared__ __align__(8) unsigned long long s_mbar[WARPS][2];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int idx = blockIdx.x * WARPS + warp;
   if (idx >= p.B * p.P) return;
   const int b = idx / p.P, path = idx - b * p.P;
+  if constexpr (TraceTag<TAG>::kMasked) {
+    if (p.mask[b] == 0) {
+      if (lane == 0) {
+        p.dec_len[idx] = 0;
+        p.ali_len[idx] = 0;
+      }
+      return;
+    }
+  }
   const int L = max(0, min(p.seq_len[b], p.T));  // out-of-range lengths are reported by the host, not walked
   int* ali = p.ali + (size_t)idx * p.T;
   int* dec = p.dec + (size_t)idx * p.T;
@@ -388,8 +422,14 @@ namespace {
 // Reduces the per-utterance flags to stats[0..5] = {OR of anomaly bits, first b with too few leaves (or
 // B), first b with sequence_length > T (or B), first b with negative sequence_length (or B), first b fed
 // more frames than a stream holds (or B), first b whose input frames never arrived (or B)}.
-__global__ void FlagsKernel(const int* flags, const int* seq_len, int B, int T, int* out) {
+// MASKED: only the utterances with mask[b] != 0 take part.
+template <bool MASKED>
+__device__ __forceinline__ void ReduceFlags(const int* flags, const int* seq_len, int B, int T, int* out,
+                                            const int* mask) {
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
+    if constexpr (MASKED) {
+      if (mask[b] == 0) continue;
+    }
     const int f = flags ? flags[b] : 0;
     if (f & 1) atomicOr(&out[0], 1);
     if (f & 2) atomicMin(&out[1], b);
@@ -398,6 +438,12 @@ __global__ void FlagsKernel(const int* flags, const int* seq_len, int B, int T, 
     if (f & 4) atomicMin(&out[4], b);
     if (f & 8) atomicMin(&out[5], b);
   }
+}
+__global__ void FlagsKernel(const int* flags, const int* seq_len, int B, int T, int* out) {
+  ReduceFlags<false>(flags, seq_len, B, T, out, nullptr);
+}
+__global__ void FlagsKernelMasked(const int* flags, const int* seq_len, int B, int T, int* out, const int* mask) {
+  ReduceFlags<true>(flags, seq_len, B, T, out, mask);
 }
 
 // flag = 1 if any entry is positive or NaN (scorer tables hold log-probabilities)
@@ -409,30 +455,54 @@ __global__ void PositiveKernel(const float* v, long long n, int* flag) {
 // Every float block holds the root (what a float kernel resumes if a float64 step advanced the frame
 // count: a valid beam, never foreign bytes), marked "no float step yet" and tagged with the stream's
 // score type; the double blocks of a float64 stream are marked unwritten.
+__device__ __forceinline__ void ResetStreamBlock(unsigned char* state, int B, int W, int score_bytes, int b) {
+  const StreamView fv(state + (size_t)b * StreamStateBytes(W), W);
+  fv.hdr->n = 1;
+  fv.hdr->gap = 0u;
+  fv.hdr->flags = kStreamNoF32Step;
+  fv.hdr->type = score_bytes;
+  fv.total[0] = 0.0f; fv.blk[0] = 0.0f; fv.lab[0] = NegInf(); fv.ab[0] = 0.0f; fv.an[0] = NegInf();
+  fv.label[0] = -1; fv.hash[0] = kRootHash; fv.phash[0] = 0ull;
+  if (score_bytes == 8) {
+    const StreamViewT<double> dv = StreamBlock64(state, B, W, b);
+    dv.hdr->n = 0;
+    dv.hdr->type = 0;
+  }
+}
 __global__ void StreamResetKernel(unsigned char* state, int B, int W, int score_bytes) {
-  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
-    const StreamView fv(state + (size_t)b * StreamStateBytes(W), W);
-    fv.hdr->n = 1;
-    fv.hdr->gap = 0u;
-    fv.hdr->flags = kStreamNoF32Step;
-    fv.hdr->type = score_bytes;
-    fv.total[0] = 0.0f; fv.blk[0] = 0.0f; fv.lab[0] = NegInf(); fv.ab[0] = 0.0f; fv.an[0] = NegInf();
-    fv.label[0] = -1; fv.hash[0] = kRootHash; fv.phash[0] = 0ull;
-    if (score_bytes == 8) {
-      const StreamViewT<double> dv = StreamBlock64(state, B, W, b);
-      dv.hdr->n = 0;
-      dv.hdr->type = 0;
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x)
+    ResetStreamBlock(state, B, W, score_bytes, b);
+}
+
+// Reset() of the utterances with mask[b] != 0: everything ctcx_stream_reset_v writes for b (the state
+// block, no frames consumed, the root as the final beam: one leaf, log-probability 0, and "fewer leaves
+// than top_paths" when P > 1), written on the device so that the launch can be captured in a graph.
+__global__ void StreamResetSlotsKernel(StreamSlotsParams p) {
+  for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < p.B; b += gridDim.x * blockDim.x) {
+    if (p.mask[b] == 0) continue;
+    ResetStreamBlock(p.state, p.B, p.W, p.score_bytes, b);
+    p.t_done[b] = 0;
+    for (int k = 0; k < p.P; ++k) {
+      if (p.score_bytes == 8) static_cast<double*>(p.fin_total)[(size_t)b * p.P + k] = 0.0;
+      else static_cast<float*>(p.fin_total)[(size_t)b * p.P + k] = 0.0f;
+      p.fin_kind[(size_t)b * p.P + k] = 0;
     }
+    p.fin_n[b] = 1;
+    p.flags[b] = (p.P > 1) ? 2 : 0;
   }
 }
 
 // A float64 step on a float stream marks the float header's type; a float step on a float64 stream drops
 // the "no float step yet" flag (float kernels rewrite the flags of every block they step).
-__global__ void StreamCheckKernel(const unsigned char* state, int B, int W, const int* table_flag, int* stats) {
+// mask: optional [B], non-zero = the utterance is checked (null = all); the table word is read for the
+// first utterance, or for every selected one.
+__global__ void StreamCheckKernel(const unsigned char* state, int B, int W, const int* table_flag, int* stats,
+                                  const int* mask) {
   for (int b = blockIdx.x * blockDim.x + threadIdx.x; b < B; b += gridDim.x * blockDim.x) {
+    if (mask != nullptr && mask[b] == 0) continue;
     const StreamHdr* h = reinterpret_cast<const StreamHdr*>(state + (size_t)b * StreamStateBytes(W));
     const bool mixed = (h->type & kStreamF64Stepped) || (h->type == 8 && !(h->flags & kStreamNoF32Step));
-    if (mixed || (b == 0 && *table_flag != 0)) atomicMin(&stats[3], 0);
+    if (mixed || ((mask != nullptr || b == 0) && *table_flag != 0)) atomicMin(&stats[3], 0);
   }
 }
 
@@ -449,7 +519,8 @@ LaunchStatus LaunchTrace(const TraceParams& tp, cudaStream_t stream) {
   if (walks >= 4096) {
     // thousands of independent walks hide the latency of the dependent loads by themselves, and
     // touch one record per frame instead of whole rows
-    TraceKernel<REC><<<(unsigned)((walks + 127) / 128), 128, 0, stream>>>(tp);
+    auto tk = tp.mask != nullptr ? TraceKernel<Masked<REC>> : TraceKernel<REC>;
+    tk<<<(unsigned)((walks + 127) / 128), 128, 0, stream>>>(tp);
   } else {
     // one warp per (utterance, path); two blocks of 2^rows_log2 back-pointer rows per warp in
     // shared memory (at most 26 KB per block: a single row of records, 8 KB at beam width 1024, is less)
@@ -458,9 +529,10 @@ LaunchStatus LaunchTrace(const TraceParams& tp, cudaStream_t stream) {
     int rows_log2 = 5;
     while (rows_log2 > 0 && ((size_t)W << rows_log2) * sizeof(REC) > kBlockBytes) --rows_log2;
     const size_t tsm = (size_t)kTraceWarps * 2 * ((size_t)W << rows_log2) * sizeof(REC);
-    auto tk = TraceWarpKernel<REC, kTraceWarps>;
-    static KernelSetup setup;
-    const cudaError_t e = setup.RaiseSmemLimit((const void*)tk, kTraceWarps * 2 * kBlockBytes);
+    const bool masked = tp.mask != nullptr;
+    auto tk = masked ? TraceWarpKernel<Masked<REC>, kTraceWarps> : TraceWarpKernel<REC, kTraceWarps>;
+    static KernelSetup setup, setup_masked;
+    const cudaError_t e = (masked ? setup_masked : setup).RaiseSmemLimit((const void*)tk, kTraceWarps * 2 * kBlockBytes);
     if (e != cudaSuccess) return LaunchFrom(e, "shared-memory limit of TraceWarpKernel");
     // a row of records that is a multiple of 16 bytes makes every block of rows one aligned span: bulk copies
     const int use_bulk = (((size_t)W * sizeof(REC)) % 16 == 0 && (reinterpret_cast<uintptr_t>(tp.bp) & 15u) == 0) ? 1 : 0;
@@ -478,7 +550,8 @@ LaunchStatus LaunchTraceScanFlags(const TraceParams& tp, int rec_bytes, const Sc
   ScanKernel<<<tp.P, 1024, 0, stream>>>(sp);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return LaunchFrom(e, "ScanKernel launch");
-  FlagsKernel<<<(tp.B + 255) / 256, 256, 0, stream>>>(flags, tp.seq_len, tp.B, tp.T, stats);
+  if (tp.mask != nullptr) FlagsKernelMasked<<<(tp.B + 255) / 256, 256, 0, stream>>>(flags, tp.seq_len, tp.B, tp.T, stats, tp.mask);
+  else FlagsKernel<<<(tp.B + 255) / 256, 256, 0, stream>>>(flags, tp.seq_len, tp.B, tp.T, stats);
   return LaunchFrom(cudaGetLastError(), "FlagsKernel launch");
 }
 
@@ -514,9 +587,14 @@ LaunchStatus LaunchStreamReset(unsigned char* state, int B, int W, int score_byt
   return LaunchFrom(cudaGetLastError(), "StreamResetKernel launch");
 }
 
+LaunchStatus LaunchStreamResetSlots(const StreamSlotsParams& p, cudaStream_t stream) {
+  StreamResetSlotsKernel<<<(unsigned)((p.B + 127) / 128), 128, 0, stream>>>(p);
+  return LaunchFrom(cudaGetLastError(), "StreamResetSlotsKernel launch");
+}
+
 LaunchStatus LaunchStreamCheck(unsigned char* state, int B, int W, const int* table_flag, int* stats,
-                               cudaStream_t stream) {
-  StreamCheckKernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(state, B, W, table_flag, stats);
+                               const int* mask, cudaStream_t stream) {
+  StreamCheckKernel<<<(unsigned)((B + 127) / 128), 128, 0, stream>>>(state, B, W, table_flag, stats, mask);
   return LaunchFrom(cudaGetLastError(), "StreamCheckKernel launch");
 }
 

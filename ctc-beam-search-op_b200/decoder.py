@@ -31,14 +31,18 @@ _RawBase = collections.namedtuple(
 
 class CTCExtBeamSearchDecoder(_RawBase):
     """The raw op's 7 output groups (indexable [0..6] like the generated TF wrapper). `.flags` carries
-    this decode's diagnostic bits (FLAG_ROUNDING_ANOMALY) -- an attribute, not an eighth output."""
+    this decode's diagnostic bits (FLAG_ROUNDING_ANOMALY) -- an attribute, not an eighth output.
+    `.slots`: the stream slots of the rows of a per-slot read (CTCExtBeamSearchDecoderStream), else None."""
     flags = 0
     d2h_bytes = 0
+    slots = None
 
 
 class DecodeResult(tuple):
-    """`(decoded, alignment, log_probability)` (README.md:19-31) plus a `.flags` attribute."""
+    """`(decoded, alignment, log_probability)` (README.md:19-31) plus `.flags` (and `.slots`, see
+    CTCExtBeamSearchDecoder) attributes."""
     flags = 0
+    slots = None
 
 
 class CtcxError(ValueError):
@@ -426,6 +430,12 @@ def ctc_ext_beam_search_decoder(inputs, sequence_length, beam_width, top_paths,
     return out
 
 
+def _to_device(a, device):
+    """A small host array on the device, through page-locked memory: the copy is only enqueued on the
+    current stream (a copy from pageable memory would wait for the work queued before it)."""
+    return torch.from_numpy(a).pin_memory().to(device, non_blocking=True)
+
+
 def _torch_dtype(dtype):
     """torch dtype of a torch or numpy dtype (np.float64, "float64", ...)."""
     if isinstance(dtype, torch.dtype):
@@ -446,6 +456,17 @@ class CTCExtBeamSearchDecoderStream:
             dec.step(chunk)                   # or dec.step(chunk, lengths) for ragged chunks
             decoded, alignment, logp = dec.top_paths()   # any time; does not disturb the state
         dec.reset()
+
+    Each of the B utterance positions (slots) can also start and finish on its own, so that a server can
+    keep B live streams in one batch: `reset(slots)` puts the selected slots back at the root (their
+    `max_time` budget starts again) and leaves the others untouched, and `top_paths(slots)` reads the
+    selected slots only:
+
+        done = [b for b in range(B) if finished[b]]
+        pending = dec.top_paths(done, wait=False)   # enqueued; stepping may go on before it is read
+        dec.reset(done)                             # the slots take new utterances from the next step
+        ...
+        decoded, alignment, logp = pending.result() # row i = slot done[i]
 
     dtype             score type of the stream (torch or numpy dtype): float32 (default) takes float32,
                       float16 and bfloat16 chunks (half chunks are read in place, as the one-shot decode
@@ -480,8 +501,9 @@ class CTCExtBeamSearchDecoderStream:
             raise RuntimeError("ctcx: no CUDA device available and there is no CPU fallback")
         self.merge_repeated, self.blank_index, self.blank_label = (bool(merge_repeated), int(blank_index),
                                                                    int(blank_label))
-        self.device = (torch.device(device) if device is not None
-                       else torch.device("cuda", torch.cuda.current_device()))
+        self.device = torch.device(device) if device is not None else torch.device("cuda")
+        if self.device.index is None:  # (an indexed device: CUDA masks are compared with it)
+            self.device = torch.device(self.device.type, torch.cuda.current_device())
         self._score_code = _lib.F64 if self._f64 else _lib.F32
         nbytes = self._lib.ctcx_stream_workspace_bytes_v(self._score_code, self.T, self.B, self.C, self.W, self.P)
         if nbytes == 0:
@@ -497,13 +519,57 @@ class CTCExtBeamSearchDecoderStream:
     def _chunk_dtypes(self):
         return (torch.float64,) if self._f64 else (torch.float32, torch.float16, torch.bfloat16)
 
-    def reset(self):
-        """Reset() (decoder.h:212-227): back to the empty prefix for every utterance."""
+    def reset(self, slots=None):
+        """Reset() (decoder.h:212-227): back to the empty prefix for every utterance, or, with `slots`, for
+        the selected slots only (the others keep their beams). A selection is one of
+          * an iterable of slot indices (list, tuple, range, ...),
+          * a bool or integer mask of shape [B] (numpy array or CPU tensor; non-zero = selected),
+          * a contiguous CUDA int32 [B] mask on the stream's device, used in place: no allocation, copy or
+            synchronisation, so `reset(mask)` can be captured into a CUDA graph with `step_device`.
+        A reset slot has consumed no frames and its flags are cleared; the stream-wide check of the scorer
+        table is not repeated (it was made at construction)."""
+        if slots is None:
+            with torch.cuda.device(self.device):
+                rc = self._lib.ctcx_stream_reset_v(self._ws.data_ptr(), self._nbytes, self._score_code, self.T,
+                                                   self.B, self.C, self.W, self.P, self._stream())
+            if rc != 0:
+                _raise(self._lib, rc)
+            return
+        mask, idx = self._selection(slots, host_indices=False)
+        if idx is not None and len(idx) == 0:
+            return
         with torch.cuda.device(self.device):
-            rc = self._lib.ctcx_stream_reset_v(self._ws.data_ptr(), self._nbytes, self._score_code, self.T, self.B,
-                                               self.C, self.W, self.P, self._stream())
+            rc = self._lib.ctcx_stream_reset_slots(self._ws.data_ptr(), self._nbytes, self._score_code, self.T,
+                                                   self.B, self.C, self.W, self.P, mask.data_ptr(), self._stream())
         if rc != 0:
             _raise(self._lib, rc)
+
+    def _selection(self, slots, host_indices=True):
+        """(device int32 [B] mask, sorted slot indices as an int64 numpy array) of a selection (see reset);
+        the indices of a CUDA mask are None unless host_indices, which then reads the mask back (one
+        synchronisation)."""
+        B = self.B
+        if isinstance(slots, torch.Tensor) and slots.is_cuda:
+            if not (slots.dtype == torch.int32 and tuple(slots.shape) == (B,) and slots.is_contiguous() and
+                    slots.device == self.device):
+                raise InvalidArgumentError(8, "a CUDA slot mask must be a contiguous int32 [%d] tensor on %s"
+                                           % (B, self.device))
+            return slots, (np.flatnonzero(slots.cpu().numpy()) if host_indices else None)
+        if isinstance(slots, (np.ndarray, torch.Tensor)):
+            m = slots.numpy() if isinstance(slots, torch.Tensor) else slots
+            if m.shape != (B,) or not (m.dtype == np.bool_ or np.issubdtype(m.dtype, np.integer)):
+                raise InvalidArgumentError(8, "a slot mask must be a bool or integer array of shape [%d], got %s %s"
+                                           % (B, m.dtype, m.shape))
+            idx = np.flatnonzero(m)
+        else:
+            vals = list(slots)
+            if not all(isinstance(v, (int, np.integer)) and not isinstance(v, (bool, np.bool_)) and 0 <= v < B
+                       for v in vals):
+                raise InvalidArgumentError(8, "slot indices must be integers in [0, %d), got %s" % (B, vals))
+            idx = np.unique(np.asarray(vals, dtype=np.int64))
+        mask = np.zeros(B, np.int32)
+        mask[idx] = 1
+        return _to_device(mask, self.device), idx.astype(np.int64)
 
     def _step(self, x, ln):
         """ctcx_stream_step_v on a frame-strided device chunk and device lengths; returns the code."""
@@ -578,33 +644,135 @@ class CTCExtBeamSearchDecoderStream:
         if rc != 0:
             _raise(self._lib, rc)
 
-    def top_paths_raw(self):
+    def top_paths_raw(self, slots=None, wait=True):
         """TopPaths() (decoder.h:229-261) of the frames consumed so far, as the raw 7 output groups
-        (device tensors; log_probability in the stream's score type)."""
-        P = self.P
+        (device tensors; log_probability in the stream's score type). Does not disturb the state.
+
+        slots   None: every utterance. Otherwise a selection (see reset): the reference's format for the
+                selected slots only, in ascending slot order -- batch index i is the i-th selected slot,
+                dense_shape[0] = n, log_probability [n, top_paths], `.slots` = the slot indices. A CUDA mask
+                is read back to learn them (one synchronisation). Over-fed slots, too few leaves and mixed
+                score types are reported for selected slots only.
+        wait    False: return a PendingDecode once the read is enqueued on the current stream; it reflects
+                the steps enqueued before this call, so the next chunk can be stepped (and the slots reset)
+                before `.result()` is read."""
+        full = slots is None
+        if full and wait:
+            return self._read(None, None, True)
+        mask, idx = self._selection(slots) if not full else (self._all_slots(), None)
+        return self._read(mask, idx, wait)
+
+    def _all_slots(self):
+        if getattr(self, "_ones", None) is None:
+            self._ones = torch.ones((self.B,), dtype=torch.int32, device=self.device)
+        return self._ones
+
+    def _read(self, mask, idx, wait):
+        """ctcx_stream_top_paths (mask None) or ctcx_stream_top_paths_slots, packed; idx = the selected slots
+        whose rows are kept (None: all rows)."""
+        lib, T, B, P, f64 = self._lib, self.T, self.B, self.P, self._f64
+        n = B if idx is None else len(idx)
+        if n == 0:
+            res = self._empty_result()
+            return res if wait else PendingDecode(lambda: res)
         arr = ctypes.c_int64 * P
         n_dec, max_dec, n_ali, max_ali = arr(), arr(), arr(), arr()
         sizes = _lib.CtcxSizes(n_dec, max_dec, n_ali, max_ali)
         flags = ctypes.c_int32(0)
+        ws, stream, attrs = self._ws.data_ptr(), self._stream(), (int(self.merge_repeated), self.blank_label)
+        # the one-shot decode's choice of route: the deferred one (one buffer of the upper bound, read later)
+        # up to DEFER_MAX_BYTES_DEVICE; beyond it the sizes first, then exactly sized outputs -- done at
+        # once, so that the result still reflects the steps enqueued before this call
+        n_bound = _bound_elems(T, B, P, torch.full((n,), T, dtype=torch.int32), f64)  # <= T frames per slot
+        deferred = not wait and 8 * n_bound <= DEFER_MAX_BYTES_DEVICE
+
+        def now():
+            with torch.cuda.device(self.device):
+                if mask is None:
+                    rc = lib.ctcx_stream_top_paths(ws, T, B, self.C, self.W, P, *attrs, stream, ctypes.byref(sizes),
+                                                   ctypes.byref(flags))
+                else:
+                    rc = lib.ctcx_stream_top_paths_slots(ws, T, B, self.C, self.W, P, *attrs, mask.data_ptr(), stream,
+                                                         ctypes.byref(sizes), ctypes.byref(flags))
+                if rc != 0:
+                    _raise(lib, rc)
+                groups, logp, _ = _pack(lib, self._ws, T, B, P, (n_dec, n_ali), self.device, stream, f64)
+                return self._rows(groups, logp, idx, int(flags.value))
+
+        if not deferred:
+            return now() if wait else PendingDecode(now, eager=True)
         with torch.cuda.device(self.device):
-            rc = self._lib.ctcx_stream_top_paths(self._ws.data_ptr(), self.T, self.B, self.C, self.W, P,
-                                                 int(self.merge_repeated), self.blank_label, self._stream(),
-                                                 ctypes.byref(sizes), ctypes.byref(flags))
+            # deferred, as a deferred one-shot decode: trace, then -- before any later step or reset rewrites
+            # the final beam -- compact pack, result block into page-locked memory, an event
+            rc = lib.ctcx_stream_top_paths_slots(ws, T, B, self.C, self.W, P, *attrs, mask.data_ptr(), stream,
+                                                 None, None)
             if rc != 0:
-                _raise(self._lib, rc)
-            groups, logp, _ = _pack(self._lib, self._ws, self.T, self.B, P, (n_dec, n_ali), self.device,
-                                    self._stream(), self._f64)
+                _raise(lib, rc)
+            buf = torch.empty((n_bound,), dtype=torch.int64, device=self.device)
+            rc = lib.ctcx_pack_compact(ws, T, B, P, 8 if f64 else 4, buf.data_ptr(), n_bound, stream)
+            if rc != 0:
+                _raise(lib, rc)
+            n_res = lib.ctcx_result_bytes(P)
+            hres = torch.empty((n_res,), dtype=torch.uint8, pin_memory=True)
+            rc = lib.ctcx_result_copy_async(ws, T, B, P, hres.data_ptr(), n_res, stream)
+            if rc != 0:
+                _raise(lib, rc)
+            done = torch.cuda.Event()
+            done.record(torch.cuda.current_stream(self.device))
+
+        def complete():
+            with torch.cuda.device(self.device):
+                done.synchronize()
+                rc = lib.ctcx_result_parse(hres.data_ptr(), T, B, P, ctypes.byref(sizes), ctypes.byref(flags))
+                if rc != 0:
+                    _raise(lib, rc)
+                groups, logp = _carve(buf[:_pack_elems(B, P, (n_dec, n_ali), f64)], B, P, (n_dec, n_ali), f64)
+                return self._rows(groups, logp, idx, int(flags.value))
+
+        return PendingDecode(complete)
+
+    def _rows(self, groups, logp, idx, flags):
+        """The raw result of the whole batch -> the rows of the slots idx (None: all), renumbered on the
+        device: batch column i = the i-th selected slot."""
+        if idx is not None:
+            n = len(idx)
+            lookup = np.full(self.B, -1, np.int64)
+            lookup[idx] = np.arange(n)
+            lookup = _to_device(lookup, self.device)
+            for p in range(self.P):
+                for g in (0, 3):
+                    if groups[g][p].shape[0]:
+                        groups[g][p][:, 0] = lookup[groups[g][p][:, 0]]
+                groups[2][p][0] = n
+                groups[5][p][0] = n
+            logp = logp[_to_device(idx, self.device)]
         res = CTCExtBeamSearchDecoder(*groups, logp)
-        res.flags = int(flags.value)
+        res.flags = flags
+        res.slots = idx
         return res
 
-    def top_paths(self):
-        raw = self.top_paths_raw()
-        decoded = [SparseTensor(i, v, s) for i, v, s in zip(raw[0], raw[1], raw[2])]
-        alignment = [SparseTensor(i, v, s) for i, v, s in zip(raw[3], raw[4], raw[5])]
-        out = DecodeResult((decoded, alignment, raw[6]))
-        out.flags = raw.flags
-        return out
+    def _empty_result(self):
+        dev, P = self.device, self.P
+        e = lambda *shape: torch.zeros(shape, dtype=torch.int64, device=dev)  # noqa: E731
+        groups = [[e(0, 2) for _ in range(P)], [e(0) for _ in range(P)], [e(2) for _ in range(P)],
+                  [e(0, 2) for _ in range(P)], [e(0) for _ in range(P)], [e(2) for _ in range(P)]]
+        res = CTCExtBeamSearchDecoder(*groups, torch.zeros((0, P), dtype=self.dtype, device=dev))
+        res.slots = np.zeros(0, np.int64)
+        return res
+
+    def top_paths(self, slots=None, wait=True):
+        """`(decoded, alignment, log_probability)` of top_paths_raw(slots, wait), `.slots` and `.flags`
+        attached; with wait=False a PendingDecode of it."""
+        def convert(raw):
+            decoded = [SparseTensor(i, v, s) for i, v, s in zip(raw[0], raw[1], raw[2])]
+            alignment = [SparseTensor(i, v, s) for i, v, s in zip(raw[3], raw[4], raw[5])]
+            out = DecodeResult((decoded, alignment, raw[6]))
+            out.flags = raw.flags
+            out.slots = raw.slots
+            return out
+
+        raw = self.top_paths_raw(slots, wait)
+        return convert(raw) if wait else PendingDecode(lambda: convert(raw.result()))
 
 
 def decode_host_cabi(inputs, sequence_length, beam_width, top_paths, merge_repeated=False,

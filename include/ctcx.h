@@ -294,6 +294,45 @@ int ctcx_stream_top_paths(void* workspace, int max_time_total, int batch, int nu
                           int beam_width, int top_paths, int merge_repeated, int blank_label,
                           void* stream, ctcx_sizes* sizes, int32_t* flags_out);
 
+/* ---- Per-utterance lifecycle of a stream: each of the `batch` positions (slots) of a stream can start
+ * and finish on its own. slot_mask_dev is a DEVICE int32 [batch]; non-zero selects the slot. Both
+ * entries only enqueue device work with no host staging of the mask, so the mask may be built or kept on
+ * the device, and ctcx_stream_reset_slots can be captured in a CUDA graph. A NULL mask is
+ * CTCX_ERR_BAD_ARGUMENT; the other argument checks are those of ctcx_stream_reset_v /
+ * ctcx_stream_top_paths, plus top_paths > beam_width (CTCX_ERR_TOO_MANY_PATHS), all before any CUDA call.
+ *
+ * ctcx_stream_reset_slots: Reset() (decoder.h:212-227) of the selected slots; the others keep their
+ * beams untouched. The workspace must have been reset once with ctcx_stream_reset_v(score_dtype, ...).
+ * A reset slot has consumed zero frames, so its max_time_total budget starts again (max_time_total
+ * bounds the longest utterance, not the frames that pass through a slot); its anomaly, overflow and
+ * too-few-leaves flags and its record of float32 / float64 steps are cleared; TopPaths of the slot before
+ * any step returns the root (one leaf, log-probability 0, empty sequences; "Less leaves" for
+ * top_paths > 1). The stream-wide mark of a scorer table with a positive entry is NOT cleared: only
+ * ctcx_stream_reset_v clears it. */
+int ctcx_stream_reset_slots(void* workspace, size_t workspace_bytes, int score_dtype, int max_time_total,
+                            int batch, int num_classes, int beam_width, int top_paths,
+                            const int32_t* slot_mask_dev, void* stream);
+/* ctcx_stream_top_paths_slots: TopPaths() (decoder.h:229-261) of the selected slots; does not disturb
+ * any state. The result has the workspace layout of ctcx_stream_top_paths for the whole batch: selected
+ * slots are traced as there, unselected ones contribute no decoded or alignment entries (lengths 0) and
+ * their log_probability rows are unspecified; dense_shape[p][1] is the maximum over the selected slots.
+ * The run-time checks cover the selected slots only: a slot fed more than max_time_total frames
+ * (CTCX_ERR_SEQ_LEN_RANGE, ctcx_error_batch_index() = the slot), too few leaves, mixed score types and
+ * the rounding-anomaly flag, so a finished slot can be read beside an over-fed or freshly reset one.
+ * sizes != NULL: synchronises `stream` once; follow with ctcx_pack_f32 / ctcx_pack_f64(workspace,
+ * max_time_total, batch, ...). sizes == NULL: deferred, only enqueues; complete it exactly like a deferred
+ * decode (ctcx_pack_compact + ctcx_finish, or ctcx_result_copy_async + ctcx_result_parse).
+ * Ordering, in both forms: the pack (ctcx_pack_f32 / _f64 / _compact) must be enqueued before the next
+ * ctcx_stream_step_*, ctcx_stream_reset* or ctcx_stream_top_paths* on the workspace, because it reads
+ * log_probability from the final beam, which every step and reset rewrites; ctcx_finish or
+ * ctcx_result_copy_async must come before the next ctcx_stream_top_paths*, which rewrites the sizes and
+ * status words. Steps and resets enqueued after the pack leave the result alone: it reflects the frames
+ * consumed by the steps enqueued before this call, even when it is read later. */
+int ctcx_stream_top_paths_slots(void* workspace, int max_time_total, int batch, int num_classes,
+                                int beam_width, int top_paths, int merge_repeated, int blank_label,
+                                const int32_t* slot_mask_dev, void* stream, ctcx_sizes* sizes,
+                                int32_t* flags_out);
+
 /* ---- Measurement and test hooks (not part of the operator's contract) ---- */
 
 /* Dense per-(b,p) rows as left in the workspace by a decode (device pointers into the workspace;
