@@ -89,18 +89,26 @@ def merge_repeats(label):
     return tuple(v for i, v in enumerate(label) if i == 0 or v != label[i - 1])
 
 
-def enumerate_labelings(lp, blank, limit=1 << 16):
+def enumerate_labelings(lp, blank, limit=1 << 16, table=None):
     """Every labeling with non-zero probability under lp = [T, C] and its exact (log p, Viterbi) pair,
     by an unpruned prefix search in float64. Only classes that are finite in a frame are expanded in
     it, so vocabularies of 65k classes with a few finite ones per frame stay cheap. Returns a dict
-    labeling -> (log p, Viterbi score); raises if more than `limit` labelings exist."""
+    labeling -> (log p, Viterbi score); raises if more than `limit` labelings exist.
+    table: a scorer table ([C + 1, C]) whose -inf entries forbid extensions: label c may follow prefix
+    `pre` only if table[(pre[-1] if pre else -1) + 1, c] is finite. The scores stay log p(l|x) and
+    Viterbi, without S(l)."""
     lp = np.asarray(lp, np.float64)
+    allowed = None if table is None else [set(np.flatnonzero(np.isfinite(np.asarray(r, np.float64))).tolist())
+                                          for r in table]
     # prefix -> [sum ending in blank, sum ending in label, max ending in blank, max ending in label]
     beams = {(): [0.0, NEG_INF, 0.0, NEG_INF]}
     for t in range(lp.shape[0]):
         row = lp[t]
         pb = row[blank]
         finite = [int(c) for c in np.flatnonzero(np.isfinite(row)) if c != blank]
+        if allowed is not None:
+            fin_set = set(finite)
+            succ = [sorted(fin_set & a) for a in allowed]
         nxt = {}
 
         def acc(key, k, v, comb):
@@ -117,7 +125,7 @@ def enumerate_labelings(lp, blank, limit=1 << 16):
             if pre and np.isfinite(row[pre[-1]]):  # the last label continues
                 acc(pre, 1, sn + row[pre[-1]], np.logaddexp)
                 acc(pre, 3, vn + row[pre[-1]], max)
-            for c in finite:
+            for c in (finite if allowed is None else succ[pre[-1] + 1 if pre else 0]):
                 ext = pre + (c,)
                 if pre and c == pre[-1]:  # a repeat needs a blank in between
                     acc(ext, 1, sb + row[c], np.logaddexp)
@@ -239,10 +247,82 @@ def masked_logits(T, B, C, blank, rng, k=(2, 3), span=40, dtype=np.float32):
     return x.astype(dtype)
 
 
-def max_labelings(x, sl, blank):
-    """The largest number of labelings with non-zero probability over the utterances of x = [T, B, C]:
-    the smallest beam width that prunes nothing."""
-    return max(len(enumerate_labelings(log_softmax(x[:sl[b], b]), blank)) for b in range(x.shape[1]))
+def max_labelings(x, sl, blank, table=None):
+    """The largest number of labelings with non-zero probability (and, with a table, a finite score)
+    over the utterances of x = [T, B, C]: the smallest beam width that prunes nothing."""
+    return max(len(enumerate_labelings(log_softmax(x[:sl[b], b]), blank, table=table)) for b in range(x.shape[1]))
+
+
+def dag_table(C, blank, seed, max_count, T=None, self_loop=False, quantum=None, n_start=None):
+    """A random constraint table [C + 1, C] float32 whose -inf entries make the labels a DAG, so that the
+    number of allowed labelings stays finite whatever T is:
+      * class l may follow class k only if l > k (non-blank classes in index order);
+      * row 0 (the empty prefix) allows a start set of n_start classes;
+      * allowed entries are random and finite (multiples of `quantum` if given, which makes ties);
+      * self_loop: one class may also follow itself (a repeat, with a blank between), which makes the
+        count grow with T; T is then required.
+    Edges are dropped at random until the allowed count (DP over the label graph: labelings that fit in
+    T frames, a repeat costing two) is at most max_count. Returns (table, count); the blank column is
+    -inf (the scorer never reads it)."""
+    rng = np.random.default_rng(seed)
+    labels = [c for c in range(C) if c != blank]
+    K = len(labels)
+    ok = np.zeros((C + 1, C), bool)
+    starts = rng.choice(labels, size=min(K, n_start or max(1, K // 3)), replace=False)
+    ok[0, starts] = True
+    p_edge = min(0.6, 8.0 / K)  # a few successors per class: the count starts above max_count, not astronomically
+    for i, k in enumerate(labels):
+        for l in labels[i + 1:]:
+            ok[k + 1, l] = rng.random() < p_edge
+    loop = None
+    if self_loop:
+        assert T is not None, "with a self-transition the count depends on T"
+        loop = int(rng.choice(labels))
+        ok[loop + 1, loop] = True
+    edges = [(r - 1, c) for r, c in zip(*np.nonzero(ok)) if r - 1 != c]  # (row label, class); the self-transition stays
+    rng.shuffle(edges)
+    n = dag_count(ok, blank, T)
+    for floor in (max_count // 2, 0):  # first keep edges whose loss would halve the count: land near max_count
+        kept = []
+        while n > max_count and edges:
+            r, c = edges.pop()
+            ok[r + 1, c] = False
+            m = dag_count(ok, blank, T)
+            if m < floor:
+                ok[r + 1, c] = True
+                kept.append((r, c))
+            else:
+                n = m
+        edges = kept
+    assert n <= max_count, (n, max_count)
+    vals = -np.abs(rng.standard_normal((C + 1, C))) * 2.0
+    if quantum is not None:
+        vals = np.round(vals / quantum) * quantum
+    table = np.where(ok, vals, -np.inf).astype(np.float32)
+    return table, n
+
+
+def dag_count(ok, blank, T=None):
+    """Labelings allowed by the boolean table `ok` ([C + 1, C]: label c may follow row r - 1) that fit in
+    T frames (None: any length; the graph must then be acyclic), the empty one included."""
+    C = ok.shape[1]
+    succ = [[c for c in np.flatnonzero(ok[r]) if c != blank] for r in range(C + 1)]
+    memo = {}
+
+    def count(row, budget):  # labelings continuing after `row` (its label is row - 1) in `budget` frames
+        key = (row, budget)
+        if key not in memo:
+            n = 1
+            for c in succ[row]:
+                cost = 2 if c == row - 1 else 1
+                if budget is None:
+                    assert c != row - 1, "a self-transition needs T"
+                    n += count(c + 1, None)
+                elif budget >= cost:
+                    n += count(c + 1, budget - cost)
+            memo[key] = n
+        return memo[key]
+    return count(0, T)
 
 
 def ctc_scores_many(lps, labels, blank):

@@ -424,25 +424,30 @@ MODEL_VARIANTS = {"exact": 0, "count_wiped_rows": 1, "four_rounds": 2}
 
 
 def model_decode_utts(logits, seq_len, beam_width, top_paths, merge_repeated=False, blank_index=0,
-                      blank_label=-1, variant="exact"):
+                      blank_label=-1, variant="exact", lm=None):
     """model_decode with the statistics of every utterance: (DenseResult, [dict per utterance],
     int32 [B, T] rounds of the revisit-wipe fixed point per frame, 0 where nobody is at risk).
     variant: "exact", or a fixed point with a known mistake -- "count_wiped_rows" (the candidates of
-    wiped rows still count) or "four_rounds" (stops after 4 rounds) -- to show that a case exposes it."""
+    wiped rows still count) or "four_rounds" (stops after 4 rounds) -- to show that a case exposes it.
+    lm: optional [C+1, C] float32 scorer table, as for oracle_decode."""
     build_model()
     lib = _load(MODEL_SO)
     logits, seq_len = _check_inputs(logits, seq_len)
     logits = logits.astype(np.float32, copy=False)
     T, B, C = logits.shape
+    if lm is not None:
+        lm = np.ascontiguousarray(lm, np.float32)
+        assert lm.shape == (C + 1, C)
     dec_len, dec, ali_len, ali, logp = _dense_out(B, top_paths, T, np.float32)
     st = np.zeros((max(B, 1), 16), np.int64)
     iters = np.zeros((max(B, 1), T), np.int32)
-    rc = lib.ctcx_model_decode_utts_f32(_ptr(logits, _c_float_p), T, B, C, _ptr(seq_len, _c_int_p),
-                                        beam_width, top_paths, int(bool(merge_repeated)), blank_index,
-                                        blank_label, _ptr(dec_len, _c_int_p), _ptr(dec, _c_int_p),
-                                        _ptr(ali_len, _c_int_p), _ptr(ali, _c_int_p), _ptr(logp, _c_float_p),
-                                        None, st.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)),
-                                        _ptr(iters, _c_int_p), MODEL_VARIANTS[variant])
+    rc = lib.ctcx_model_decode_lm_utts_f32(_ptr(logits, _c_float_p), T, B, C, _ptr(seq_len, _c_int_p),
+                                           beam_width, top_paths, int(bool(merge_repeated)), blank_index,
+                                           blank_label, None if lm is None else _ptr(lm, _c_float_p),
+                                           _ptr(dec_len, _c_int_p), _ptr(dec, _c_int_p),
+                                           _ptr(ali_len, _c_int_p), _ptr(ali, _c_int_p), _ptr(logp, _c_float_p),
+                                           None, st.ctypes.data_as(ctypes.POINTER(ctypes.c_longlong)),
+                                           _ptr(iters, _c_int_p), MODEL_VARIANTS[variant])
     if rc != 0:
         raise OracleError({2: "max_time is 0", 6: "requested more paths than the beam width.",
                            7: "Less leaves in the beam search than requested."}.get(rc, "error %d" % rc))
@@ -512,11 +517,13 @@ class Golden:
 # ----------------------------------------------------------------------------------------------
 # Revisit-wipe cases found by a search on the CPU model (tests/golden/make_wipe_cases.py)
 WIPE_NPZ = os.path.join(ROOT, "tests", "golden", "wipe_cases.npz")
+WIPE_TABLE_NPZ = os.path.join(ROOT, "tests", "golden", "wipe_table_cases.npz")  # (make_wipe_table_cases.py)
 
 
 class WipeCase:
     """One utterance of wipe_cases.npz: logits k/16 (float32, [T, 1, C]), decode attributes, and the
-    model's statistics (dict over MODEL_STATS) and fixed-point rounds per frame recorded for it."""
+    model's statistics (dict over MODEL_STATS) and fixed-point rounds per frame recorded for it. `lm`: the
+    case's scorer table ([C + 1, C] float32, k/16 with -inf) for wipe_table_cases.npz, else None."""
 
     def __init__(self, arr, name):
         k = arr[name + "/k"]
@@ -530,8 +537,16 @@ class WipeCase:
         self.stats = dict(zip(MODEL_STATS, arr[name + "/stats"].tolist()))
         self.iters = arr[name + "/iters"].astype(np.int32)
         self.sl = np.array([self.T], np.int32)
+        self.lm = None
+        if name + "/lm" in arr.files:
+            q = arr[name + "/lm"]
+            self.lm = np.where(q == -32768, -np.inf, q.astype(np.float32) / 16).astype(np.float32)
 
 
-def wipe_cases():
-    arr = np.load(WIPE_NPZ)
+def wipe_cases(path=WIPE_NPZ):
+    arr = np.load(path)
     return [WipeCase(arr, str(n)) for n in arr["names"]]
+
+
+def wipe_table_cases():
+    return wipe_cases(WIPE_TABLE_NPZ)

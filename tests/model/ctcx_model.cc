@@ -67,11 +67,16 @@ enum { kExact = 0, kCountWipedRows = 1, kFourRounds = 2 };
 struct Beam {
   int W, C, blank, blank_label;
   int variant = kExact;
+  const float* lm = nullptr;  // scorer table [C + 1, C] (row = label of the extended entry + 1), or null
   int n;
   std::vector<float> total, blk, lab, ab, an;
   std::vector<int> label;
   std::vector<uint64_t> hash, phash;
   std::vector<std::vector<BackPtr> > bp;
+
+  // GetStateExpansionScore (decoder.h:103,114,176,182): the base of a child of an entry with last label
+  // `from` (-1: the root) plus the table's entry, or the base unchanged without a table
+  float Expand(int from, int to, float base) const { return lm ? base + lm[(size_t)(from + 1) * C + to] : base; }
 
   void Reset() {  // decoder.h:212-227
     n = 1;
@@ -112,12 +117,12 @@ struct Beam {
         const int j = pslot[i];
         if (j >= 0) {
           if (label[i] == label[j]) {
-            v_nl = Lse(lab[i], blk[j]) + x[label[i]] - off;
+            v_nl = Lse(lab[i], Expand(label[j], label[i], blk[j])) + x[label[i]] - off;
             v_an = ab[j] + p; r.an_kind = AN_PAR_AB; r.an_src = j;
             float c2 = an[i] + p;
             if (c2 > v_an) { v_an = c2; r.an_kind = AN_SELF_AN; r.an_src = i; }
           } else {
-            v_nl = Lse(lab[i], total[j]) + x[label[i]] - off;
+            v_nl = Lse(lab[i], Expand(label[j], label[i], total[j])) + x[label[i]] - off;
             v_an = ab[j] + p; r.an_kind = AN_PAR_AB; r.an_src = j;
             float c2 = an[j] + p;
             if (c2 > v_an) { v_an = c2; r.an_kind = AN_PAR_AN; r.an_src = j; }
@@ -160,10 +165,10 @@ struct Beam {
         const float p = x[l] - off;
         Cand c; c.row = b; c.label = l;
         if (l == label[b]) {
-          c.s = p + blk[b];
+          c.s = p + Expand(label[b], l, blk[b]);
           c.an = ab[b] + p; c.an_kind = AN_PAR_AB;
         } else {
-          c.s = p + total[b];
+          c.s = p + Expand(label[b], l, total[b]);
           c.an = ab[b] + p; c.an_kind = AN_PAR_AB;
           float c2 = an[b] + p;
           if (c2 > c.an) { c.an = c2; c.an_kind = AN_PAR_AN; }
@@ -214,7 +219,7 @@ struct Beam {
         // rounding anomaly: the re-scored member would beat its own former total (see DESIGN.md)
         const int b = pslot[m];
         const float p = x[label[m]] - off;
-        const float s = (label[m] == label[b]) ? p + blk[b] : p + total[b];
+        const float s = p + Expand(label[b], label[m], (label[m] == label[b]) ? blk[b] : total[b]);
         if (s > nt[m]) st->anomalies++;
       }
       st->frames_wipe_matters += matters;
@@ -237,7 +242,7 @@ struct Beam {
         const int b = pslot[m];
         if (b < 0 || kept[m]) continue;
         const float p = x[label[m]] - off;
-        if (((label[m] == label[b]) ? p + blk[b] : p + total[b]) > nt[m]) st->suspects_dropped++;
+        if (p + Expand(label[b], label[m], (label[m] == label[b]) ? blk[b] : total[b]) > nt[m]) st->suspects_dropped++;
       }
     }
 
@@ -304,18 +309,20 @@ struct Beam {
 
 // stats_out: the statistics summed over the batch (maxima for *_max); utt_stats_out: optional [B,16],
 // the same per utterance; iters_out: optional [B,T], the fixed-point rounds of every frame (0 past the
-// utterance's length). variant: kExact, or one of the mistaken fixed points above.
-extern "C" int ctcx_model_decode_utts_f32(const float* logits, int T, int B, int C, const int* seq_len,
-                                          int W, int P, int merge_repeated, int blank_index,
-                                          int blank_label, int* dec_len, int* dec, int* ali_len, int* ali,
-                                          float* logp, long long* stats_out, long long* utt_stats_out,
-                                          int* iters_out, int variant) {
+// utterance's length). variant: kExact, or one of the mistaken fixed points above. lm: the scorer table
+// of ctcx_decode_scorer_f32 ([C + 1, C], entries <= 0, -inf allowed), or null for the default scorer.
+extern "C" int ctcx_model_decode_lm_utts_f32(const float* logits, int T, int B, int C, const int* seq_len,
+                                             int W, int P, int merge_repeated, int blank_index,
+                                             int blank_label, const float* lm, int* dec_len, int* dec,
+                                             int* ali_len, int* ali, float* logp, long long* stats_out,
+                                             long long* utt_stats_out, int* iters_out, int variant) {
   static_assert(sizeof(Stats) <= 16 * sizeof(long long), "the stats array has 16 slots");
   if (T == 0) return 2;
   for (int b = 0; b < B; ++b) if (!(seq_len[b] <= T)) return 5;
   Stats st; std::memset(&st, 0, sizeof(st));
   Beam beam; beam.W = W; beam.C = C; beam.blank = blank_index; beam.blank_label = blank_label;
   beam.variant = variant;
+  beam.lm = lm;
   std::vector<int> d, a;
   for (int b = 0; b < B; ++b) {
     Stats us; std::memset(&us, 0, sizeof(us));
@@ -349,6 +356,16 @@ extern "C" int ctcx_model_decode_utts_f32(const float* logits, int T, int B, int
   }
   if (stats_out) std::memcpy(stats_out, &st, sizeof(st));
   return 0;
+}
+
+extern "C" int ctcx_model_decode_utts_f32(const float* logits, int T, int B, int C, const int* seq_len,
+                                          int W, int P, int merge_repeated, int blank_index,
+                                          int blank_label, int* dec_len, int* dec, int* ali_len, int* ali,
+                                          float* logp, long long* stats_out, long long* utt_stats_out,
+                                          int* iters_out, int variant) {
+  return ctcx_model_decode_lm_utts_f32(logits, T, B, C, seq_len, W, P, merge_repeated, blank_index, blank_label,
+                                       nullptr, dec_len, dec, ali_len, ali, logp, stats_out, utt_stats_out,
+                                       iters_out, variant);
 }
 
 extern "C" int ctcx_model_decode_f32(const float* logits, int T, int B, int C, const int* seq_len,

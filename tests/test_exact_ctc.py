@@ -64,6 +64,50 @@ def test_exact_reference_with_masked_classes():
         assert abs(got[lab][0] - s) <= 1e-12 * (1 + abs(s)) and abs(got[lab][1] - m) <= 1e-12 * (1 + abs(m))
 
 
+def _allowed(table, lab):
+    """Every extension of the labeling has a finite table entry (row 0: the empty prefix)."""
+    return all(np.isfinite(table[(lab[k - 1] if k else -1) + 1, c]) for k, c in enumerate(lab))
+
+
+@pytest.mark.parametrize("T,C,blank,loop", [(4, 4, 0, False), (5, 4, 2, False), (6, 3, 1, True), (5, 4, 3, True),
+                                            (6, 4, 0, True)])
+def test_constrained_reference_against_brute_force(T, C, blank, loop):
+    """A DAG table (-inf entries forbid extensions): enumerate_labelings(table=) returns exactly the
+    brute-force labelings whose every extension is allowed, with unchanged scores, and dag_table's
+    count (DP over the label graph) is their number whenever every allowed labeling fits in T frames."""
+    rng = np.random.default_rng(10 * T + C + loop)
+    x = rng.standard_normal((T, C)) * 2.0
+    lp = X.log_softmax(x)
+    table, n = X.dag_table(C, blank, seed=T * C + loop, max_count=1 << 20, T=T, self_loop=loop)
+    assert np.isneginf(table).any() and np.isfinite(table).any()
+    want = {k: v for k, v in _brute_force(lp, blank).items() if _allowed(table, k)}
+    got = X.enumerate_labelings(lp, blank, table=table)
+    assert set(got) == set(want)
+    assert len(got) == n
+    assert n == X.dag_count(np.isfinite(table), blank, T)
+    if loop:
+        assert X.dag_count(np.isfinite(table), blank, T + 4) >= n  # the count grows with T
+    for lab, (s, m) in want.items():
+        assert abs(got[lab][0] - s) <= 1e-12 * (1 + abs(s)), lab
+        assert abs(got[lab][1] - m) <= 1e-12 * (1 + abs(m)), lab
+
+
+def test_dag_table_counts_and_shapes():
+    """dag_table lands at or below max_count (near it when the graph allows), keeps the DAG order l > k
+    off the self-transition, and its count does not depend on T once T exceeds the longest path."""
+    for C, blank, mc in ((12, 0, 42), (29, 28, 200), (32, 31, 255), (40, 3, 300), (300, 3, 600)):
+        table, n = X.dag_table(C, blank, seed=C + mc, max_count=mc)
+        ok = np.isfinite(table)
+        assert mc // 2 <= n <= mc, (C, n)
+        assert not ok[:, blank].any()
+        r, c = np.nonzero(ok[1:])
+        assert (c > r).all()
+        assert X.dag_count(ok, blank, T=C) == X.dag_count(ok, blank, T=10 * C) == n
+    table, n = X.dag_table(12, 3, seed=5, max_count=1000, quantum=0.25)
+    fin = table[np.isfinite(table)]
+    assert np.array_equal(fin, np.round(fin * 4) / 4) and len(np.unique(fin)) < len(fin)
+
+
 def _dense_paths(res, b, P):
     return [(res.decoded(b, p), res.alignment(b, p), float(res.logp[b, p])) for p in range(P)]
 
@@ -73,7 +117,7 @@ def _check_exact_regime(x, sl, W, P, merge, blank, table=None, exact=True):
     res = L.oracle_decode(x, sl, W, P, merge, blank, -1, lm=table)
     for b in range(x.shape[1]):
         lp = X.log_softmax(x[:sl[b], b])
-        labs = X.enumerate_labelings(lp, blank) if exact else None
+        labs = X.enumerate_labelings(lp, blank, table=table) if exact else None
         if exact:
             assert len(labs) <= W, "the beam can prune: %d labelings, beam %d" % (len(labs), W)
         bad = X.check_paths(_dense_paths(res, b, P), lp, blank, -1, merge, exact=exact, table=table,
@@ -114,6 +158,24 @@ def test_oracle_scorer_in_the_exact_regime(merge):
         x = rng.standard_normal((T, 3, C)).astype(np.float32)
         table = (-np.abs(rng.standard_normal((C + 1, C))) * 1.5).astype(np.float32)
         _check_exact_regime(x, np.full(3, T, np.int32), W, 4, merge, blank, table=table)
+
+
+@pytest.mark.parametrize("merge", [False, True])
+def test_oracle_constrained_exact_regime(merge):
+    """A DAG constraint table keeps the number of allowed labelings finite whatever T is, so the exact
+    regime is reachable at realistic T and C: at W = the count (the beam just fills) and W = 256 (it
+    never fills) the oracle returns the best labelings by log p(l|x) + S(l); one path more than the count
+    is the reference's "Less leaves" error."""
+    rng = np.random.default_rng(17 + merge)
+    for T, C, blank, mc in ((50, 12, 0, 42), (200, 29, 28, 120), (120, 32, 31, 255)):
+        table, n = X.dag_table(C, blank, seed=T + C + merge, max_count=mc)
+        x = (rng.standard_normal((T, 2, C)) * 1.5).astype(np.float32)
+        sl = np.array([T, T - 7], np.int32)
+        assert X.max_labelings(x, sl, blank, table=table) == n
+        for W in (n, 256):
+            _check_exact_regime(x, sl, W, min(n, 12), merge, blank, table=table)
+        with pytest.raises(L.OracleError, match="Less leaves"):
+            L.oracle_decode(x, sl, n + 1, n + 1, merge, blank, -1, lm=table)
 
 
 def test_oracle_masked_vocabulary_in_the_exact_regime():

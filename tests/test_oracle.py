@@ -12,6 +12,7 @@ import os
 import numpy as np
 import pytest
 
+import ctcx_exact as X
 import ctcx_testlib as L
 
 
@@ -147,6 +148,57 @@ def test_model_equals_oracle_random_shapes(seed):
                 L.model_decode(x, sl, W, P, merge, blank, -1)
             continue
         assert not L.same_result(a, L.model_decode(x, sl, W, P, merge, blank, -1))
+
+
+def _random_table(kind, C, blank, rng):
+    """A scorer table of one of the kinds the table tests use: dense random, a DAG of -inf constraints,
+    quantised (exact ties between children), or with entries of -1e3 / -1e4 beside mild ones."""
+    if kind == "random":
+        return (-np.abs(rng.standard_normal((C + 1, C))) * float(rng.choice([0.5, 1.5, 4]))).astype(np.float32)
+    if kind == "dag":
+        return X.dag_table(C, blank, int(rng.integers(0, 10000)), max_count=int(rng.integers(2, 300)))[0]
+    if kind == "quantised":
+        return (-np.floor(rng.random((C + 1, C)) * 4) / 4).astype(np.float32)
+    t = (-np.abs(rng.standard_normal((C + 1, C)))).astype(np.float32)
+    far = rng.random((C + 1, C)) < 0.3
+    return np.where(far, rng.choice([-1e3, -1e4], (C + 1, C)), t).astype(np.float32)
+
+
+@pytest.mark.parametrize("seed", range(4))
+def test_model_equals_oracle_with_scorer_tables(seed):
+    """The CPU model of the parallel formulation with a scorer table added to the member update's parent
+    base, the candidate scores and the wipe queries equals the oracle bit for bit, on dense, DAG,
+    quantised and far-negative tables; and the table cases do reach the revisit-wipe fixed point."""
+    rng = np.random.default_rng(2000 + seed)
+    at_risk = wiped = 0
+    for kind in ("random", "dag", "quantised", "far") * 2:
+        C = int(rng.integers(3, 40)); W = int(rng.integers(1, 64)); T = int(rng.integers(1, 60))
+        B = int(rng.integers(1, 6)); blank = int(rng.integers(0, C)); merge = bool(rng.integers(0, 2))
+        x = L.make_logits(["gauss", "peaky"][int(rng.integers(0, 2))], T, B, C, blank, int(rng.integers(0, 10000)),
+                          float(rng.choice([0.5, 1, 2])))
+        sl = L.ragged_lengths(T, B, seed)
+        table = _random_table(kind, C, blank, rng)
+        P = int(rng.integers(1, W + 1))
+        try:
+            a = L.oracle_decode(x, sl, W, P, merge, blank, -1, lm=table)
+        except L.OracleError as e:
+            with pytest.raises(L.OracleError, match=str(e)[:20]):
+                L.model_decode_utts(x, sl, W, P, merge, blank, -1, lm=table)
+            continue
+        res, st, _ = L.model_decode_utts(x, sl, W, P, merge, blank, -1, lm=table)
+        assert not L.same_result(a, res), (kind, C, W, T)
+        at_risk += sum(s["at_risk"] for s in st)
+        wiped += sum(s["wiped"] for s in st)
+    assert at_risk > 0 and wiped > 0, (at_risk, wiped)
+
+
+def test_model_with_a_zero_table_is_the_model_without():
+    """+0 on every expansion changes no score: results, statistics and fixed-point rounds are identical."""
+    x = L.make_logits("gauss", 80, 3, 29, 28, 4)
+    sl = L.ragged_lengths(80, 3, 4)
+    a = L.model_decode_utts(x, sl, 40, 3, True, 28, -1)
+    b = L.model_decode_utts(x, sl, 40, 3, True, 28, -1, lm=np.zeros((30, 29), np.float32))
+    assert not L.same_result(a[0], b[0]) and a[1] == b[1] and np.array_equal(a[2], b[2])
 
 
 def test_model_equals_oracle_cfg2_scale():
